@@ -90,6 +90,16 @@ def test_scale_tracing(cabi):
     assert scale.trace(lambda x: numpy.sqrt(x), 3) is None
 
 
+def test_negative_discard_is_rejected():
+    """The C ABI takes discard unsigned and ctypes wraps -1 around to 2^64 - 1, which would move the first Halton index to 0;
+    the binding refuses it instead (a traced scaling creates no context, so this needs no GPU)."""
+    import varsens_b200 as vb
+    with pytest.raises(vb.VarsensError, match="discard"):
+        vb.Sample(6, 8, lambda x: x, discard=-1)
+    from varsens_b200 import _cabi
+    assert _cabi.discard_arg(0) == 0 and _cabi.discard_arg(7) == 7
+
+
 def test_shard_range_partitions():
     from varsens_b200 import dist
     for total in (0, 1, 7, 1024, 2 ** 24 + 5):

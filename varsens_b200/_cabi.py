@@ -112,6 +112,15 @@ def check(status):
         raise err
 
 
+def discard_arg(discard):
+    """``discard`` as the C ABI takes it.  The ABI is unsigned: ctypes would wrap a negative value around 2^64 instead of
+    refusing it, so it is rejected here."""
+    d = int(discard)
+    if d < 0:
+        raise VarsensError("discard must be >= 0, got %d" % d)
+    return d
+
+
 def _is_torch_tensor(x):
     return type(x).__module__.startswith("torch") and hasattr(x, "data_ptr")
 
@@ -324,7 +333,7 @@ class Context(object):
         pp, pm, pk = buf(perm, numpy.uint32)
         rp, rm, rk = buf(raw, numpy.float64)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_sample_flat(self._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(row_begin),
+        check(lib().vs_sample_flat(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(row_begin),
                                    int(row_end), op, om))
         return out
 
@@ -337,7 +346,7 @@ class Context(object):
         pp, pm, pk = buf(perm, numpy.uint32)
         rp, rm, rk = buf(raw, numpy.float64)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_sample_flat_shard(self._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(i_begin), int(i_end), op, om))
+        check(lib().vs_sample_flat_shard(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(i_begin), int(i_end), op, om))
         return out
 
     # ---- objective values / estimators --------------------------------------------------------
@@ -350,7 +359,7 @@ class Context(object):
         pp, pm, pk = buf(perm, numpy.uint32)
         rp, rm, rk = buf(raw, numpy.float64)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_eval_values(self._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(objective),
+        check(lib().vs_eval_values(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
                                    par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end), op, om))
         return out
 
@@ -414,7 +423,7 @@ class Context(object):
         pp, pm, pk = buf(perm, numpy.uint32)
         rp, rm, rk = buf(raw, numpy.float64)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_fused_partials(self._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(objective),
+        check(lib().vs_fused_partials(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
                                       par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end),
                                       int(flags), op, om))
         return out
@@ -426,7 +435,7 @@ class Context(object):
         sp, keep = scale.c_struct(k)
         pp, pm, pk = buf(perm, numpy.uint32)
         rp, rm, rk = buf(raw, numpy.float64)
-        check(lib().vs_run_fused(self._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(objective),
+        check(lib().vs_run_fused(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
                                  par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(flags), ctypes.byref(cs)))
         return res
 
@@ -443,7 +452,7 @@ def _run_fused_p2p(self, k, n, perm, objective, params, world_size, rank, peer_b
     rp, rm, rk = buf(raw, numpy.float64)
     pb = (ctypes.c_uint64 * world_size)(*[int(x) for x in peer_bufs])
     pf = (ctypes.c_uint64 * world_size)(*[int(x) for x in peer_flags])
-    check(lib().vs_run_fused_p2p(self._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(objective),
+    check(lib().vs_run_fused_p2p(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
                                  par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end), int(flags),
                                  int(world_size), int(rank), pb, pf, int(epoch), ctypes.byref(cs)))
     return res
@@ -490,14 +499,14 @@ class FusedPlan(object):
             if i_begin != 0 or i_end != n:
                 raise VarsensError("a single-GPU plan covers the whole design")
             self._fn = L.vs_run_fused
-            self._args = (ctx._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(objective),
+            self._args = (ctx._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
                           par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(flags))
         else:
             pb = (ctypes.c_uint64 * exchange.world)(*[int(x) for x in exchange.peer_bufs])
             pf = (ctypes.c_uint64 * exchange.world)(*[int(x) for x in exchange.peer_flags])
             self._keep += (pb, pf)
             self._fn = L.vs_run_fused_p2p
-            self._args = (ctx._h, int(k), int(n), int(discard), pp, pm, rp, rm, sp, int(objective),
+            self._args = (ctx._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
                           par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end), int(flags),
                           int(exchange.world), int(exchange.rank), pb, pf)
 

@@ -354,6 +354,10 @@ int make_source(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *
                 uint64_t perm_count, const double *raw, int raw_mem, SourceDev *out) {
     memset(out, 0, sizeof(*out));
     VS_REQUIRE(perm, VS_ERR_ARG, "perm is NULL");
+    // Both bounds hold before anything is added, so start + 2n - 1 below cannot wrap around 2^64 (a wrapped start would
+    // reach Halton index 0, which is not a point of the sequence).
+    VS_REQUIRE(discard < (1ull << 32) && n < (1ull << 32), VS_ERR_RANGE, "discard %llu or n %llu does not fit 32 bits",
+               (unsigned long long)discard, (unsigned long long)n);
     out->n = n;
     out->start = 20ull * (uint64_t)k + discard + 1ull;          // saltelli.py:83: 20k + discard points skipped
     if (raw) {

@@ -76,7 +76,7 @@ class Sample(object):
         self.n = int(n)
         self.scaling = scaling
         self.verbose = verbose
-        self.discard = int(discard)
+        self.discard = _cabi.discard_arg(discard)
         self._ctx = None
         self._device = device
         self._explicit = None        # (M_1, M_2, N_j, N_nj) given by a flattened file
