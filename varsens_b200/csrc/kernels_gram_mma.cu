@@ -26,6 +26,7 @@
 #include "vs_internal.cuh"
 
 #include <algorithm>
+#include <cstdio>
 #include <cstdlib>
 #include <type_traits>
 #include <vector>
@@ -416,6 +417,15 @@ static int launch_mma_t(vs_ctx *c, const MmaGeom &g, size_t smem, uint64_t rows,
     time_end(c);
     c->launches++;
     VS_CUDA(cudaGetLastError());
+    if (!c->opt.trace.empty()) {
+        // VS_TRACE: the instantiation and plan that ran (the tests read chunks per CTA = ceil(ceil(rows / rc) / gx) from it)
+        if (FILE *f = fopen(c->opt.trace.c_str(), "a")) {
+            fprintf(f, "# gram_mma_kernel ST=%d multi=%d guard=%d gen=%d oddrun=%d warps=%d rs=%d upc=%d passes=%d rc=%d nstage=%d gx=%d rows=%llu second=%d\n",
+                    ST, (int)MULTI, (int)GUARD, (int)GEN, g.oddrun, g.warps, g.rs, g.upc, g.passes, g.rc, g.nstage, gx,
+                    (unsigned long long)rows, g.second);
+            fclose(f);
+        }
+    }
     // (without the second-order block only the block rows holding f(M_1), f(M_2) -- coordinates < 2l -- exist in the image)
     gram_mma_scatter_kernel<<<(unsigned)(((size_t)g.m * (g.m + 1) / 2 + 4 * g.l + 7) / 8), 256, 0, c->stream>>>(g.m, g.mpad, g.l, g.second ? g.m : 8 * g.imax, gx,
                                                                                  (const double *)c->block_buf.p, partials);

@@ -1,6 +1,7 @@
 // Objective evaluation to HBM (two-phase path), Gram/partial-sum reduction of given values, finalisation.
 #include "device.cuh"
 
+#include <cstdio>
 #include <type_traits>
 #include <vector>
 
@@ -237,6 +238,13 @@ static int launch_eval_pf_t(vs_ctx *c, int k, const SourceDev &src, const ScaleD
     time_end(c);
     c->launches++;
     VS_CUDA(cudaGetLastError());
+    if (!c->opt.trace.empty()) {                      // VS_TRACE: the form that ran; tiles per CTA = ceil(ntiles / grid)
+        if (FILE *fp = fopen(c->opt.trace.c_str(), "a")) {
+            fprintf(fp, "# eval_values_pf_kernel NR=%d grid=%u ntiles=%llu rows=%llu\n", NR, grid, (unsigned long long)ntiles,
+                    (unsigned long long)rows);
+            fclose(fp);
+        }
+    }
     return VS_OK;
 }
 
@@ -533,6 +541,13 @@ static int launch_gram_t(vs_ctx *c, const GramGeom &g, uint64_t rows, const doub
     time_end(c);
     c->launches++;
     VS_CUDA(cudaGetLastError());
+    if (!c->opt.trace.empty()) {                      // VS_TRACE: the form that ran; chunks per CTA = ceil(ceil(rows / R) / gx)
+        if (FILE *f = fopen(c->opt.trace.c_str(), "a")) {
+            fprintf(f, "# gram_kernel T=%d LG=%d RG=%d passes=%d R=%d gx=%d rows=%llu\n", T, g.LG, g.RG, g.passes, g.R, gx,
+                    (unsigned long long)rows);
+            fclose(f);
+        }
+    }
     return launch_gram_scatter(c, g, gx, (const double *)c->block_buf.p, partials, plen);
 }
 
