@@ -6,6 +6,45 @@
 namespace vs {
 
 // ---------------------------------------------------------------------------------------------
+// Inline PTX shared by the kernels: shared-window addresses, mbarriers, the FP64 tensor MMA, the global timer.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t *bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+// hint_ns: suspend-time hint of try_wait -- the warp sleeps in hardware instead of spinning
+constexpr uint32_t MBAR_HINT_NS = 0x989680u;   // the fused and Gram kernels' hint (the export kernel passes a shorter one)
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity, uint32_t hint_ns) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "WAIT_%=:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
+        "@p bra DONE_%=;\n"
+        "bra WAIT_%=;\n"
+        "DONE_%=:\n"
+        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"(hint_ns)
+        : "memory");
+}
+// mma.sync m8n8k4 f64: {c0, c1} += a * b (one A and one B element per lane)
+__device__ __forceinline__ void dmma_m8n8k4(double &c0, double &c1, double a, double b) {
+    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
+                 : "+d"(c0), "+d"(c1)
+                 : "d"(a), "d"(b));
+}
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Halton: ghalton's in-order digit sum (call sites varsens/saltelli.py:82-84; SURVEY.md App. C).
 //   x = 0; for j = 0.. (least-significant digit first): x += digit_j / b^(j+1)
 // digit_j / b^(j+1) is read from the host-built table, so the device performs exactly the same
@@ -514,8 +553,7 @@ __device__ __forceinline__ bool ll_reduce(const uint64_t *__restrict__ bufs, int
                                           double *__restrict__ dst, unsigned long long timeout_ns) {
     const int set = (int)(epoch & 1u);
     const char *mine = reinterpret_cast<const char *>(bufs[rank]) + ((size_t)set * world * plen) * 16;
-    unsigned long long t0;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t0));
+    const unsigned long long t0 = globaltimer_ns();
     bool ok = true;
     for (int e = threadIdx.x; e < plen; e += blockDim.x) {
         double s = 0.0;
@@ -525,9 +563,7 @@ __device__ __forceinline__ bool ll_reduce(const uint64_t *__restrict__ bufs, int
             for (;;) {
                 asm volatile("ld.volatile.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(lo), "=r"(f0), "=r"(hi), "=r"(f1) : "l"(p) : "memory");
                 if (f0 == epoch && f1 == epoch) break;
-                unsigned long long t1;
-                asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t1));
-                if (t1 - t0 > timeout_ns) { ok = false; break; }
+                if (globaltimer_ns() - t0 > timeout_ns) { ok = false; break; }
             }
             if (!ok) break;
             s += __hiloint2double((int)hi, (int)lo);

@@ -55,10 +55,8 @@ struct FusedConst {            // kernel parameter -> constant bank; indexed wit
     uint32_t ndc[K];           // digit rows the cached global table holds per dimension (layout: toff)
     int small_index;           // every Halton index of the run is < 2^29
     int poll_perm;             // see FusedTail::poll_perm
-    int alternate;             // (EPS == 2) E-warp teams alternate generate / evaluate phases -- measured slower, off
     long long *trace;          // profiling only (VS_TRACE): per-warp clock stamps of CTA 0, else nullptr
     int scale_kind;
-    int debug;                 // profiling only (VS_DEBUG_SKIP): bit 0 = skip generation, bit 1 = skip evaluation
 };
 
 // Everything the fused kernel does once the CTA partial sums are in HBM (one launch per step): two-level fixed-order combine
@@ -96,11 +94,6 @@ __device__ __forceinline__ unsigned ld_acquire_sys_u32(const unsigned *p) {
 }
 __device__ __forceinline__ void st_release_sys_u32(unsigned *p, unsigned v) {
     asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
 }
 
 // compile-time loop: fn(std::integral_constant<int, I>{}) for I in [0, N)
@@ -227,18 +220,13 @@ __device__ __forceinline__ void load_fixed_table(double *__restrict__ dst, const
 // (The compiler found that form by itself but re-built the {0, base} register pair with two moves for every step -- 270
 // IMAD.MOV per 32 rows in the ncu source view of the first single-launch build, profiles/r02_fused_stalls_by_line.txt.)
 // FIRST: the first term initialises the sum (0.0 + t == t for the non-negative table terms; saves a DADD per coordinate).
-#ifndef VS_ADDR_MODE
-#define VS_ADDR_MODE 4
-#endif
 template <uint32_t B, bool FAST, bool FIRST, uint32_t ROWOFF>
-__device__ __forceinline__ void digit_step(uint32_t &m, double &x, const char *__restrict__ tb, uint64_t basehi) {
+__device__ __forceinline__ void digit_step(uint32_t &m, double &x, uint64_t basehi) {
     double t;
-#if VS_ADDR_MODE == 4
     // The whole step in PTX, so that exactly these instructions come out: IMAD.WIDE (m * c), IMAD.HI with the persistent
     // {0, base} pair as addend (address of the term), LDS with the row offset as immediate, and the DADD.  (Written in C++ the
     // compiler decomposed the 64-bit product, added a uniform zero to the high word and masked low bits of the low word --
     // one or two extra instructions per step.)
-    (void)tb;
     if constexpr (FAST) {
         constexpr uint32_t C = (uint32_t)((0x100000000ull + B - 1) / B);
         asm("{\n\t"
@@ -259,53 +247,6 @@ __device__ __forceinline__ void digit_step(uint32_t &m, double &x, const char *_
         m = q;
         asm("ld.shared.f64 %0, [%1+%2];" : "=d"(t) : "l"((uint64_t)addr), "n"(ROWOFF));
     }
-#elif VS_ADDR_MODE == 0
-    uint32_t off8;
-    if constexpr (FAST) {
-        constexpr uint32_t C = (uint32_t)((0x100000000ull + B - 1) / B);
-        const uint64_t w = (uint64_t)m * C;
-        off8 = __umulhi((uint32_t)w, 8u * B);
-        m = (uint32_t)(w >> 32);
-    } else {
-        const uint32_t q = m / B;
-        off8 = (m - q * B) * 8u;
-        m = q;
-    }
-    (void)basehi;
-    t = *reinterpret_cast<const double *>(tb + ROWOFF + off8);
-#elif VS_ADDR_MODE == 1 || VS_ADDR_MODE == 2
-    uint32_t addr;
-    if constexpr (FAST) {
-        constexpr uint32_t C = (uint32_t)((0x100000000ull + B - 1) / B);
-        const uint64_t w = (uint64_t)m * C;
-        addr = (uint32_t)(((uint64_t)(uint32_t)w * (uint64_t)(8u * B) + basehi) >> 32);
-        m = (uint32_t)(w >> 32);
-    } else {
-        const uint32_t q = m / B;
-        addr = (m - q * B) * 8u + (uint32_t)(basehi >> 32);
-        m = q;
-    }
-    (void)tb;
-#if VS_ADDR_MODE == 1
-    asm("ld.shared.f64 %0, [%1+%2];" : "=d"(t) : "l"((uint64_t)addr), "n"(ROWOFF));
-#else
-    asm("ld.shared.f64 %0, [%1+%2];" : "=d"(t) : "r"(addr), "n"(ROWOFF));
-#endif
-#else
-    uint32_t off8;
-    if constexpr (FAST) {
-        constexpr uint32_t C = (uint32_t)((0x100000000ull + B - 1) / B);
-        const uint64_t w = (uint64_t)m * C;
-        off8 = __umulhi((uint32_t)w, 8u * B);
-        m = (uint32_t)(w >> 32);
-    } else {
-        const uint32_t q = m / B;
-        off8 = (m - q * B) * 8u;
-        m = q;
-    }
-    (void)tb;
-    asm("ld.shared.f64 %0, [%1+%2];" : "=d"(t) : "l"((basehi >> 32) + (uint64_t)off8), "n"(ROWOFF));
-#endif
     if constexpr (FIRST) x = t;
     else x = __dadd_rn(x, t);
 }
@@ -350,8 +291,7 @@ template <int K>
 __host__ __device__ constexpr int halton_groups() { return K > 1 ? (K - 1 + HG - 1) / HG : 1; }
 
 template <int K, int SCALE, int G, int IB, class Emit>
-__device__ __forceinline__ void halton_group(const FusedConst<K> &fc, const double *__restrict__ terms, uint64_t basehi, uint32_t ia,
-                                             uint32_t ib, Emit &&emit) {
+__device__ __forceinline__ void halton_group(const FusedConst<K> &fc, uint64_t basehi, uint32_t ia, uint32_t ib, Emit &&emit) {
     if constexpr (G == 0)
         emit(0, scale_coord<K, SCALE>(fc, 0, (double)__brev(ia) * 2.3283064365386962890625e-10),
              scale_coord<K, SCALE>(fc, 0, (double)__brev(ib) * 2.3283064365386962890625e-10));
@@ -361,23 +301,19 @@ __device__ __forceinline__ void halton_group(const FusedConst<K> &fc, const doub
         constexpr int JMAX = nd_ib<IB>(prime_at(D0));       // the smallest base of the group has the most digits
         uint32_t ma[N], mb[N];
         double xa[N], xb[N];
-        int ndmax = 0;
 #pragma unroll
         for (int u = 0; u < N; ++u) {
             ma[u] = ia;
             mb[u] = ib;
             xa[u] = 0.0;
             xb[u] = 0.0;
-            ndmax = ndmax > (int)fc.nd[D0 + u] ? ndmax : (int)fc.nd[D0 + u];
         }
-        const char *tb = reinterpret_cast<const char *>(terms);
         const bool small = IB <= 29 || fc.small_index != 0; // every index of the run < 2^29: FAST from digit 1 on
         // All digit positions an IB-bit index can have are executed unconditionally: one straight-line block per group, so
         // the scheduler can run the index chains ahead and keep many table loads in flight (with a branch per digit the
         // loads of digit j+1 could not be hoisted over the additions of digit j and every digit paid a full, queue-inflated
         // LDS latency).  Positions beyond a run's digit count see m == 0 and add +0.0 (exact).  IB is a template parameter
         // (26 or 32): BASELINE's configs all stay below 2^26 and visit 132 instead of 159 positions per point at k = 20.
-        (void)ndmax;
         static_for<JMAX>([&](auto Jc) {
             constexpr int J = decltype(Jc)::value;
             {
@@ -390,21 +326,21 @@ __device__ __forceinline__ void halton_group(const FusedConst<K> &fc, const doub
                         constexpr int AU = AR ? (D0 + U - AR_D0) : 0, AJ = J < AR_J ? J : AR_J - 1;
                         constexpr bool F1 = J == 0;
                         if constexpr (J == 0 && !(IB <= 29 && 8ull * B * ((1ull << (IB < 32 ? IB : 31))) <= 0x100000000ull)) {
-                            digit_step<B, false, F1, RO>(ma[U], xa[U], tb, basehi);
+                            digit_step<B, false, F1, RO>(ma[U], xa[U], basehi);
                             if constexpr (AR) digit_step_arith<B, false, F1>(mb[U], xb[U], fc.arh[AU][AJ], fc.arl[AU][AJ]);
-                            else digit_step<B, false, F1, RO>(mb[U], xb[U], tb, basehi);
+                            else digit_step<B, false, F1, RO>(mb[U], xb[U], basehi);
                         } else if constexpr (J == 0 || J >= jfast(B) || IB <= 29) {
-                            digit_step<B, true, F1, RO>(ma[U], xa[U], tb, basehi);
+                            digit_step<B, true, F1, RO>(ma[U], xa[U], basehi);
                             if constexpr (AR) digit_step_arith<B, true, F1>(mb[U], xb[U], fc.arh[AU][AJ], fc.arl[AU][AJ]);
-                            else digit_step<B, true, F1, RO>(mb[U], xb[U], tb, basehi);
+                            else digit_step<B, true, F1, RO>(mb[U], xb[U], basehi);
                         } else if (small) {
-                            digit_step<B, true, F1, RO>(ma[U], xa[U], tb, basehi);
+                            digit_step<B, true, F1, RO>(ma[U], xa[U], basehi);
                             if constexpr (AR) digit_step_arith<B, true, F1>(mb[U], xb[U], fc.arh[AU][AJ], fc.arl[AU][AJ]);
-                            else digit_step<B, true, F1, RO>(mb[U], xb[U], tb, basehi);
+                            else digit_step<B, true, F1, RO>(mb[U], xb[U], basehi);
                         } else {
-                            digit_step<B, false, F1, RO>(ma[U], xa[U], tb, basehi);
+                            digit_step<B, false, F1, RO>(ma[U], xa[U], basehi);
                             if constexpr (AR) digit_step_arith<B, false, F1>(mb[U], xb[U], fc.arh[AU][AJ], fc.arl[AU][AJ]);
-                            else digit_step<B, false, F1, RO>(mb[U], xb[U], tb, basehi);
+                            else digit_step<B, false, F1, RO>(mb[U], xb[U], basehi);
                         }
                     }
                 });
@@ -416,8 +352,8 @@ __device__ __forceinline__ void halton_group(const FusedConst<K> &fc, const doub
 }
 
 template <int K, int SCALE, int IB, class Emit>
-__device__ __forceinline__ bool gen_rows_impl(const SourceDev &src, const FusedConst<K> &fc, const double *__restrict__ terms,
-                                         uint64_t basehi, uint64_t i_begin, uint64_t rows, uint64_t bt, int lane, Emit &&emit) {
+__device__ __forceinline__ bool gen_rows_impl(const SourceDev &src, const FusedConst<K> &fc, uint64_t basehi, uint64_t i_begin,
+                                              uint64_t rows, uint64_t bt, int lane, Emit &&emit) {
     uint64_t r = bt * 32 + lane;
     const bool valid = r < rows;
     const uint64_t i = i_begin + (valid ? r : rows - 1);
@@ -444,18 +380,18 @@ __device__ __forceinline__ bool gen_rows_impl(const SourceDev &src, const FusedC
         for (int d = 0; d < K; ++d) emit(d, scale_coord<K, SCALE>(fc, d, ra[d]), scale_coord<K, SCALE>(fc, d, rb[d]));
     } else {
         const uint32_t ia = (uint32_t)(src.start + i), ib = (uint32_t)(src.start + src.n + pi);
-        static_for<halton_groups<K>()>([&](auto Gc) { halton_group<K, SCALE, decltype(Gc)::value, IB>(fc, terms, basehi, ia, ib, emit); });
+        static_for<halton_groups<K>()>([&](auto Gc) { halton_group<K, SCALE, decltype(Gc)::value, IB>(fc, basehi, ia, ib, emit); });
     }
     return valid;
 }
 
 // One warp-uniform branch on the scale kind for the whole row (not one per coordinate).
 template <int K, int IB = 32, class Emit>
-__device__ __forceinline__ bool gen_rows(const SourceDev &src, const FusedConst<K> &fc, const double *__restrict__ terms,
-                                         uint64_t basehi, uint64_t i_begin, uint64_t rows, uint64_t bt, int lane, Emit &&emit) {
-    if (fc.scale_kind == VS_SCALE_IDENTITY) return gen_rows_impl<K, VS_SCALE_IDENTITY, IB>(src, fc, terms, basehi, i_begin, rows, bt, lane, emit);
-    if (fc.scale_kind == VS_SCALE_LINEAR) return gen_rows_impl<K, VS_SCALE_LINEAR, IB>(src, fc, terms, basehi, i_begin, rows, bt, lane, emit);
-    return gen_rows_impl<K, VS_SCALE_POWER, IB>(src, fc, terms, basehi, i_begin, rows, bt, lane, emit);
+__device__ __forceinline__ bool gen_rows(const SourceDev &src, const FusedConst<K> &fc, uint64_t basehi, uint64_t i_begin, uint64_t rows,
+                                         uint64_t bt, int lane, Emit &&emit) {
+    if (fc.scale_kind == VS_SCALE_IDENTITY) return gen_rows_impl<K, VS_SCALE_IDENTITY, IB>(src, fc, basehi, i_begin, rows, bt, lane, emit);
+    if (fc.scale_kind == VS_SCALE_LINEAR) return gen_rows_impl<K, VS_SCALE_LINEAR, IB>(src, fc, basehi, i_begin, rows, bt, lane, emit);
+    return gen_rows_impl<K, VS_SCALE_POWER, IB>(src, fc, basehi, i_begin, rows, bt, lane, emit);
 }
 
 // {0, shared-window address of the term table} as one opaque 64-bit value (see digit_step)
@@ -622,7 +558,7 @@ __device__ __forceinline__ void rows_phase(const SourceDev &src, const FusedCons
                                            uint64_t rows, uint64_t bt, int lane, double *__restrict__ Yrow, double shift,
                                            double &sA, double &qA, double &sB, double &qB) {
     double a[K], b[K];
-    const bool valid = gen_rows<K>(src, fc, terms, table_basehi(terms), i_begin, rows, bt, lane, [&](int d, double xa, double xb) {
+    const bool valid = gen_rows<K>(src, fc, table_basehi(terms), i_begin, rows, bt, lane, [&](int d, double xa, double xb) {
         a[d] = xa;
         b[d] = xb;
     });
@@ -739,54 +675,6 @@ fused_kernel(SourceDev src, FusedConst<K> fc, F f, uint64_t i_begin, uint64_t i_
 // ---------------------------------------------------------------------------------------------
 constexpr int WS_S = 4;                       // one S-warp per SM sub-partition
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity), "r"(0x989680u)   // suspend-time hint: sleep in hardware instead of spinning
-        : "memory");
-}
-
-// Consumer-side wait with explicit back-off.  try_wait with a suspend hint compiles to a TRYWAIT / NANOSLEEP.SYNCS / BRA loop that
-// still issued ~680 instructions per 32-row batch from the (mostly idle) S-warps -- 14 % of all issued instructions in the ncu
-// capture of the first single-launch build, competing with the E-warps of the same sub-partition for issue slots.  The S-warp has
-// slack (it works ~15 % of the time), so it polls with test_wait and sleeps VS_SBACKOFF ns between polls.
-#ifndef VS_SBACKOFF
-#define VS_SBACKOFF 0
-#endif
-__device__ __forceinline__ void mbar_wait_consumer(uint64_t *bar, uint32_t parity) {
-#if VS_SBACKOFF > 0
-    for (;;) {
-        uint32_t done;
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n"
-            : "=r"(done)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-        if (done) break;
-        __nanosleep(VS_SBACKOFF);
-    }
-#else
-    mbar_wait(bar, parity);
-#endif
-}
-
 // ---------------------------------------------------------------------------------------------
 // Two-role variant with the Gram update on the FP64 tensor path (DMMA, mma.sync m8n8k4.f64).
 // Measured on B200 (profiles/r01_fp64_pipes_microbench.txt): DMMA and DFMA share one 36-37 TFLOP/s
@@ -799,16 +687,7 @@ __device__ __forceinline__ void mbar_wait_consumer(uint64_t *bar, uint32_t parit
 //   G[P][Q] += Y[r0..r0+4, P]^T Y[r0..r0+4, Q]  and loads conflict-free in two wavefronts.
 //   M is padded to NB = ceil(M/8) blocks (rows M..8NB-1 of the tile stay zero).
 // ---------------------------------------------------------------------------------------------
-template <int N> __device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
-template <int N> __device__ __forceinline__ void reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
-
 constexpr int YT_PITCH = 36;
-
-__device__ __forceinline__ void dmma_m8n8k4(double &c0, double &c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
-}
 
 template <int K, class F, bool SEPARABLE>
 __host__ __device__ constexpr bool wsd_paired() { return pm_pays<K>() && F::separable && !SEPARABLE; }
@@ -1142,66 +1021,32 @@ fused_wsd_kernel(SourceDev src, FusedConst<K> fc, F f, uint64_t i_begin, uint64_
 
     if (warp >= WS_S) {
         // ------------------------------------ E-warp ------------------------------------
-#ifdef VS_SETMAXNREG
-        if constexpr (EPS == 2) reg_inc<192>();          // 12 warps: S warpgroup 112, E warpgroups 192 registers per thread
-#endif
         const int e = warp - WS_S;
         const double shift = shift_sh;
         const uint64_t basehi = table_basehi(terms);
         const uint64_t cnt = count_of(e);
         uint64_t bt = first_batch(e);
-        // Phase alternation between the two E-warp teams (team = e / WS_S; every sub-partition has one warp of each).
-        // Generation is bound by the SM-wide shared-memory pipe (random 8-byte table lookups cost 3-5 wavefronts
-        // each), evaluation by the per-sub-partition FP64 pipe.  Left alone, the E-warps drift into lock-step --
-        // a warp that generates while the others evaluate finds the LSU free, finishes early and catches up -- and
-        // then the two phases add up (clock stamps: 12.6k + 10.5k cycles per batch).  A named barrier over the E-warps
-        // after every phase pins team 0 to "generate" while team 1 "evaluates" and vice versa.
-        // (a barrier-pinned generate/evaluate/evaluate rotation of the three E-warps was measured at 6.08 ms vs 5.23 and removed)
-        const bool alternate = (EPS == 2) && fc.alternate;
-        auto ebar = [&]() { asm volatile("bar.sync 1, %0;" ::"n"(WS_E * 32) : "memory"); };
-        const int team = e / WS_S;
-        const uint64_t bars_total = 2 * count_of(0) + 1;              // count_of(0) is the largest batch count in the CTA
-        uint64_t bars_done = 0;
-        if (alternate && team == 1) { ebar(); ++bars_done; }
         for (uint64_t it = 0; it < cnt; ++it, bt += G) {
             const int slot = (int)(it % NBUF);
             double a[K], b[K];
-            bool valid = bt * 32 + lane < rows;
             const bool tr_on = fc.trace && blockIdx.x == 0 && lane == 0 && it < 64;
             long long *trp = fc.trace + ((size_t)warp * 64 + (it < 64 ? it : 0)) * 4;
             if (tr_on) trp[0] = clock64();
-            if (fc.debug & 1) {
-#pragma unroll
-                for (int d = 0; d < K; ++d) { a[d] = 0.25 + 1e-3 * lane + 1e-9 * (double)bt; b[d] = 0.75 - 1e-3 * lane; }
-            } else {
-                valid = gen_rows<K, IB>(src, fc, terms, basehi, i_begin, rows, bt, lane, [&](int d, double xa, double xb) {
-                    a[d] = xa;
-                    b[d] = xb;
-                });
-            }
+            const bool valid = gen_rows<K, IB>(src, fc, basehi, i_begin, rows, bt, lane, [&](int d, double xa, double xb) {
+                a[d] = xa;
+                b[d] = xb;
+            });
             if (tr_on) trp[1] = clock64();
-            if (alternate) { ebar(); ++bars_done; }
-            mbar_wait(empty_bar(e, slot), (uint32_t)(((it / NBUF) & 1) ^ 1));
+            mbar_wait(empty_bar(e, slot), (uint32_t)(((it / NBUF) & 1) ^ 1), MBAR_HINT_NS);
             if (tr_on) trp[2] = clock64();
             double *Y = tiles + ((size_t)e * NBUF + slot) * TILE;
-            if (fc.debug & 2) {
-#pragma unroll
-                for (int d = 0; d < K; ++d) { Y[lane + (2 + d) * YT_PITCH] = a[d]; Y[lane + (2 + K + d) * YT_PITCH] = b[d]; }
-            } else {
-                eval_rows<K, F, SEPARABLE, PM>(f, tokp, a, b, valid, Y + lane, shift, sA, qA, sB, qB, YT_PITCH);
-            }
+            eval_rows<K, F, SEPARABLE, PM>(f, tokp, a, b, valid, Y + lane, shift, sA, qA, sB, qB, YT_PITCH);
             __syncwarp();
             if (tr_on) trp[3] = clock64();
             if (lane == 0) mbar_arrive(full_bar(e, slot));
-            if (alternate) { ebar(); ++bars_done; }
         }
-        if (alternate)
-            for (; bars_done < bars_total; ++bars_done) ebar();       // keep the other team's barriers matched
     } else {
         // ------------------------------------ S-warp ------------------------------------
-#ifdef VS_SETMAXNREG
-        if constexpr (EPS == 2) reg_dec<112>();
-#endif
         uint64_t cn[EPS], cmax = 0;
 #pragma unroll
         for (int h = 0; h < EPS; ++h) {
@@ -1219,7 +1064,7 @@ fused_wsd_kernel(SourceDev src, FusedConst<K> fc, F f, uint64_t i_begin, uint64_
                 const bool tr_on = fc.trace && blockIdx.x == 0 && lane == 0 && it < 32;
                 long long *trp = fc.trace + ((size_t)warp * 64 + (it < 32 ? it * EPS + h : 0)) * 4;
                 if (tr_on) trp[0] = clock64();
-                mbar_wait_consumer(full_bar(e, slot), par);
+                mbar_wait(full_bar(e, slot), par, MBAR_HINT_NS);
                 if (tr_on) trp[1] = clock64();
                 const double *Y = tiles + ((size_t)e * NBUF + slot) * TILE + foff;
 #pragma unroll 2
@@ -1487,7 +1332,6 @@ static int launch_fused_t(vs_ctx *c, const SourceDev &src, const FusedConst<K> &
 template <int K>
 static int fill_const(vs_ctx *c, const SourceDev &src, const ScaleDev &s, FusedConst<K> &fc) {
     fc.scale_kind = s.kind;
-    fc.debug = c->opt.debug_skip;
     const double *h = s.host;                                   // lb | wr
     for (int d = 0; d < K; ++d) {
         fc.lb[d] = s.kind != VS_SCALE_IDENTITY ? h[d] : 0.0;
@@ -1499,7 +1343,6 @@ static int fill_const(vs_ctx *c, const SourceDev &src, const ScaleDev &s, FusedC
     fc.small_index = 0;
     fc.poll_perm = 0;
     fc.trace = nullptr;
-    fc.alternate = c->opt.alternate;
     for (int u = 0; u < FusedConst<K>::AR_N; ++u)
         for (int j = 0; j < AR_J; ++j) { fc.arh[u][j] = 0.0; fc.arl[u][j] = 0.0; }
     if (!c->opt.trace.empty()) {

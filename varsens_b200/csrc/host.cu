@@ -64,20 +64,16 @@ void load_options(Options &o) {
     o = Options();
     o.fused_variant = env_int("VS_FUSED_VARIANT", 0);
     o.no_pipeline = env_int("VS_NO_PIPELINE", 0);
-    o.alternate = env_int("VS_ALTERNATE", 0);
-    o.debug_skip = env_int("VS_DEBUG_SKIP", 0);
     if (const char *t = getenv("VS_TRACE")) o.trace = t;
     o.gram_mma = env_int("VS_GRAM_MMA", -1);
     o.gram_mma_gen = env_int("VS_GRAM_GEN", -1);
     o.export_slow_gen = env_int("VS_EXPORT_SLOW_GEN", 0);
     o.export_copies = env_int("VS_EXPORT_COPIES", 0);
-    o.export_smem_kb = env_int("VS_EXPORT_SMEM_KB", 0);
     o.gram_st = env_int("VS_GRAM_ST", 0);
     o.gram_warps = env_int("VS_GRAM_WARPS", 0);
     o.pf_rows = env_int("VS_PF_ROWS", 0);
     o.gram_rc = env_int("VS_GRAM_RC", 0);
     o.gram_stages = env_int("VS_GRAM_STAGES", 0);
-    o.gram_hint = env_int("VS_GRAM_HINT", 0x989680);
     o.gram_debug = env_int("VS_GRAM_DEBUG", 0);
     o.p2p_timeout_ms = env_int("VS_P2P_TIMEOUT_MS", 10000);
     o.halton_mode = env_int("VS_HALTON_MODE", 0);

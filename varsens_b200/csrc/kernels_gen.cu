@@ -185,29 +185,10 @@ __device__ __forceinline__ void ex_stamp(const ExportGeom &g, uint64_t it, int s
 }
 
 #ifndef EX_WAIT_HINT_NS
-#define EX_WAIT_HINT_NS 500u
+#define EX_WAIT_HINT_NS 500u   // short suspend hint of the mbarrier waits: the hand-over latency is on the tile's critical path
 #endif
-__device__ __forceinline__ uint32_t ex_smem(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void ex_bar_init(uint64_t *b, uint32_t n) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(ex_smem(b)), "r"(n) : "memory");
-}
-__device__ __forceinline__ void ex_bar_arrive(uint64_t *b) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(ex_smem(b)) : "memory");
-}
-__device__ __forceinline__ void ex_bar_wait(uint64_t *b, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "W_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-        "@p bra D_%=;\n"
-        "bra W_%=;\n"
-        "D_%=:\n"
-        "}\n" ::"r"(ex_smem(b)), "r"(parity), "r"(EX_WAIT_HINT_NS)      // short suspend hint: the hand-over latency is on the tile's critical path
-        : "memory");
-}
 __device__ __forceinline__ void ex_bulk_store(double *dst, const double *src_smem, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(ex_smem(src_smem)), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(src_smem)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void ex_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void ex_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
@@ -236,14 +217,14 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
     unsigned char *uwarp = reinterpret_cast<unsigned char *>(sarl + (size_t)k * EX_AR_J);   // [warp][HL_MAXQ]: the units of every generator warp
     double *table = sarl + (size_t)k * EX_AR_J + HL_LIST_BYTES / 8;
     double *tiles = table + ((g.table_len + 1) & ~1u);
-    const uint32_t table_saddr = ex_smem(table);
+    const uint32_t table_saddr = smem_u32(table);
     const size_t tile = (size_t)TI * k;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     if (tid == 0) {
-        ex_bar_init(bars + 0, EX_GEN / 32);
-        ex_bar_init(bars + 1, EX_GEN / 32);
-        ex_bar_init(bars + 2, (uint32_t)NC);                   // every store warp releases the buffer pair
-        ex_bar_init(bars + 3, (uint32_t)NC);
+        mbar_init(bars + 0, EX_GEN / 32);
+        mbar_init(bars + 1, EX_GEN / 32);
+        mbar_init(bars + 2, (uint32_t)NC);                   // every store warp releases the buffer pair
+        mbar_init(bars + 3, (uint32_t)NC);
     }
     if (!src.raw) {
         for (int d = tid; d < k; d += EX_THREADS) {
@@ -284,7 +265,7 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
             if (gw == 1) ex_stamp(g, it, 0, lane);
             const uint64_t pi = src.perm[i];
             if (gw == 1 && pi != ~0ull) ex_stamp(g, it, 1, lane);                        // (the compare makes the stamp wait for the load)
-            ex_bar_wait(bars + 2 + pb, (uint32_t)(((it >> 1) & 1) ^ 1));                 // the store warp is done with this buffer pair
+            mbar_wait(bars + 2 + pb, (uint32_t)(((it >> 1) & 1) ^ 1), EX_WAIT_HINT_NS);   // the store warp is done with this buffer pair
             if (gw == 1) ex_stamp(g, it, 2, lane);
             auto emit = [&](int d, double pa, double pbv) {
                 if (s.kind == VS_SCALE_LINEAR) { pa = __dadd_rn(__dmul_rn(pa, swr[d]), slb[d]); pbv = __dadd_rn(__dmul_rn(pbv, swr[d]), slb[d]); }
@@ -356,7 +337,7 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
             if (gw == 1) ex_stamp(g, it, 3, lane);
             ex_fence_async();                                   // my tile entries must be visible to the TMA (async proxy)
             __syncwarp();
-            if (lane == 0) ex_bar_arrive(bars + pb);
+            if (lane == 0) mbar_arrive(bars + pb);
             if (gw == 1) ex_stamp(g, it, 4, lane);
         }
         return;
@@ -375,7 +356,7 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
         const uint64_t i0 = g.i_lo + (blockIdx.x + it * gridDim.x) * (uint64_t)TI;
         const int rows = (int)((i0 + TI <= g.i_hi) ? TI : (g.i_hi - i0));
         double *A = tiles + (size_t)(2 * NC * pb + 2 * sw) * tile, *B = A + tile;        // this warp's copy
-        ex_bar_wait(bars + pb, (uint32_t)((it >> 1) & 1));
+        mbar_wait(bars + pb, (uint32_t)((it >> 1) & 1), EX_WAIT_HINT_NS);
         if (sw == 0) ex_stamp(g, it, 5, lane);
         // blocks [t_min, t_max] of this tile intersect the window (R0(t) = t n + i0 is monotonic in t).  With the window ends
         // split on the host into (block, row) = (qb, rb) and (qe, re) no division is needed: block t covers the tile's rows
@@ -457,7 +438,7 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
         if (sw == 0) ex_stamp(g, it, 6, lane);
         if (lane == 0) ex_wait_read<0>();                       // this warp's tile buffers may be overwritten by the generators now
         __syncwarp();
-        if (lane == 0) ex_bar_arrive(bars + 2 + pb);
+        if (lane == 0) mbar_arrive(bars + 2 + pb);
         if (sw == 0) ex_stamp(g, it, 7, lane);
     }
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // all bulk stores complete before the CTA exits
@@ -521,7 +502,6 @@ static int launch_sample_flat_bulk(vs_ctx *c, int k, const SourceDev &src, const
     g.table_len = with_table ? (uint32_t)tab_terms : 0;
     g.ntiles = (i_hi - i_lo + TI - 1) / TI;
     size_t smem = fixed + (with_table ? tab : 0) + 4 * (size_t)copies * TI * k * 8;
-    if (c->opt.export_smem_kb > 0 && smem < (size_t)c->opt.export_smem_kb * 1024) smem = (size_t)c->opt.export_smem_kb * 1024;   // VS_EXPORT_SMEM_KB
     if (smem > avail) smem = avail;
     static size_t smem_set[64] = {};
     if (c->device >= 64 || smem_set[c->device] < smem) {

@@ -47,36 +47,13 @@ struct MmaGeom {
     int sumu;              // position of super-tile (0,0) in the list: its warps also accumulate the shifted sums
     unsigned char witem[32];   // consumer warp -> work item (super-tile of this pass * rs + row subset), 255 = idle
     unsigned char ui[128], uj[128];   // super-tile list, heaviest first
-    int hint;              // try_wait suspend-time hint, ns
     int debug;             // elimination experiments (VS_GRAM_DEBUG): 1 = no Gram update, 2 = no copies
 };
 
-__device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void bar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void bar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_addr(bar)) : "memory");
-}
-__device__ __forceinline__ void bar_arrive_expect(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bar_wait(uint64_t *bar, uint32_t parity, uint32_t hint) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_addr(bar)), "r"(parity), "r"(hint)
-        : "memory");
-}
 // global -> shared bulk copy (16-byte aligned on both sides, size a multiple of 16), completion counted on `bar`
 __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_addr(dst)),
-                 "l"(src), "r"(bytes), "r"(smem_addr(bar))
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst)),
+                 "l"(src), "r"(bytes), "r"(smem_u32(bar))
                  : "memory");
 }
 __device__ __forceinline__ bool elect_one() {
@@ -89,11 +66,6 @@ __device__ __forceinline__ bool elect_one() {
         "}\n"
         : "=r"(pred));
     return pred != 0;
-}
-__device__ __forceinline__ void dmma(double &c0, double &c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1)
-                 : "d"(a), "d"(b));
 }
 
 
@@ -155,7 +127,7 @@ __device__ __forceinline__ void mma_steps(double (&acc)[ST * ST][2], double (&sS
         for (int x = 0; x < ST; ++x)
 #pragma unroll
             for (int y = DIAG ? x : 0; y < ST; ++y)
-                if (!GUARD || (x < xmax && y < ymax)) dmma(acc[x * ST + y][0], acc[x * ST + y][1], fa[x], fb[y]);
+                if (!GUARD || (x < xmax && y < ymax)) dmma_m8n8k4(acc[x * ST + y][0], acc[x * ST + y][1], fa[x], fb[y]);
     }
 }
 
@@ -181,8 +153,8 @@ gram_mma_kernel(MmaGeom g, uint64_t rows, const double *__restrict__ fvals, cons
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < g.nstage; ++s) {
-            bar_init(full + s, 1);
-            bar_init(empty + s, (uint32_t)W);
+            mbar_init(full + s, 1);
+            mbar_init(empty + s, (uint32_t)W);
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -220,18 +192,18 @@ gram_mma_kernel(MmaGeom g, uint64_t rows, const double *__restrict__ fvals, cons
         uint32_t par = 0;
         uint32_t ch = blockIdx.x;
         for (uint32_t c = 0; c < cnt; ++c, ch += gridDim.x) {
-            bar_wait(empty + s, par ^ 1u, (uint32_t)g.hint);
+            mbar_wait(empty + s, par ^ 1u, MBAR_HINT_NS);
             const uint64_t r0 = (uint64_t)ch * g.rc;
             const uint32_t valid = ch + 1 == nchunks ? (uint32_t)last_valid : (uint32_t)g.rc;
             // One elected lane issues every copy from a warp-uniform loop: the operands stay in uniform registers.  (A
             // lane-strided loop compiles to an ELECT + 5x R2UR + UBLKCP round per lane, ~100 cycles per copy, and the
             // producer became the bottleneck: 0.89 ms instead of the 0.3 ms FP64 bound at k = 20, n = 2^22.)
             if (g.debug == 2) {
-                if (lane == 0) bar_arrive(full + s);
+                if (lane == 0) mbar_arrive(full + s);
             } else if (elect_one()) {
                 double *dst = stages + (size_t)s * stage_elems;
                 if constexpr (!GEN) {
-                    bar_arrive_expect(full + s, (uint32_t)g.m * valid * 8u);
+                    mbar_arrive_expect_tx(full + s, (uint32_t)g.m * valid * 8u);
                     const double *src = fvals + r0;
 #pragma unroll 4
                     for (int t = 0; t < g.m; ++t) bulk_g2s(dst + (size_t)t * g.pitch, src + (uint64_t)t * rows, valid * 8u, full + s);
@@ -240,7 +212,7 @@ gram_mma_kernel(MmaGeom g, uint64_t rows, const double *__restrict__ fvals, cons
                     // blocks too unless rows*l is odd -- then they start one element early.  Sizes rounded up to 16 bytes.
                     const uint32_t nel = valid * (uint32_t)g.l;
                     const uint32_t be = ((nel + 1u) & ~1u) * 8u, bo = ((nel + (uint32_t)g.oddrun + 1u) & ~1u) * 8u;
-                    bar_arrive_expect(full + s, (uint32_t)(g.nt / 2) * (be + bo));
+                    mbar_arrive_expect_tx(full + s, (uint32_t)(g.nt / 2) * (be + bo));
                     const double *src = fvals + r0 * (uint64_t)g.l;
                     const uint64_t run = rows * (uint64_t)g.l;
 #pragma unroll 2
@@ -291,7 +263,7 @@ gram_mma_kernel(MmaGeom g, uint64_t rows, const double *__restrict__ fvals, cons
         uint32_t par = 0;
         uint32_t ch = blockIdx.x;
         for (uint32_t c = 0; c < cnt; ++c, ch += gridDim.x) {
-            bar_wait(full + s, par, (uint32_t)g.hint);
+            mbar_wait(full + s, par, MBAR_HINT_NS);
             if (active && g.debug != 1) {
                 const double *Ya = Ya0 + (size_t)s * stage_elems, *Yb = Yb0 + (size_t)s * stage_elems;
                 const bool fullc = ch + 1 != nchunks || last_valid == g.rc;
@@ -311,7 +283,7 @@ gram_mma_kernel(MmaGeom g, uint64_t rows, const double *__restrict__ fvals, cons
                 }
             }
             __syncwarp();
-            if (lane == 0) bar_arrive(empty + s);
+            if (lane == 0) mbar_arrive(empty + s);
             if (++s == g.nstage) { s = 0; par ^= 1u; }
         }
     }
@@ -556,7 +528,6 @@ int launch_gram_mma(vs_ctx *c, int k, int l, uint64_t rows, const double *fvals,
     }
     if (g.nstage < 2) return VS_OK;
     if (c->opt.gram_stages >= 1 && c->opt.gram_stages < g.nstage) g.nstage = c->opt.gram_stages;
-    g.hint = c->opt.gram_hint;
     g.debug = c->opt.gram_debug;
     if (smem < MMA_BAR_DOUBLES * sizeof(double) + tail) smem = MMA_BAR_DOUBLES * sizeof(double) + tail;
     if (smem > avail) return VS_OK;

@@ -115,18 +115,14 @@ struct HaltonCache {
 struct Options {
     int fused_variant = 0;      // VS_FUSED_VARIANT  (0 = default choice per k)
     int no_pipeline = 0;        // VS_NO_PIPELINE    host permutation: one copy, then the launch (no chunk flags)
-    int legacy_launch = 0;      // VS_LEGACY_LAUNCH  fused step as separate shift / fused / scatter / finalize launches
-    int alternate = 0;          // VS_ALTERNATE
-    int debug_skip = 0;         // VS_DEBUG_SKIP
     std::string trace;          // VS_TRACE          file for CTA 0's clock stamps
     int gram_mma = -1;          // VS_GRAM_MMA       (-1 = default)
     int export_slow_gen = 0;    // VS_EXPORT_SLOW_GEN=1: generic digit loop in the bulk export kernel (comparison runs)
-    int export_smem_kb = 0;     // VS_EXPORT_SMEM_KB: request at least this much dynamic shared memory (L1 carve-out experiments)
     int export_copies = 0;      // VS_EXPORT_COPIES=1|2: store warps / tile copies of the bulk export kernel (0: by window shape)
     int gram_mma_gen = -1;      // VS_GRAM_GEN       0: register-tile kernel for l > 1 outputs / odd row counts
     int pf_rows = 0;            // VS_PF_ROWS=64: 64-row tiles (two row groups per lane) in the product-form evaluation kernel (measured slower)
     int gram_warps = 0;         // VS_GRAM_WARPS=15|31: consumer warps of the 2 x 2 super-tile form (0: 31 where that saves a pass)
-    int gram_st = 0, gram_rc = 0, gram_stages = 0, gram_hint = 0x989680, gram_debug = 0;
+    int gram_st = 0, gram_rc = 0, gram_stages = 0, gram_debug = 0;
     int p2p_timeout_ms = 10000; // VS_P2P_TIMEOUT_MS bounded wait for the peers' flags in the exchange
     int halton_mode = 0;        // VS_HALTON_MODE    term-table arithmetic (enum vs_halton_mode)
     int index_bits = 0;         // VS_INDEX_BITS=32 forces the general (32-bit index) fused kernel
