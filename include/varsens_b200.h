@@ -59,8 +59,27 @@ typedef struct vs_scale {
  *   ISHIGAMI   : {A, B}, k >= 3               f = sin x0 + A sin^2 x1 + B x2^4 sin x0
  *   RK4_CHAIN  : {dt, nsteps}, k even         reversible mass-action chain X_0 <-> ... <-> X_{k/2},
  *                forward rates x[0..k/2), reverse rates x[k/2..k), X(0) = e_0, classic RK4,
- *                f = X_{k/2}(nsteps*dt)       (spec frozen in oracle/objectives.py) */
-enum vs_objective { VS_OBJ_GFUNCTION = 0, VS_OBJ_ISHIGAMI = 1, VS_OBJ_RK4_CHAIN = 2 };
+ *                f = X_{k/2}(nsteps*dt)       (spec frozen in oracle/objectives.py)
+ *   MASS_ACTION: a run-time mass-action reaction network integrated by classic fixed-step RK4, L observables
+ *                (l = L outputs per point).  params, indices stored as exact integers, -1 = none / use the constant:
+ *                  [0] S  [1] R  [2] L  [3] dt  [4] nsteps
+ *                  R records of 8:  a0 a1 b0 b1  kf_coord kf_const  kr_coord kr_const
+ *                                   (a = reactants, b = products: species index or -1; kr_coord = -1 with kr_const = 0
+ *                                    is an irreversible reaction, its reverse term is not evaluated)
+ *                  S records of 2:  init_coord init_const
+ *                  L*S weights:     w[o][s]      observable o = sum_s w[o][s] X_s(nsteps*dt), zero weights skipped
+ *                n_params == 5 + 8R + 2S + L*S.  A rate or initial amount is x[coord] (the scaled sample coordinate,
+ *                coord < k) when coord >= 0, else the constant.  Limits: 1 <= S <= 128, 1 <= R <= 512, 1 <= L <= 64,
+ *                dt finite, 0 <= nsteps < 2^31, species indices < S, coordinates < k; anything else is VS_ERR_ARG.
+ *                A network whose per-trajectory state does not fit the kernel's shared memory (k + 3S + R doubles per
+ *                thread, 32 threads at least) is VS_ERR_UNSUPPORTED.  Two-phase route only; VS_FLAG_SEPARABLE is
+ *                VS_ERR_UNSUPPORTED.  Frozen arithmetic (bit-identical to the oracle, and to RK4_CHAIN for the chain
+ *                written as a network) in varsens_b200/csrc/device.cuh: MassAction.
+ *
+ * Every objective has l outputs per point: 1 for the first three, L for MASS_ACTION (vs_objective_outputs).  The entry
+ * points that take an objective write l columns: vs_eval_values rows*(2+2k)*l doubles, vs_fused_partials
+ * vs_partials_len(k, l) doubles, vs_run_fused / vs_run_fused_p2p vs_result arrays sized for l. */
+enum vs_objective { VS_OBJ_GFUNCTION = 0, VS_OBJ_ISHIGAMI = 1, VS_OBJ_RK4_CHAIN = 2, VS_OBJ_MASS_ACTION = 3 };
 
 /* fp64 arithmetic of the Halton radical inverse (the reference delegates it to the third-party ghalton package,
  * varsens/saltelli.py:82-84, whose source is not part of the reference; see DESIGN.md "parity unpinned").  The first three are
@@ -135,6 +154,9 @@ int vs_reference_permutation(uint64_t n, uint32_t seed, uint32_t *perm, uint32_t
  * i.e. exactly the combinations vs_finalize adds up (saltelli.py:612-613, 618-619); vectors from
  * vs_partials_from_values hold the plain entries.  Both kinds add up across shards and ranks. */
 size_t vs_partials_len(int k, int l);
+/* Outputs per point l of a registered objective (1, or L for VS_OBJ_MASS_ACTION) in *l, after the same validation of
+ * k, objective and params the evaluating entry points run (VS_ERR_ARG on a malformed description). */
+int vs_objective_outputs(int k, int objective, const double *params, int n_params, int *l);
 
 /* ---- generators ---------------------------------------------------------------------------- */
 /* ghalton.Halton(k).get() points of 1-based indices first_index .. first_index+count-1, scaled;
@@ -168,7 +190,7 @@ int vs_sample_flat_shard(vs_ctx *ctx, int k, uint64_t n, uint64_t discard, const
 
 /* ---- objective evaluation --------------------------------------------------------------------- */
 /* Objective values of base rows [i_begin,i_end) for a registered functor, sample rows generated on
- * the fly (never stored): fvals[(t*rows + (i-i_begin))], t in [0,2+2k), rows = i_end-i_begin --
+ * the fly (never stored): fvals[(t*rows + (i-i_begin))*l + o], t in [0,2+2k), o in [0,l), rows = i_end-i_begin --
  * for the full range this is Objective.flat().  Replaces varsens/saltelli.py:308-353. */
 int vs_eval_values(vs_ctx *ctx, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
                    const double *raw, int raw_mem, const vs_scale *scale, int objective,

@@ -15,7 +15,7 @@ LIB_PATH = os.environ.get("VS_LIB") or os.path.join(_HERE, "libvarsens_b200.so")
 VS_OK = 0
 MEM_HOST, MEM_DEVICE = 0, 1
 SCALE_IDENTITY, SCALE_LINEAR, SCALE_POWER = 0, 1, 2
-OBJ_GFUNCTION, OBJ_ISHIGAMI, OBJ_RK4_CHAIN = 0, 1, 2
+OBJ_GFUNCTION, OBJ_ISHIGAMI, OBJ_RK4_CHAIN, OBJ_MASS_ACTION = 0, 1, 2, 3
 FLAG_SECOND_ORDER, FLAG_SEPARABLE = 1, 2
 
 # every symbol include/varsens_b200.h declares (tests/test_cabi_symbols.py checks the header against this)
@@ -26,6 +26,7 @@ SYMBOLS = (
     "vs_finalize_device", "vs_allreduce_finalize_p2p", "vs_indices_from_values", "vs_fused_partials", "vs_run_fused", "vs_measure_fp64_peak", "vs_last_kernel_ms",
     "vs_ctx_reload_env", "vs_ctx_set_halton_mode", "vs_halton_terms_mode", "vs_run_fused_p2p", "vs_last_tail_ns",
     "vs_halton_arith_check", "vs_reference_permutation", "vs_ctx_set_timing", "vs_sample_flat_shard",
+    "vs_objective_outputs",
 )
 HALTON_DIVIDE, HALTON_RECIPROCAL, HALTON_RUNNING_RECIPROCAL, HALTON_HORNER = 0, 1, 2, 3
 ERR_TIMEOUT = 6
@@ -97,6 +98,7 @@ def lib():
         L.vs_reference_permutation.argtypes = [u64, ctypes.c_uint32, vp, vp, P(i32)]
         L.vs_measure_fp64_peak.argtypes = [vp, P(ctypes.c_double)]
         L.vs_last_kernel_ms.argtypes = [vp, P(ctypes.c_float)]
+        L.vs_objective_outputs.argtypes = [i32, i32, vp, i32, P(i32)]
         for name in SYMBOLS:
             fn = getattr(L, name)
             if fn.restype is ctypes.c_int and name not in ("vs_abi_version",):
@@ -110,6 +112,17 @@ def check(status):
         err = VarsensError("libvarsens_b200: status %d: %s" % (status, lib().vs_last_error().decode()))
         err.status = status
         raise err
+
+
+def objective_outputs(k, objective, params):
+    """Outputs per point l of a registered objective (vs_objective_outputs: host only, validates the parameters).  Every
+    objective but a mass-action network has one, known without a call."""
+    if int(objective) != OBJ_MASS_ACTION:
+        return 1
+    par = numpy.ascontiguousarray(params, dtype=numpy.float64)
+    l = ctypes.c_int()
+    check(lib().vs_objective_outputs(int(k), int(objective), par.ctypes.data_as(ctypes.c_void_p), int(par.size), ctypes.byref(l)))
+    return int(l.value)
 
 
 def discard_arg(discard):
@@ -352,8 +365,11 @@ class Context(object):
     # ---- objective values / estimators --------------------------------------------------------
     def eval_values(self, k, n, perm, objective, params, discard=0, scale=IDENTITY, raw=None, i_begin=0, i_end=None,
                     out=None):
+        """(2+2k, rows) values, or (2+2k, rows, l) for an objective with l > 1 outputs (fvals[(t*rows + r)*l + o])."""
         i_end = n if i_end is None else i_end
-        out = numpy.empty((2 + 2 * k, int(i_end - i_begin))) if out is None else out
+        l = objective_outputs(k, objective, params)
+        if out is None:
+            out = numpy.empty((2 + 2 * k, int(i_end - i_begin)) + ((l,) if l > 1 else ()))
         par = numpy.ascontiguousarray(params, dtype=numpy.float64)
         sp, keep = scale.c_struct(k)
         pp, pm, pk = buf(perm, numpy.uint32)
@@ -416,7 +432,7 @@ class Context(object):
     def fused_partials(self, k, n, perm, objective, params, discard=0, scale=IDENTITY, raw=None, i_begin=0, i_end=None,
                        flags=FLAG_SECOND_ORDER, out=None):
         i_end = n if i_end is None else i_end
-        plen = int(lib().vs_partials_len(int(k), 1))
+        plen = int(lib().vs_partials_len(int(k), objective_outputs(k, objective, params)))
         out = numpy.empty(plen) if out is None else out
         par = numpy.ascontiguousarray(params, dtype=numpy.float64)
         sp, keep = scale.c_struct(k)
@@ -429,7 +445,7 @@ class Context(object):
         return out
 
     def run_fused(self, k, n, perm, objective, params, discard=0, scale=IDENTITY, raw=None, flags=FLAG_SECOND_ORDER):
-        res = Result(k, 1, bool(flags & FLAG_SECOND_ORDER))
+        res = Result(k, objective_outputs(k, objective, params), bool(flags & FLAG_SECOND_ORDER))
         cs = res.c_struct()
         par = numpy.ascontiguousarray(params, dtype=numpy.float64)
         sp, keep = scale.c_struct(k)
@@ -444,7 +460,7 @@ def _run_fused_p2p(self, k, n, perm, objective, params, world_size, rank, peer_b
                    discard=0, scale=IDENTITY, raw=None, flags=FLAG_SECOND_ORDER):
     """vs_run_fused_p2p: this rank's shard [i_begin,i_end) of the fused step, all-reduce over NVLink peer memory and
     estimators inside the ONE kernel launch; returns the Result (identical bits on every rank)."""
-    res = Result(k, 1, bool(flags & FLAG_SECOND_ORDER))
+    res = Result(k, objective_outputs(k, objective, params), bool(flags & FLAG_SECOND_ORDER))
     cs = res.c_struct()
     par = numpy.ascontiguousarray(params, dtype=numpy.float64)
     sp, keep = scale.c_struct(k)
@@ -479,9 +495,10 @@ class FusedPlan(object):
         pp, pm, pk = buf(perm, numpy.uint32)
         rp, rm, rk = buf(raw, numpy.float64)
         self._keep = (par, keep, pk, rk, sp)
-        self._len = Result.flat_len(self.k, 1) if self.second else 2 + 4 * self.k
-        kk = self.k
-        o = (0, 1, 2, 2 + kk, 2 + 2 * kk, 2 + 3 * kk, 2 + 4 * kk, 2 + 4 * kk + kk * kk)
+        self.l = l = objective_outputs(k, objective, params)
+        kl = self.k * l
+        self._len = Result.flat_len(self.k, l) if self.second else 2 * l + 4 * kl
+        o = (0, l, 2 * l, 2 * l + kl, 2 * l + 2 * kl, 2 * l + 3 * kl, 2 * l + 4 * kl, 2 * l + 4 * kl + kl * kl)
         self._out = []                                   # two output sets: (flat buffer, vs_result struct, byref, Result views)
         for _ in range(2):
             flat = numpy.empty(self._len)
@@ -491,7 +508,7 @@ class FusedPlan(object):
                                base + 8 * o[6], base + 8 * o[7])
             else:
                 cs = vs_result(base, base + 8 * o[1], base + 8 * o[2], base + 8 * o[3], base + 8 * o[4], base + 8 * o[5], None, None)
-            self._out.append((flat, cs, ctypes.byref(cs), Result.views(self.k, 1, flat, self.second)))
+            self._out.append((flat, cs, ctypes.byref(cs), Result.views(self.k, l, flat, self.second)))
         self._turn = 0
         L = lib()
         i_end = n if i_end is None else i_end

@@ -80,6 +80,13 @@ int take_tail_result(vs_ctx *c, int k, int flags, vs_result *r) {
     return VS_OK;
 }
 
+// Outputs per point of `objective`: 1 for every objective but a mass-action network, whose description is validated here.
+int outputs_of(int k, int objective, const double *params, int n_params, int *l) {
+    *l = 1;
+    if (objective != VS_OBJ_MASS_ACTION) return VS_OK;
+    return objective_host(k, objective, params, n_params, nullptr, l);
+}
+
 }  // namespace
 
 extern "C" int vs_halton(vs_ctx *c, int k, uint64_t first_index, uint64_t count, const vs_scale *scale, double *out,
@@ -173,7 +180,7 @@ extern "C" int vs_eval_values(vs_ctx *c, int k, uint64_t n, uint64_t discard, co
     VS_TRY(get_scale(c, k, scale, &s));
     ObjectiveDev od;
     VS_TRY(get_objective(c, k, objective, params, n_params, &od));
-    OutStage o{c, fvals, fvals_mem, (i_end - i_begin) * (uint64_t)(2 + 2 * k) * sizeof(double)};
+    OutStage o{c, fvals, fvals_mem, (i_end - i_begin) * (uint64_t)(2 + 2 * k) * od.l * sizeof(double)};
     VS_TRY(o.begin(c->io_buf));
     VS_TRY(launch_eval_values(c, k, src, s, od, i_begin, i_end, (double *)o.dev));
     VS_TRY(o.end());
@@ -331,12 +338,13 @@ static int fused_step(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint
     VS_REQUIRE(!(flags & VS_FLAG_SEPARABLE), VS_ERR_UNSUPPORTED, "VS_FLAG_SEPARABLE needs a fused kernel (objective %d, k=%d)",
                objective, k);
     VS_REQUIRE(partials_dev, VS_ERR_ARG, "two-phase path needs a partial-sum buffer");
-    VS_TRY(ensure(c, c->io_buf, rows * (uint64_t)(2 + 2 * k) * sizeof(double)));
+    const int l = od.l;                              // values laid out fvals[(t*rows + r)*l + o]
+    VS_TRY(ensure(c, c->io_buf, rows * (uint64_t)(2 + 2 * k) * l * sizeof(double)));
     VS_TRY(launch_eval_values(c, k, src, s, od, i_begin, i_end, (double *)c->io_buf.p));
-    // common shift f(M_1[0]) must not depend on the shard: evaluate base row 0 separately
-    VS_TRY(ensure(c, c->misc_buf, (size_t)(64 + 2 + 2 * k) * sizeof(double)));
+    // common shift: the l values of f(M_1[0]), which must not depend on the shard: evaluate base row 0 separately
+    VS_TRY(ensure(c, c->misc_buf, (size_t)(64 + (2 + 2 * k) * l) * sizeof(double)));
     if (i_begin == 0) {
-        VS_CUDA(cudaMemcpyAsync(c->misc_buf.p, c->io_buf.p, sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+        VS_CUDA(cudaMemcpyAsync(c->misc_buf.p, c->io_buf.p, l * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
     } else {
         SourceDev src0 = src;
         if (perm_mem == VS_MEM_HOST) {   // row 0's permutation entry is outside the staged slice
@@ -346,9 +354,9 @@ static int fused_step(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint
         }
         double *tmp = (double *)c->misc_buf.p + 64;
         VS_TRY(launch_eval_values(c, k, src0, s, od, 0, 1, tmp));
-        VS_CUDA(cudaMemcpyAsync(c->misc_buf.p, tmp, sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+        VS_CUDA(cudaMemcpyAsync(c->misc_buf.p, tmp, l * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
     }
-    return launch_partials_from_values(c, k, 1, rows, (const double *)c->io_buf.p, (const double *)c->misc_buf.p, flags,
+    return launch_partials_from_values(c, k, l, rows, (const double *)c->io_buf.p, (const double *)c->misc_buf.p, flags,
                                        partials_dev);
 }
 
@@ -357,7 +365,9 @@ extern "C" int vs_fused_partials(vs_ctx *c, int k, uint64_t n, uint64_t discard,
                                  int n_params, uint64_t i_begin, uint64_t i_end, int flags, double *partials, int partials_mem) {
     VS_TRY(check_common(c, k));
     VS_REQUIRE(n >= 2 && i_begin <= i_end && i_end <= n && partials, VS_ERR_ARG, "bad arguments");
-    size_t plen = vs_partials_len(k, 1);
+    int l = 1;
+    VS_TRY(outputs_of(k, objective, params, n_params, &l));
+    size_t plen = vs_partials_len(k, l);
     OutStage o{c, partials, partials_mem, plen * sizeof(double)};
     VS_TRY(o.begin(c->part_buf));
     if (i_begin == i_end) {
@@ -381,7 +391,9 @@ extern "C" int vs_run_fused(vs_ctx *c, int k, uint64_t n, uint64_t discard, cons
                             int n_params, int flags, vs_result *result) {
     VS_TRY(check_common(c, k));
     VS_REQUIRE(n >= 2 && result, VS_ERR_ARG, "bad arguments");
-    VS_TRY(ensure(c, c->part_buf, vs_partials_len(k, 1) * sizeof(double)));
+    int l = 1;
+    VS_TRY(outputs_of(k, objective, params, n_params, &l));
+    VS_TRY(ensure(c, c->part_buf, vs_partials_len(k, l) * sizeof(double)));
     FusedReq req;
     req.mode = 1;
     req.n_total = req.rows_total = n;
@@ -389,7 +401,7 @@ extern "C" int vs_run_fused(vs_ctx *c, int k, uint64_t n, uint64_t discard, cons
     VS_TRY(fused_step(c, k, n, discard, perm, perm_mem, raw, raw_mem, scale, objective, params, n_params, 0, n, flags,
                       (double *)c->part_buf.p, &req, &finalized));
     if (finalized) return take_tail_result(c, k, flags, result);
-    return finalize_to_host(c, k, 1, n, n, (const double *)c->part_buf.p, flags, result);
+    return finalize_to_host(c, k, l, n, n, (const double *)c->part_buf.p, flags, result);
 }
 
 extern "C" int vs_run_fused_p2p(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
@@ -409,8 +421,10 @@ extern "C" int vs_run_fused_p2p(vs_ctx *c, int k, uint64_t n, uint64_t discard, 
         c->peer_tab = want;
         VS_CUDA(cudaMemcpyAsync(tab, c->peer_tab.data(), 128 * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
     }
-    VS_TRY(ensure(c, c->part_buf, 2 * vs_partials_len(k, 1) * sizeof(double)));
-    double *mine = (double *)c->part_buf.p + vs_partials_len(k, 1);       // [0, plen) is the scratch of the stand-alone exchange kernel
+    int l = 1;
+    VS_TRY(outputs_of(k, objective, params, n_params, &l));
+    VS_TRY(ensure(c, c->part_buf, 2 * vs_partials_len(k, l) * sizeof(double)));
+    double *mine = (double *)c->part_buf.p + vs_partials_len(k, l);       // [0, plen) is the scratch of the stand-alone exchange kernel
     FusedReq req;
     req.mode = 2;
     req.n_total = req.rows_total = n;
@@ -424,13 +438,13 @@ extern "C" int vs_run_fused_p2p(vs_ctx *c, int k, uint64_t n, uint64_t discard, 
                       mine, &req, &finalized));
     if (finalized) return take_tail_result(c, k, flags, result);
     // kernels without the in-kernel tail (two-phase path, legacy variants): exchange + estimators in the stand-alone kernel
-    VS_TRY(ensure_host_res(c, result_len(k, 1) + HOST_RES_EXTRA));
-    c->host_res[result_len(k, 1)] = 0.0;
-    VS_TRY(launch_p2p_reduce_finalize(c, k, 1, n, n, world_size, rank, tab, tab + 64, epoch, mine, flags, c->host_res));
+    VS_TRY(ensure_host_res(c, result_len(k, l) + HOST_RES_EXTRA));
+    c->host_res[result_len(k, l)] = 0.0;
+    VS_TRY(launch_p2p_reduce_finalize(c, k, l, n, n, world_size, rank, tab, tab + 64, epoch, mine, flags, c->host_res));
     VS_CUDA(cudaStreamSynchronize(c->stream));
-    VS_REQUIRE(c->host_res[result_len(k, 1)] == 0.0, VS_ERR_TIMEOUT,
+    VS_REQUIRE(c->host_res[result_len(k, l)] == 0.0, VS_ERR_TIMEOUT,
                "peer-memory all-reduce: a rank did not publish its partial sums within %d ms", c->opt.p2p_timeout_ms);
-    unpack_result(c->host_res, k, 1, flags, result);
+    unpack_result(c->host_res, k, l, flags, result);
     return VS_OK;
 }
 

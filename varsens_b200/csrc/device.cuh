@@ -455,6 +455,18 @@ struct RK4ChainDyn {
     }
 };
 
+// MassAction (VS_OBJ_MASS_ACTION, a run-time network; kernel in kernels_network.cu).  FROZEN ARITHMETIC, restated by the
+// oracle (oracle/mass_action.c: f_mass_action) so trajectories are bit-identical given bit-identical rates and initial amounts:
+//   P      = 1.0 (no species on the side), X[s0] (one), __dmul_rn(X[s0], X[s1]) (two)      Pf over reactants, Pr over products
+//   flux_r = fma(kf, Pf, -__dmul_rn(kr, Pr))   reversible;   __dmul_rn(kf, Pf)   irreversible (reverse term not evaluated)
+//   d_s    = 0.0, then over the reactions with net coefficient c != 0 for s (products - reactants; a catalyst nets to 0),
+//            ascending:  c = +1: __dadd_rn(d, flux)   c = -1: __dsub_rn(d, flux)   |c| = 2: fma(c, flux, d)
+//   stages and update exactly RK4Chain's (h2 = 0.5*dt, h6 = dt/6, T = fma(h, d, X), a = k1, a = fma(2, k2, a),
+//            a = fma(2, k3, a), X = fma(h6, __dadd_rn(a, k4), X))
+//   observable o: acc = 0.0, acc = fma(w[o][s], X_s, acc) over the nonzero weights, ascending s.
+// The chain written as a network (X_s <-> X_{s+1}, kf = x[s], kr = x[S+s], X(0) = e_0, observable X_S) therefore yields the
+// same bits as RK4Chain<S> and RK4ChainDyn.
+
 __host__ __device__ __forceinline__ void tile_coords(int id, int nt, int &tr, int &tc) {
     tr = 0;
     int rowlen = nt;

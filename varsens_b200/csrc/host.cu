@@ -305,8 +305,10 @@ int get_scale(vs_ctx *c, int k, const vs_scale *s, ScaleDev *out) {
     return VS_OK;
 }
 
-int get_objective(vs_ctx *c, int k, int objective, const double *params, int n_params, ObjectiveDev *out) {
-    std::vector<double> h;
+int objective_host(int k, int objective, const double *params, int n_params, std::vector<double> *hp, int *l) {
+    std::vector<double> scratch;
+    std::vector<double> &h = hp ? *hp : scratch;
+    *l = 1;
     switch (objective) {
     case VS_OBJ_GFUNCTION:
         VS_REQUIRE(params && n_params == k, VS_ERR_ARG, "g-function needs k=%d parameters a_c, got %d", k, n_params);
@@ -328,10 +330,19 @@ int get_objective(vs_ctx *c, int k, int objective, const double *params, int n_p
         VS_REQUIRE(params && n_params == 2 && params[1] >= 0, VS_ERR_ARG, "RK4 chain needs parameters {dt, nsteps}");
         h.assign(params, params + 2);
         break;
+    case VS_OBJ_MASS_ACTION:
+        return network_describe(k, params, n_params, hp, l);
     default:
         set_error("unknown objective id %d", objective);
         return VS_ERR_ARG;
     }
+    return VS_OK;
+}
+
+int get_objective(vs_ctx *c, int k, int objective, const double *params, int n_params, ObjectiveDev *out) {
+    std::vector<double> h;
+    int l = 1;
+    VS_TRY(objective_host(k, objective, params, n_params, &h, &l));
     if (!(c->obj_id_cached == objective && c->obj_host == h && c->obj_buf.p)) {
         VS_CUDA(cudaStreamSynchronize(c->stream));   // a kernel in flight may still read the old parameters
         c->obj_host = h;
@@ -340,6 +351,7 @@ int get_objective(vs_ctx *c, int k, int objective, const double *params, int n_p
         c->obj_id_cached = objective;
     }
     out->id = objective;
+    out->l = l;
     out->params = (const double *)c->obj_buf.p;
     out->n_params = (int)h.size();
     out->host = c->obj_host.data();
@@ -383,6 +395,12 @@ int make_source(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *
 using namespace vs;
 
 extern "C" int vs_abi_version(void) { return VS_ABI_VERSION; }
+
+extern "C" int vs_objective_outputs(int k, int objective, const double *params, int n_params, int *l) {
+    VS_REQUIRE(l, VS_ERR_ARG, "l is NULL");
+    VS_REQUIRE(k >= 1 && k <= 4096, VS_ERR_ARG, "k=%d out of range [1,4096]", k);
+    return objective_host(k, objective, params, n_params, nullptr, l);
+}
 
 extern "C" const char *vs_last_error(void) { return g_err; }
 

@@ -337,6 +337,8 @@ int launch_eval_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s
         }
         }
     }
+    case VS_OBJ_MASS_ACTION:
+        return launch_network_values(c, k, src, s, o, i_begin, i_end, fvals);
     }
     set_error("unknown objective id %d", o.id);
     return VS_ERR_ARG;

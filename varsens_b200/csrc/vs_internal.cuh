@@ -89,6 +89,7 @@ struct ObjectiveDev {
     const double *params;   // device copy of the host params (plus derived values, see device.cuh)
     int n_params;
     const double *host;     // the same values on the host (lives in the ctx)
+    int l = 1;              // outputs per point (L of a mass-action network)
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -177,6 +178,9 @@ int ensure(vs_ctx *c, DevBuf &b, size_t bytes);
 int get_halton(vs_ctx *c, int k, uint64_t max_index, HaltonDev *out);
 int get_scale(vs_ctx *c, int k, const vs_scale *s, ScaleDev *out);
 int get_objective(vs_ctx *c, int k, int objective, const double *params, int n_params, ObjectiveDev *out);
+// Validation of (k, objective, params) without a ctx: the outputs per point in *l and, if h != nullptr, the parameter block
+// get_objective uploads (host.cu).
+int objective_host(int k, int objective, const double *params, int n_params, std::vector<double> *h, int *l);
 // Returns a device pointer for an input buffer (staging a host buffer through `scratch`).
 int stage_in(vs_ctx *c, DevBuf &scratch, const void *p, int mem, size_t bytes, const void **dev);
 int make_source(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
@@ -205,6 +209,11 @@ int launch_gram_scatter(vs_ctx *c, const GramGeom &g, int nblocks, const double 
 // kernels_gram_mma.cu: tensor-path Gram (*handled = false -> caller falls back to gram_kernel)
 int launch_gram_mma(vs_ctx *c, int k, int l, uint64_t rows, const double *fvals, const double *shift_dev, int flags,
                     double *partials, bool *handled);
+// kernels_network.cu: VS_OBJ_MASS_ACTION
+int network_describe(int k, const double *params, int n_params, std::vector<double> *h, int *l);
+int network_check_fit(vs_ctx *c, int k, const ObjectiveDev &o);       // VS_ERR_UNSUPPORTED if the state does not fit
+int launch_network_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, const ObjectiveDev &o, uint64_t i_begin,
+                          uint64_t i_end, double *fvals);
 // kernels_fused.cu
 bool fused_supported(int k, int objective, int flags);
 // true if the kernel chosen for (k, objective, flags) runs the whole step in ONE launch (FusedReq modes 1/2, chunk flags)

@@ -5,6 +5,8 @@ scale-out mechanism is file batching (varsens/saltelli.py:173-193 -> cluster/acc
 every rank writes its own contiguous window of flat rows."""
 import os
 
+from ._cabi import objective_outputs
+
 
 def world():
     """(rank, world_size) of the initialised torch.distributed process group, else (0, 1).
@@ -104,22 +106,32 @@ def use_nccl():
     return os.environ.get("VS_NCCL", "0") == "1"
 
 
+def outputs_of_partials(k, length):
+    """The outputs per point l whose partial-sum vector for k factors has `length` entries."""
+    for l in range(1, 65):
+        if partials_layout(k, l)["length"] == int(length):
+            return l
+    raise ValueError("%d is not a partial-sum length for k = %d" % (length, k))
+
+
 def reduce_and_finalize(ctx, k, n, part, flags):
-    """Sum a rank's partial-sum tensor over the group and compute the indices (every rank returns the same Result).
+    """Sum a rank's partial-sum tensor over the group and compute the indices (every rank returns the same Result; the
+    outputs per point l follow from the tensor's length).
     Default: the stand-alone peer-memory exchange kernel (vs_allreduce_finalize_p2p) over torch symmetric memory; with
     VS_NCCL=1, or when symmetric memory is unavailable: one NCCL all_reduce followed by vs_finalize.  The collective runs
     on torch's current stream, so the ctx is switched onto that stream for the call: the kernel that produced `part`,
     the all-reduce and the finalisation are then ordered by the stream itself."""
     import torch
     rank, ws = world()
+    l = outputs_of_partials(k, part.numel())
     if ws == 1:
-        return ctx.finalize(k, 1, n, part, flags)
+        return ctx.finalize(k, l, n, part, flags)
     ex = None if use_nccl() else peer_exchange(part.numel(), part.device)
     with on_torch_stream(ctx, part.device):
         if ex is not None:
-            return ctx.allreduce_finalize_p2p(k, 1, n, ex.world, ex.rank, ex.peer_bufs, ex.peer_flags, ex.next_epoch(), part, flags)
+            return ctx.allreduce_finalize_p2p(k, l, n, ex.world, ex.rank, ex.peer_bufs, ex.peer_flags, ex.next_epoch(), part, flags)
         allreduce_partials(part)
-        return ctx.finalize(k, 1, n, part, flags)
+        return ctx.finalize(k, l, n, part, flags)
 
 
 class on_torch_stream(object):
@@ -153,7 +165,8 @@ def fused_step(ctx, k, n, perm, objective, params, discard, scale, raw, flags):
         return ctx.run_fused(k, n, perm, objective, params, discard, scale, raw, flags)
     lo, hi = shard_range(n, rank, ws)
     device = torch.device("cuda", ctx.device)
-    plen = partials_layout(k)["length"]
+    l = objective_outputs(k, objective, params)
+    plen = partials_layout(k, l)["length"]
     ex = None if use_nccl() else peer_exchange(plen, device)
     if ex is not None and hi > lo:
         return ctx.fused_plan(k, n, perm, objective, params, discard, scale, raw, flags, lo, hi, ex).run()
@@ -161,4 +174,4 @@ def fused_step(ctx, k, n, perm, objective, params, discard, scale, raw, flags):
     with on_torch_stream(ctx, device):
         ctx.fused_partials(k, n, perm, objective, params, discard, scale, raw, lo, hi, flags, out=part)
         allreduce_partials(part)
-        return ctx.finalize(k, 1, n, part, flags)
+        return ctx.finalize(k, l, n, part, flags)

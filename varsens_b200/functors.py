@@ -18,6 +18,10 @@ class Functor(object):
     def params(self, k):
         raise NotImplementedError
 
+    def outputs(self, k):
+        """Outputs per sample point (the l of fM_1 (n, l) and sens (k, l))."""
+        return 1
+
     def __call__(self, x):
         raise _cabi.VarsensError(
             "%s is a device functor: pass it to Objective/Varsens instead of calling it on the host"
@@ -61,6 +65,121 @@ class RK4Chain(Functor):
 
     def params(self, k):
         return numpy.array([self.dt, float(self.nsteps)])
+
+
+class Param(object):
+    """Coordinate ``c`` of the (scaled) sample point, as a rate constant or initial amount of a MassActionNetwork."""
+
+    def __init__(self, c):
+        if isinstance(c, bool) or not isinstance(c, (int, numpy.integer)) or c < 0:
+            raise _cabi.VarsensError("Param needs a coordinate index >= 0, got %r" % (c,))
+        self.c = int(c)
+
+    def __repr__(self):
+        return "Param(%d)" % self.c
+
+
+class MassActionNetwork(Functor):
+    """Mass-action reaction network integrated by classic fixed-step RK4 on the GPU; the objective is L observables, each a
+    weighted sum of species amounts at T = nsteps * dt (the l = L outputs of every sample point).
+
+    ``species``      a count, or a list of names;
+    ``reactions``    tuples ``(reactants, products, kf, kr=None)``: each side a species, a list of at most two species (a
+                     species may appear twice) or an empty list; species by name or index; ``kr=None`` = irreversible;
+    ``initial``      one initial amount per species;
+    ``observables``  a list of ``{species: weight}`` dicts or of single species (weight 1).
+    A rate or initial amount is a number (a constant) or ``Param(c)``: coordinate c of the scaled sample point.  Packed
+    layout and frozen arithmetic: include/varsens_b200.h (VS_OBJ_MASS_ACTION)."""
+    objective_id = _cabi.OBJ_MASS_ACTION
+
+    def __init__(self, species, reactions, initial, observables, dt=0.01, nsteps=1000):
+        err = _cabi.VarsensError
+        if isinstance(species, (int, numpy.integer)) and not isinstance(species, bool):
+            self.names = None
+            S = int(species)
+        else:
+            self.names = [str(s) for s in species]
+            if len(set(self.names)) != len(self.names):
+                raise err("MassActionNetwork: species names are not unique")
+            S = len(self.names)
+        if not 1 <= S <= 128:
+            raise err("MassActionNetwork: %d species, need 1..128" % S)
+        self.S = S
+        self._max_coord = -1                       # largest sample coordinate a Param refers to
+        self.dt, self.nsteps = float(dt), nsteps
+        if not numpy.isfinite(self.dt):
+            raise err("MassActionNetwork: dt = %r is not finite" % (dt,))
+        if isinstance(nsteps, bool) or not isinstance(nsteps, (int, numpy.integer)) or not 0 <= nsteps < 2 ** 31:
+            raise err("MassActionNetwork: nsteps = %r, need an integer in [0, 2^31)" % (nsteps,))
+        self.nsteps = int(nsteps)
+        reactions = list(reactions)
+        if not 1 <= len(reactions) <= 512:
+            raise err("MassActionNetwork: %d reactions, need 1..512" % len(reactions))
+        recs = []
+        for r, rx in enumerate(reactions):
+            rx = tuple(rx)
+            if len(rx) not in (3, 4):
+                raise err("MassActionNetwork: reaction %d must be (reactants, products, kf[, kr])" % r)
+            a = self._side(rx[0], "reaction %d reactants" % r)
+            b = self._side(rx[1], "reaction %d products" % r)
+            kfc, kf = self._value(rx[2], "reaction %d kf" % r)
+            kr = rx[3] if len(rx) == 4 else None
+            krc, krv = (-1, 0.0) if kr is None else self._value(kr, "reaction %d kr" % r)
+            recs.append(a + b + [kfc, kf, krc, krv])
+        initial = list(initial)
+        if len(initial) != S:
+            raise err("MassActionNetwork: %d initial amounts for %d species" % (len(initial), S))
+        init = [self._value(v, "initial amount of species %d" % s) for s, v in enumerate(initial)]
+        observables = list(observables)
+        if not 1 <= len(observables) <= 64:
+            raise err("MassActionNetwork: %d observables, need 1..64" % len(observables))
+        w = numpy.zeros((len(observables), S))
+        for o, ob in enumerate(observables):
+            items = ob.items() if isinstance(ob, dict) else [(ob, 1.0)]
+            for sp, wt in items:
+                if isinstance(wt, Param) or isinstance(wt, bool) or not isinstance(wt, (int, float, numpy.number)):
+                    raise err("MassActionNetwork: observable %d, weight %r is not a number" % (o, wt))
+                w[o, self._species(sp, "observable %d" % o)] += float(wt)
+        self.L = len(observables)
+        self._packed = numpy.array([S, len(recs), self.L, self.dt, self.nsteps] + [x for rec in recs for x in rec] +
+                                   [x for iv in init for x in iv] + list(w.ravel()), dtype=numpy.float64)
+
+    def _species(self, sp, what):
+        err = _cabi.VarsensError
+        if isinstance(sp, str):
+            if self.names is None or sp not in self.names:
+                raise err("MassActionNetwork: %s: unknown species %r" % (what, sp))
+            return self.names.index(sp)
+        if isinstance(sp, bool) or not isinstance(sp, (int, numpy.integer)) or not 0 <= sp < self.S:
+            raise err("MassActionNetwork: %s: species %r is neither a name nor an index in [0, %d)" % (what, sp, self.S))
+        return int(sp)
+
+    def _side(self, side, what):
+        if side is None:
+            side = []
+        elif isinstance(side, (str, int, numpy.integer)):
+            side = [side]
+        side = [self._species(sp, what) for sp in side]
+        if len(side) > 2:
+            raise _cabi.VarsensError("MassActionNetwork: %s: %d species, at most 2" % (what, len(side)))
+        return side + [-1] * (2 - len(side))
+
+    def _value(self, v, what):
+        if isinstance(v, Param):
+            self._max_coord = max(self._max_coord, v.c)
+            return [v.c, 0.0]
+        if isinstance(v, bool) or not isinstance(v, (int, float, numpy.number)):
+            raise _cabi.VarsensError("MassActionNetwork: %s = %r: need a number or Param(c)" % (what, v))
+        return [-1, float(v)]
+
+    def params(self, k):
+        if self._max_coord >= k:
+            raise _cabi.VarsensError("MassActionNetwork uses coordinate %d, the sample has k = %d" % (self._max_coord, k))
+        _cabi.objective_outputs(k, self.objective_id, self._packed)          # the library's own validation
+        return self._packed
+
+    def outputs(self, k):
+        return _cabi.objective_outputs(k, self.objective_id, self.params(k))
 
 
 def vectorized(fn):
