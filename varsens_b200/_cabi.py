@@ -40,9 +40,20 @@ class vs_scale(ctypes.Structure):
     _fields_ = [("kind", ctypes.c_int), ("lower", ctypes.c_void_p), ("upper", ctypes.c_void_p)]
 
 
+def _result_fields(k, l, second_order=True):
+    """(name, length, shape) of each array of a result block, in the library's order; a first-order block ends after sens_t."""
+    kl = k * l
+    fields = [("E_2", l, (l,)), ("var_y", l, (l,)), ("U_j", kl, (k, l)), ("U_nj", kl, (k, l)), ("sens", kl, (k, l)),
+              ("sens_t", kl, (k, l)), ("sens_2", kl * kl, (k, l, k, l)), ("sens_2n", kl * kl, (k, l, k, l))]
+    return fields if second_order else fields[:6]
+
+
+def _block_len(k, l, second_order=True):
+    return sum(cnt for _, cnt, _ in _result_fields(k, l, second_order))
+
+
 class vs_result(ctypes.Structure):
-    _fields_ = [(name, ctypes.c_void_p) for name in
-                ("E_2", "var_y", "U_j", "U_nj", "sens", "sens_t", "sens_2", "sens_2n")]
+    _fields_ = [(name, ctypes.c_void_p) for name, _, _ in _result_fields(1, 1)]
 
 
 _lib = None
@@ -99,10 +110,6 @@ def lib():
         L.vs_measure_fp64_peak.argtypes = [vp, P(ctypes.c_double)]
         L.vs_last_kernel_ms.argtypes = [vp, P(ctypes.c_float)]
         L.vs_objective_outputs.argtypes = [i32, i32, vp, i32, P(i32)]
-        for name in SYMBOLS:
-            fn = getattr(L, name)
-            if fn.restype is ctypes.c_int and name not in ("vs_abi_version",):
-                pass
         _lib = L
         return _lib
 
@@ -163,6 +170,22 @@ def buf(x, dtype=None, out=False):
     return a.ctypes.data_as(ctypes.c_void_p), MEM_HOST, a
 
 
+def _source_args(k, perm, raw, scale, params=None):
+    """The design's source and objective parameters as the C ABI takes them: ((perm, perm_mem, raw, raw_mem, scale),
+    (params, n_params) or () without params, the objects that must stay alive while the library reads them)."""
+    sp, sk = scale.c_struct(k)
+    pp, pm, pk = buf(perm, numpy.uint32)
+    rp, rm, rk = buf(raw, numpy.float64)
+    par = None if params is None else numpy.ascontiguousarray(params, dtype=numpy.float64)
+    pa = () if par is None else (par.ctypes.data_as(ctypes.c_void_p), int(par.size))
+    return (pp, pm, rp, rm, sp), pa, (sk, pk, rk, par)
+
+
+def _peer_arrays(world, peer_bufs, peer_flags):
+    """The uint64[world] tables of an exchange: every rank's buffer and every rank's flag array."""
+    return tuple((ctypes.c_uint64 * world)(*[int(x) for x in a]) for a in (peer_bufs, peer_flags))
+
+
 class Scale(object):
     """Host descriptor lowered to vs_scale (identity / linear / power)."""
 
@@ -193,59 +216,35 @@ class Result(object):
     """Host arrays shaped like the reference's attributes (varsens/saltelli.py:577-622)."""
 
     def __init__(self, k, l, second_order=True):
+        self._view(k, l, numpy.zeros(_block_len(k, l, second_order)), second_order)
+
+    def _view(self, k, l, flat, second_order):
         self.k, self.l = k, l
-        self.E_2 = numpy.zeros(l)
-        self.var_y = numpy.zeros(l)
-        self.U_j = numpy.zeros((k, l))
-        self.U_nj = numpy.zeros((k, l))
-        self.sens = numpy.zeros((k, l))
-        self.sens_t = numpy.zeros((k, l))
-        self.sens_2 = numpy.zeros((k, l, k, l)) if second_order else None
-        self.sens_2n = numpy.zeros((k, l, k, l)) if second_order else None
+        self.sens_2 = self.sens_2n = None
+        at = 0
+        for name, cnt, shape in _result_fields(k, l, second_order):
+            setattr(self, name, flat[at:at + cnt].reshape(shape))
+            at += cnt
+        return self
 
     @classmethod
     def views(cls, k, l, flat, second_order=True):
         """Result whose arrays are views of one flat float64 buffer in the library's result order (no copies)."""
-        r = cls.__new__(cls)
-        r.k, r.l = k, l
-        kl = k * l
-        r.E_2, r.var_y = flat[0:l], flat[l:2 * l]
-        at = 2 * l
-        r.U_j = flat[at:at + kl].reshape(k, l)
-        r.U_nj = flat[at + kl:at + 2 * kl].reshape(k, l)
-        r.sens = flat[at + 2 * kl:at + 3 * kl].reshape(k, l)
-        r.sens_t = flat[at + 3 * kl:at + 4 * kl].reshape(k, l)
-        at += 4 * kl
-        if second_order:
-            r.sens_2 = flat[at:at + kl * kl].reshape(k, l, k, l)
-            r.sens_2n = flat[at + kl * kl:at + 2 * kl * kl].reshape(k, l, k, l)
-        else:
-            r.sens_2 = r.sens_2n = None
-        return r
+        return cls.__new__(cls)._view(k, l, flat, second_order)
 
     @staticmethod
     def flat_len(k, l):
-        return 2 * l + 4 * k * l + 2 * (k * l) ** 2
+        return _block_len(k, l)
 
     @classmethod
     def from_flat(cls, k, l, flat, second_order=True):
         """Unpack the device result layout of vs_finalize_device (a host numpy copy of it)."""
-        r = cls(k, l, second_order)
-        kl, at = k * l, 0
-        for name, cnt, shape in (("E_2", l, (l,)), ("var_y", l, (l,)), ("U_j", kl, (k, l)), ("U_nj", kl, (k, l)),
-                                 ("sens", kl, (k, l)), ("sens_t", kl, (k, l)), ("sens_2", kl * kl, (k, l, k, l)),
-                                 ("sens_2n", kl * kl, (k, l, k, l))):
-            if name.startswith("sens_2") and not second_order:
-                break
-            setattr(r, name, numpy.array(flat[at:at + cnt], dtype=numpy.float64).reshape(shape))
-            at += cnt
-        return r
+        return cls.views(k, l, numpy.array(flat[:_block_len(k, l, second_order)], dtype=numpy.float64), second_order)
 
     def c_struct(self):
-        def p(a):
-            return None if a is None else a.ctypes.data_as(ctypes.c_void_p)
-        return vs_result(p(self.E_2), p(self.var_y), p(self.U_j), p(self.U_nj), p(self.sens), p(self.sens_t),
-                         p(self.sens_2), p(self.sens_2n))
+        """vs_result pointing at these arrays (NULL for the second-order arrays of a first-order result)."""
+        arrays = [getattr(self, name) for name, _ in vs_result._fields_]
+        return vs_result(*[None if a is None else a.ctypes.data for a in arrays])
 
 
 class Context(object):
@@ -342,12 +341,9 @@ class Context(object):
         total = 2 * n * (1 + k)
         row_end = total if row_end is None else row_end
         out = numpy.empty((int(row_end - row_begin), int(k))) if out is None else out
-        sp, keep = scale.c_struct(k)
-        pp, pm, pk = buf(perm, numpy.uint32)
-        rp, rm, rk = buf(raw, numpy.float64)
+        src, _, keep = _source_args(k, perm, raw, scale)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_sample_flat(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(row_begin),
-                                   int(row_end), op, om))
+        check(lib().vs_sample_flat(self._h, int(k), int(n), discard_arg(discard), *src, int(row_begin), int(row_end), op, om))
         return out
 
     def sample_flat_shard(self, k, n, perm, i_begin, i_end, discard=0, scale=IDENTITY, raw=None, out=None):
@@ -355,11 +351,9 @@ class Context(object):
         export mode (vs_sample_flat_shard)."""
         rows = int(i_end - i_begin)
         out = numpy.empty((2 + 2 * int(k), rows, int(k))) if out is None else out
-        sp, keep = scale.c_struct(k)
-        pp, pm, pk = buf(perm, numpy.uint32)
-        rp, rm, rk = buf(raw, numpy.float64)
+        src, _, keep = _source_args(k, perm, raw, scale)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_sample_flat_shard(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(i_begin), int(i_end), op, om))
+        check(lib().vs_sample_flat_shard(self._h, int(k), int(n), discard_arg(discard), *src, int(i_begin), int(i_end), op, om))
         return out
 
     # ---- objective values / estimators --------------------------------------------------------
@@ -370,13 +364,10 @@ class Context(object):
         l = objective_outputs(k, objective, params)
         if out is None:
             out = numpy.empty((2 + 2 * k, int(i_end - i_begin)) + ((l,) if l > 1 else ()))
-        par = numpy.ascontiguousarray(params, dtype=numpy.float64)
-        sp, keep = scale.c_struct(k)
-        pp, pm, pk = buf(perm, numpy.uint32)
-        rp, rm, rk = buf(raw, numpy.float64)
+        src, par, keep = _source_args(k, perm, raw, scale, params)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_eval_values(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
-                                   par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end), op, om))
+        check(lib().vs_eval_values(self._h, int(k), int(n), discard_arg(discard), *src, int(objective), *par, int(i_begin),
+                                   int(i_end), op, om))
         return out
 
     def partials_from_values(self, k, l, rows, fvals, shift=None, flags=FLAG_SECOND_ORDER, out=None):
@@ -411,8 +402,7 @@ class Context(object):
         """All-reduce over NVLink peer memory fused with the finalisation (vs_allreduce_finalize_p2p)."""
         res = Result(k, l, bool(flags & FLAG_SECOND_ORDER))
         cs = res.c_struct()
-        pb = (ctypes.c_uint64 * world_size)(*[int(x) for x in peer_bufs])
-        pf = (ctypes.c_uint64 * world_size)(*[int(x) for x in peer_flags])
+        pb, pf = _peer_arrays(world_size, peer_bufs, peer_flags)
         pp, pm, pk = buf(partials, numpy.float64)
         if pm != MEM_DEVICE:
             raise VarsensError("partials must be a device tensor")
@@ -434,47 +424,35 @@ class Context(object):
         i_end = n if i_end is None else i_end
         plen = int(lib().vs_partials_len(int(k), objective_outputs(k, objective, params)))
         out = numpy.empty(plen) if out is None else out
-        par = numpy.ascontiguousarray(params, dtype=numpy.float64)
-        sp, keep = scale.c_struct(k)
-        pp, pm, pk = buf(perm, numpy.uint32)
-        rp, rm, rk = buf(raw, numpy.float64)
+        src, par, keep = _source_args(k, perm, raw, scale, params)
         op, om, _ = buf(out, numpy.float64, out=True)
-        check(lib().vs_fused_partials(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
-                                      par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end),
-                                      int(flags), op, om))
+        check(lib().vs_fused_partials(self._h, int(k), int(n), discard_arg(discard), *src, int(objective), *par, int(i_begin),
+                                      int(i_end), int(flags), op, om))
         return out
 
     def run_fused(self, k, n, perm, objective, params, discard=0, scale=IDENTITY, raw=None, flags=FLAG_SECOND_ORDER):
         res = Result(k, objective_outputs(k, objective, params), bool(flags & FLAG_SECOND_ORDER))
         cs = res.c_struct()
-        par = numpy.ascontiguousarray(params, dtype=numpy.float64)
-        sp, keep = scale.c_struct(k)
-        pp, pm, pk = buf(perm, numpy.uint32)
-        rp, rm, rk = buf(raw, numpy.float64)
-        check(lib().vs_run_fused(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
-                                 par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(flags), ctypes.byref(cs)))
+        src, par, keep = _source_args(k, perm, raw, scale, params)
+        check(lib().vs_run_fused(self._h, int(k), int(n), discard_arg(discard), *src, int(objective), *par, int(flags),
+                                 ctypes.byref(cs)))
         return res
 
+    def run_fused_p2p(self, k, n, perm, objective, params, world_size, rank, peer_bufs, peer_flags, epoch, i_begin, i_end,
+                      discard=0, scale=IDENTITY, raw=None, flags=FLAG_SECOND_ORDER):
+        """vs_run_fused_p2p: this rank's shard [i_begin,i_end) of the fused step, all-reduce over NVLink peer memory and
+        estimators inside the ONE kernel launch; returns the Result (identical bits on every rank)."""
+        res = Result(k, objective_outputs(k, objective, params), bool(flags & FLAG_SECOND_ORDER))
+        cs = res.c_struct()
+        src, par, keep = _source_args(k, perm, raw, scale, params)
+        pb, pf = _peer_arrays(world_size, peer_bufs, peer_flags)
+        check(lib().vs_run_fused_p2p(self._h, int(k), int(n), discard_arg(discard), *src, int(objective), *par, int(i_begin),
+                                     int(i_end), int(flags), int(world_size), int(rank), pb, pf, int(epoch), ctypes.byref(cs)))
+        return res
 
-def _run_fused_p2p(self, k, n, perm, objective, params, world_size, rank, peer_bufs, peer_flags, epoch, i_begin, i_end,
-                   discard=0, scale=IDENTITY, raw=None, flags=FLAG_SECOND_ORDER):
-    """vs_run_fused_p2p: this rank's shard [i_begin,i_end) of the fused step, all-reduce over NVLink peer memory and
-    estimators inside the ONE kernel launch; returns the Result (identical bits on every rank)."""
-    res = Result(k, objective_outputs(k, objective, params), bool(flags & FLAG_SECOND_ORDER))
-    cs = res.c_struct()
-    par = numpy.ascontiguousarray(params, dtype=numpy.float64)
-    sp, keep = scale.c_struct(k)
-    pp, pm, pk = buf(perm, numpy.uint32)
-    rp, rm, rk = buf(raw, numpy.float64)
-    pb = (ctypes.c_uint64 * world_size)(*[int(x) for x in peer_bufs])
-    pf = (ctypes.c_uint64 * world_size)(*[int(x) for x in peer_flags])
-    check(lib().vs_run_fused_p2p(self._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
-                                 par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end), int(flags),
-                                 int(world_size), int(rank), pb, pf, int(epoch), ctypes.byref(cs)))
-    return res
-
-
-Context.run_fused_p2p = _run_fused_p2p
+    def fused_plan(self, *args, **kwargs):
+        """FusedPlan(self, *args, **kwargs): a fused step prepared once and run many times."""
+        return FusedPlan(self, *args, **kwargs)
 
 
 class FusedPlan(object):
@@ -490,25 +468,13 @@ class FusedPlan(object):
                  i_begin=0, i_end=None, exchange=None):
         self.ctx, self.k, self.second = ctx, int(k), bool(flags & FLAG_SECOND_ORDER)
         self.exchange = exchange
-        par = numpy.ascontiguousarray(params, dtype=numpy.float64)
-        sp, keep = scale.c_struct(k)
-        pp, pm, pk = buf(perm, numpy.uint32)
-        rp, rm, rk = buf(raw, numpy.float64)
-        self._keep = (par, keep, pk, rk, sp)
+        src, par, self._keep = _source_args(k, perm, raw, scale, params)
         self.l = l = objective_outputs(k, objective, params)
-        kl = self.k * l
-        self._len = Result.flat_len(self.k, l) if self.second else 2 * l + 4 * kl
-        o = (0, l, 2 * l, 2 * l + kl, 2 * l + 2 * kl, 2 * l + 3 * kl, 2 * l + 4 * kl, 2 * l + 4 * kl + kl * kl)
-        self._out = []                                   # two output sets: (flat buffer, vs_result struct, byref, Result views)
+        self._out = []                                   # two output sets: (byref of the vs_result struct, Result, struct)
         for _ in range(2):
-            flat = numpy.empty(self._len)
-            base = flat.ctypes.data
-            if self.second:
-                cs = vs_result(base, base + 8 * o[1], base + 8 * o[2], base + 8 * o[3], base + 8 * o[4], base + 8 * o[5],
-                               base + 8 * o[6], base + 8 * o[7])
-            else:
-                cs = vs_result(base, base + 8 * o[1], base + 8 * o[2], base + 8 * o[3], base + 8 * o[4], base + 8 * o[5], None, None)
-            self._out.append((flat, cs, ctypes.byref(cs), Result.views(self.k, l, flat, self.second)))
+            res = Result(self.k, l, self.second)
+            cs = res.c_struct()
+            self._out.append((ctypes.byref(cs), res, cs))
         self._turn = 0
         L = lib()
         i_end = n if i_end is None else i_end
@@ -516,20 +482,16 @@ class FusedPlan(object):
             if i_begin != 0 or i_end != n:
                 raise VarsensError("a single-GPU plan covers the whole design")
             self._fn = L.vs_run_fused
-            self._args = (ctx._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
-                          par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(flags))
+            self._args = (ctx._h, int(k), int(n), discard_arg(discard), *src, int(objective), *par, int(flags))
         else:
-            pb = (ctypes.c_uint64 * exchange.world)(*[int(x) for x in exchange.peer_bufs])
-            pf = (ctypes.c_uint64 * exchange.world)(*[int(x) for x in exchange.peer_flags])
-            self._keep += (pb, pf)
             self._fn = L.vs_run_fused_p2p
-            self._args = (ctx._h, int(k), int(n), discard_arg(discard), pp, pm, rp, rm, sp, int(objective),
-                          par.ctypes.data_as(ctypes.c_void_p), int(par.size), int(i_begin), int(i_end), int(flags),
-                          int(exchange.world), int(exchange.rank), pb, pf)
+            self._args = (ctx._h, int(k), int(n), discard_arg(discard), *src, int(objective), *par, int(i_begin), int(i_end),
+                          int(flags), int(exchange.world), int(exchange.rank),
+                          *_peer_arrays(exchange.world, exchange.peer_bufs, exchange.peer_flags))
 
     def run(self):
         self._turn ^= 1
-        _, _, ref, res = self._out[self._turn]
+        ref, res, _ = self._out[self._turn]
         if self.exchange is None:
             st = self._fn(*self._args, ref)
         else:
@@ -537,9 +499,6 @@ class FusedPlan(object):
         if st != VS_OK:
             check(st)
         return res
-
-
-Context.fused_plan = lambda self, *a, **kw: FusedPlan(self, *a, **kw)
 
 
 def reference_permutation(n, seed=1):

@@ -43,8 +43,22 @@ int check_common(vs_ctx *c, int k) {
     return VS_OK;
 }
 
-void unpack_result(const double *p, int k, int l, int flags, vs_result *r) {
-    size_t kl = (size_t)k * l;
+// Results the kernels write straight into the ctx's mapped host buffer (no copy call), in two steps around the launch.
+// Before: a buffer large enough and a cleared status slot (finalize_kernel never writes it, so a time-out left by an earlier
+// exchange cannot leak into a later call).
+int host_result_begin(vs_ctx *c, int k, int l) {
+    VS_TRY(ensure_host_res(c, result_len(k, l) + HOST_RES_EXTRA));
+    c->host_res[result_len(k, l) + HOST_RES_STATUS] = 0.0;
+    return VS_OK;
+}
+
+// After: wait for the kernel, fail on a peer time-out, copy out the fields the caller asked for.
+int host_result_end(vs_ctx *c, int k, int l, int flags, vs_result *r) {
+    VS_CUDA(cudaStreamSynchronize(c->stream));
+    VS_REQUIRE(c->host_res[result_len(k, l) + HOST_RES_STATUS] == 0.0, VS_ERR_TIMEOUT,
+               "peer-memory all-reduce: a rank did not publish its partial sums within %d ms", c->opt.p2p_timeout_ms);
+    const double *p = c->host_res;
+    const size_t kl = (size_t)k * l;
     auto take = [&](double *dst, size_t cnt) {
         if (dst) memcpy(dst, p, cnt * sizeof(double));
         p += cnt;
@@ -59,24 +73,43 @@ void unpack_result(const double *p, int k, int l, int flags, vs_result *r) {
         take(r->sens_2, kl * kl);
         take(r->sens_2n, kl * kl);
     }
-}
-
-// Estimators from partial sums in HBM: finalize_kernel writes straight into the ctx's mapped host buffer (no copy call).
-int finalize_to_host(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, const double *partials_dev, int flags, vs_result *r) {
-    VS_TRY(ensure_host_res(c, result_len(k, l) + HOST_RES_EXTRA));
-    VS_TRY(launch_finalize(c, k, l, n, rows, partials_dev, flags, c->host_res));
-    VS_CUDA(cudaStreamSynchronize(c->stream));
-    unpack_result(c->host_res, k, l, flags, r);
     return VS_OK;
 }
 
-// Results the tail of the fused kernel left in the mapped host buffer (after the stream has been synchronised).
-int take_tail_result(vs_ctx *c, int k, int flags, vs_result *r) {
-    VS_CUDA(cudaStreamSynchronize(c->stream));
-    const double *x = c->host_res + result_len(k, 1);
-    VS_REQUIRE(x[0] == 0.0, VS_ERR_TIMEOUT, "peer-memory all-reduce: a rank did not publish its partial sums within %d ms",
-               c->opt.p2p_timeout_ms);
-    unpack_result(c->host_res, k, 1, flags, r);
+// Estimators from partial sums in HBM.
+int finalize_to_host(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, const double *partials_dev, int flags, vs_result *r) {
+    VS_TRY(host_result_begin(c, k, l));
+    VS_TRY(launch_finalize(c, k, l, n, rows, partials_dev, flags, c->host_res));
+    return host_result_end(c, k, l, flags, r);
+}
+
+int check_estimator_args(int l, uint64_t n, uint64_t rows, bool pointers_set) {
+    VS_REQUIRE(l >= 1 && l <= 64 && n >= 2 && rows >= 1 && rows <= n && pointers_set, VS_ERR_ARG, "bad arguments");
+    return VS_OK;
+}
+
+// An all-device call only enqueues its work, but a host input it staged must have left the caller's buffer before it returns.
+int sync_staged_inputs(vs_ctx *c, int out_mem, int perm_mem, const double *raw, int raw_mem) {
+    if (out_mem == VS_MEM_DEVICE && (perm_mem == VS_MEM_HOST || (raw && raw_mem == VS_MEM_HOST)))
+        VS_CUDA(cudaStreamSynchronize(c->stream));
+    return VS_OK;
+}
+
+// The peer tables of an exchange as device arrays: every rank's buffer at [0, 64), its flag array at [64, 128) of peer_buf.
+// Uploaded only when they change, once per exchange rather than once per step, after the work queued on the stream is done.
+int peer_table(vs_ctx *c, int world_size, int rank, const uint64_t *peer_bufs, const uint64_t *peer_flags, uint32_t epoch,
+               const uint64_t **tab) {
+    VS_REQUIRE(world_size >= 1 && world_size <= 64 && rank >= 0 && rank < world_size && peer_bufs && epoch >= 1,
+               VS_ERR_ARG, "bad peer description");
+    VS_TRY(ensure(c, c->peer_buf, 2 * 64 * sizeof(uint64_t)));
+    std::vector<uint64_t> want(128, 0);
+    for (int r = 0; r < world_size; ++r) { want[r] = peer_bufs[r]; want[64 + r] = peer_flags ? peer_flags[r] : 0; }
+    if (want != c->peer_tab) {
+        VS_CUDA(cudaStreamSynchronize(c->stream));
+        c->peer_tab = want;
+        VS_CUDA(cudaMemcpyAsync(c->peer_buf.p, c->peer_tab.data(), 128 * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
+    }
+    *tab = (const uint64_t *)c->peer_buf.p;
     return VS_OK;
 }
 
@@ -141,9 +174,7 @@ extern "C" int vs_sample_flat(vs_ctx *c, int k, uint64_t n, uint64_t discard, co
     VS_TRY(o.begin(c->io_buf));
     VS_TRY(launch_sample_flat(c, k, src, s, row_begin, row_end, (double *)o.dev));
     VS_TRY(o.end());
-    if (out_mem == VS_MEM_DEVICE && (perm_mem == VS_MEM_HOST || (raw && raw_mem == VS_MEM_HOST)))
-        VS_CUDA(cudaStreamSynchronize(c->stream));
-    return VS_OK;
+    return sync_staged_inputs(c, out_mem, perm_mem, raw, raw_mem);
 }
 
 extern "C" int vs_sample_flat_shard(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
@@ -162,9 +193,7 @@ extern "C" int vs_sample_flat_shard(vs_ctx *c, int k, uint64_t n, uint64_t disca
     VS_TRY(o.begin(c->io_buf));
     VS_TRY(launch_sample_shard(c, k, src, s, i_begin, i_end, (double *)o.dev));
     VS_TRY(o.end());
-    if (out_mem == VS_MEM_DEVICE && (perm_mem == VS_MEM_HOST || (raw && raw_mem == VS_MEM_HOST)))
-        VS_CUDA(cudaStreamSynchronize(c->stream));
-    return VS_OK;
+    return sync_staged_inputs(c, out_mem, perm_mem, raw, raw_mem);
 }
 
 extern "C" int vs_eval_values(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
@@ -217,7 +246,7 @@ extern "C" int vs_partials_from_values(vs_ctx *c, int k, int l, uint64_t rows, c
 extern "C" int vs_finalize(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, const double *partials, int partials_mem,
                            int flags, vs_result *result) {
     VS_TRY(check_common(c, k));
-    VS_REQUIRE(l >= 1 && l <= 64 && n >= 2 && rows >= 1 && rows <= n && partials && result, VS_ERR_ARG, "bad arguments");
+    VS_TRY(check_estimator_args(l, n, rows, partials && result));
     const void *pdev = nullptr;
     VS_TRY(stage_in(c, c->part_buf, partials, partials_mem, vs_partials_len(k, l) * sizeof(double), &pdev));
     return finalize_to_host(c, k, l, n, rows, (const double *)pdev, flags, result);
@@ -226,7 +255,7 @@ extern "C" int vs_finalize(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, c
 extern "C" int vs_finalize_device(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, const double *partials_dev, int flags,
                                   double *result_dev) {
     VS_TRY(check_common(c, k));
-    VS_REQUIRE(l >= 1 && l <= 64 && n >= 2 && rows >= 1 && rows <= n && partials_dev && result_dev, VS_ERR_ARG, "bad arguments");
+    VS_TRY(check_estimator_args(l, n, rows, partials_dev && result_dev));
     return launch_finalize(c, k, l, n, rows, partials_dev, flags, result_dev);
 }
 
@@ -234,32 +263,18 @@ extern "C" int vs_allreduce_finalize_p2p(vs_ctx *c, int k, int l, uint64_t n, ui
                                          const uint64_t *peer_bufs, const uint64_t *peer_flags, uint32_t epoch,
                                          const double *partials_dev, int flags, vs_result *result) {
     VS_TRY(check_common(c, k));
-    VS_REQUIRE(l >= 1 && l <= 64 && n >= 2 && rows >= 1 && rows <= n && partials_dev && result, VS_ERR_ARG, "bad arguments");
-    VS_REQUIRE(world_size >= 1 && world_size <= 64 && rank >= 0 && rank < world_size && peer_bufs && epoch >= 1,
-               VS_ERR_ARG, "bad peer description");
-    // the two pointer tables travel as kernel-visible device arrays (dir_buf: world_size * 2 pointers)
-    VS_TRY(ensure(c, c->peer_buf, 2 * 64 * sizeof(uint64_t)));
-    uint64_t *tab = (uint64_t *)c->peer_buf.p;
-    std::vector<uint64_t> want(128, 0);
-    for (int r = 0; r < world_size; ++r) { want[r] = peer_bufs[r]; want[64 + r] = peer_flags ? peer_flags[r] : 0; }
-    if (want != c->peer_tab) {                              // uploaded once per exchange, not per call
-        c->peer_tab = want;
-        VS_CUDA(cudaMemcpyAsync(tab, c->peer_tab.data(), 128 * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
-    }
-    VS_TRY(ensure_host_res(c, result_len(k, l) + HOST_RES_EXTRA));
-    c->host_res[result_len(k, l)] = 0.0;
+    VS_TRY(check_estimator_args(l, n, rows, partials_dev && result));
+    const uint64_t *tab = nullptr;
+    VS_TRY(peer_table(c, world_size, rank, peer_bufs, peer_flags, epoch, &tab));
+    VS_TRY(host_result_begin(c, k, l));
     VS_TRY(launch_p2p_reduce_finalize(c, k, l, n, rows, world_size, rank, tab, tab + 64, epoch, partials_dev, flags, c->host_res));
-    VS_CUDA(cudaStreamSynchronize(c->stream));
-    VS_REQUIRE(c->host_res[result_len(k, l)] == 0.0, VS_ERR_TIMEOUT,
-               "peer-memory all-reduce: a rank did not publish its partial sums within %d ms", c->opt.p2p_timeout_ms);
-    unpack_result(c->host_res, k, l, flags, result);
-    return VS_OK;
+    return host_result_end(c, k, l, flags, result);
 }
 
 extern "C" int vs_indices_from_values(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, const double *fvals, int fvals_mem,
                                       int flags, vs_result *result) {
     VS_TRY(check_common(c, k));
-    VS_REQUIRE(l >= 1 && l <= 64 && n >= 2 && rows >= 1 && rows <= n && fvals && result, VS_ERR_ARG, "bad arguments");
+    VS_TRY(check_estimator_args(l, n, rows, fvals && result));
     const void *fdev = nullptr;
     VS_TRY(stage_in(c, c->io_buf, fvals, fvals_mem, rows * (uint64_t)(2 + 2 * k) * l * sizeof(double), &fdev));
     // common shift = first row of fM_1 (any value works; this one is cheap and data-scaled)
@@ -379,11 +394,8 @@ extern "C" int vs_fused_partials(vs_ctx *c, int k, uint64_t n, uint64_t discard,
     VS_TRY(fused_step(c, k, n, discard, perm, perm_mem, raw, raw_mem, scale, objective, params, n_params, i_begin, i_end, flags,
                       (double *)o.dev, &req, &finalized));
     VS_TRY(o.end());
-    // all-device call: only enqueued (the caller's next op on the same stream, e.g. the all-reduce, orders after it);
-    // with a host input the staged copy must have left the caller's buffer before we return
-    if (partials_mem == VS_MEM_DEVICE && (perm_mem == VS_MEM_HOST || (raw && raw_mem == VS_MEM_HOST)))
-        VS_CUDA(cudaStreamSynchronize(c->stream));
-    return VS_OK;
+    // all-device call: only enqueued (the caller's next op on the same stream, e.g. the all-reduce, orders after it)
+    return sync_staged_inputs(c, partials_mem, perm_mem, raw, raw_mem);
 }
 
 extern "C" int vs_run_fused(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
@@ -398,10 +410,11 @@ extern "C" int vs_run_fused(vs_ctx *c, int k, uint64_t n, uint64_t discard, cons
     req.mode = 1;
     req.n_total = req.rows_total = n;
     bool finalized = false;
+    VS_TRY(host_result_begin(c, k, l));
     VS_TRY(fused_step(c, k, n, discard, perm, perm_mem, raw, raw_mem, scale, objective, params, n_params, 0, n, flags,
                       (double *)c->part_buf.p, &req, &finalized));
-    if (finalized) return take_tail_result(c, k, flags, result);
-    return finalize_to_host(c, k, l, n, n, (const double *)c->part_buf.p, flags, result);
+    if (!finalized) VS_TRY(launch_finalize(c, k, l, n, n, (const double *)c->part_buf.p, flags, c->host_res));
+    return host_result_end(c, k, l, flags, result);
 }
 
 extern "C" int vs_run_fused_p2p(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint32_t *perm, int perm_mem,
@@ -410,17 +423,8 @@ extern "C" int vs_run_fused_p2p(vs_ctx *c, int k, uint64_t n, uint64_t discard, 
                                 const uint64_t *peer_bufs, const uint64_t *peer_flags, uint32_t epoch, vs_result *result) {
     VS_TRY(check_common(c, k));
     VS_REQUIRE(n >= 2 && i_begin < i_end && i_end <= n && result, VS_ERR_ARG, "bad arguments (every rank needs at least one base row)");
-    VS_REQUIRE(world_size >= 1 && world_size <= 64 && rank >= 0 && rank < world_size && peer_bufs && epoch >= 1,
-               VS_ERR_ARG, "bad peer description");
-    VS_TRY(ensure(c, c->peer_buf, 2 * 64 * sizeof(uint64_t)));
-    uint64_t *tab = (uint64_t *)c->peer_buf.p;
-    std::vector<uint64_t> want(128, 0);
-    for (int r = 0; r < world_size; ++r) { want[r] = peer_bufs[r]; want[64 + r] = peer_flags ? peer_flags[r] : 0; }
-    if (want != c->peer_tab) {                              // uploaded once per exchange, not per call
-        VS_CUDA(cudaStreamSynchronize(c->stream));
-        c->peer_tab = want;
-        VS_CUDA(cudaMemcpyAsync(tab, c->peer_tab.data(), 128 * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
-    }
+    const uint64_t *tab = nullptr;
+    VS_TRY(peer_table(c, world_size, rank, peer_bufs, peer_flags, epoch, &tab));
     int l = 1;
     VS_TRY(outputs_of(k, objective, params, n_params, &l));
     VS_TRY(ensure(c, c->part_buf, 2 * vs_partials_len(k, l) * sizeof(double)));
@@ -434,24 +438,19 @@ extern "C" int vs_run_fused_p2p(vs_ctx *c, int k, uint64_t n, uint64_t discard, 
     req.peer_bufs_dev = tab;
     req.peer_flags_dev = tab + 64;
     bool finalized = false;
+    VS_TRY(host_result_begin(c, k, l));
     VS_TRY(fused_step(c, k, n, discard, perm, perm_mem, raw, raw_mem, scale, objective, params, n_params, i_begin, i_end, flags,
                       mine, &req, &finalized));
-    if (finalized) return take_tail_result(c, k, flags, result);
     // kernels without the in-kernel tail (two-phase path, legacy variants): exchange + estimators in the stand-alone kernel
-    VS_TRY(ensure_host_res(c, result_len(k, l) + HOST_RES_EXTRA));
-    c->host_res[result_len(k, l)] = 0.0;
-    VS_TRY(launch_p2p_reduce_finalize(c, k, l, n, n, world_size, rank, tab, tab + 64, epoch, mine, flags, c->host_res));
-    VS_CUDA(cudaStreamSynchronize(c->stream));
-    VS_REQUIRE(c->host_res[result_len(k, l)] == 0.0, VS_ERR_TIMEOUT,
-               "peer-memory all-reduce: a rank did not publish its partial sums within %d ms", c->opt.p2p_timeout_ms);
-    unpack_result(c->host_res, k, l, flags, result);
-    return VS_OK;
+    if (!finalized)
+        VS_TRY(launch_p2p_reduce_finalize(c, k, l, n, n, world_size, rank, tab, tab + 64, epoch, mine, flags, c->host_res));
+    return host_result_end(c, k, l, flags, result);
 }
 
 extern "C" int vs_last_tail_ns(vs_ctx *c, int k, double *ns8) {
     VS_REQUIRE(c && ns8 && c->host_res, VS_ERR_ARG, "no fused step has run on this ctx");
-    const double *x = c->host_res + result_len(k, 1);
-    for (int i = 0; i < 11; ++i) ns8[i] = x[1 + i];
+    const double *x = c->host_res + result_len(k, 1) + HOST_RES_STAMPS;    // the fused kernel's tail has one output per point
+    for (int i = 0; i < 11; ++i) ns8[i] = x[i];
     return VS_OK;
 }
 

@@ -765,7 +765,7 @@ __device__ __forceinline__ double packed_pq(const double *__restrict__ D, int p,
 template <int K, int NB, int HB, bool PM>
 __host__ __device__ constexpr size_t wsd_tail_smem_doubles() {
     constexpr int LROW = wsd_lrow<NB, HB, PM>();
-    constexpr int m = 2 + 2 * K, plen = 4 + m * (m + 1) / 2, rlen = 2 + 4 * K + 2 * K * K;
+    constexpr int m = 2 + 2 * K, plen = 4 + m * (m + 1) / 2, rlen = (int)result_len(K, 1);
     return (size_t)128 + LROW + 2 * (size_t)(plen + 4) + rlen + 8;      // combine scratch | D | Pk | Pr | R
 }
 
@@ -858,7 +858,7 @@ __device__ __forceinline__ void fused_tail(const FusedTail &tail, double *__rest
                                            unsigned long long tb, unsigned long long tc) {
     constexpr int LROW = wsd_lrow<NB, HB, PM>();
     constexpr int NTL = wsd_ntl<NB, HB, PM>();
-    constexpr int m = 2 + 2 * K, plen = 4 + m * (m + 1) / 2, rlen = 2 + 4 * K + 2 * K * K;
+    constexpr int m = 2 + 2 * K, plen = 4 + m * (m + 1) / 2, rlen = (int)result_len(K, 1);
     double *D = smem + 128;                                // [LROW] (after the combine scratch)
     double *Pk = D + LROW;                                 // [plen] packed partial sums of this rank
     double *Pr = Pk + plen + 4;                            // [plen] reduced over ranks (mode 2)
@@ -905,16 +905,16 @@ __device__ __forceinline__ void fused_tail(const FusedTail &tail, double *__rest
         if (tail.res_host) tail.res_host[e] = v;
     }
     if (tail.res_host && tid == 0) {
-        double *x = tail.res_host + rlen;
-        x[0] = timed_out ? 1.0 : 0.0;
-        x[1] = (double)(t1 - t0);                       // two-level combine (this CTA's share) + pack, ns
-        x[2] = (double)(t2 - t1);                       // peer stores (issue)
-        x[3] = (double)(t3 - t2);                       // wait for the peers' elements + rank-order sum
-        x[4] = (double)(globaltimer_ns() - t3);         // estimators + result stores
-        x[5] = (double)(ta - t0);                       // first-level combine (my group's rows)
-        x[6] = (double)(tb - ta);                       // group row to HBM + fence + second-level ticket
-        x[7] = (double)(tc - tb);                       // second-level combine
-        x[8] = (double)(t1 - tc);                       // packed partial-sum vector
+        tail.res_host[rlen + HOST_RES_STATUS] = timed_out ? 1.0 : 0.0;
+        double *x = tail.res_host + rlen + HOST_RES_STAMPS;
+        x[0] = (double)(t1 - t0);                       // two-level combine (this CTA's share) + pack, ns
+        x[1] = (double)(t2 - t1);                       // peer stores (issue)
+        x[2] = (double)(t3 - t2);                       // wait for the peers' elements + rank-order sum
+        x[3] = (double)(globaltimer_ns() - t3);         // estimators + result stores
+        x[4] = (double)(ta - t0);                       // first-level combine (my group's rows)
+        x[5] = (double)(tb - ta);                       // group row to HBM + fence + second-level ticket
+        x[6] = (double)(tc - tb);                       // second-level combine
+        x[7] = (double)(t1 - tc);                       // packed partial-sum vector
     }
 }
 
@@ -1152,10 +1152,10 @@ fused_wsd_kernel(SourceDev src, FusedConst<K> fc, F f, uint64_t i_begin, uint64_
     }
     fused_tail<K, NB, HB, PM>(tail, smem, t0, ta, tb, tc);
     if (tail.mode >= 1 && tail.res_host && threadIdx.x == 0) {      // this CTA's own phases (diagnostics)
-        double *x = tail.res_host + (2 + 4 * K + 2 * K * K);
-        x[9] = (double)(t_pro - t_entry);                            // prologue: table copy, tile zeroing, barriers, shift
-        x[10] = (double)(t_loop - t_pro);                            // main loop
-        x[11] = (double)(t0 - t_loop);                               // CTA combine + row to HBM + fence + first-level ticket
+        double *x = tail.res_host + result_len(K, 1) + HOST_RES_STAMPS;
+        x[8] = (double)(t_pro - t_entry);                            // prologue: table copy, tile zeroing, barriers, shift
+        x[9] = (double)(t_loop - t_pro);                             // main loop
+        x[10] = (double)(t0 - t_loop);                               // CTA combine + row to HBM + fence + first-level ticket
     }
 }
 
@@ -1221,7 +1221,6 @@ static int launch_fused_t(vs_ctx *c, const SourceDev &src, const FusedConst<K> &
             constexpr int HBk = pm_hb<K>();
             constexpr int NBk = PMk ? 2 * HBk : (M + 7) / 8, MPADk = NBk * 8;
             constexpr int LROWk = wsd_lrow<NBk, HBk, PMk>(), NTLk = wsd_ntl<NBk, HBk, PMk>();
-            constexpr int RLEN = 2 + 4 * K + 2 * K * K;
             const int eps = variant == 6 ? 3 : 2;
             uint64_t wantd = (nbatch + eps * WS_S - 1) / (eps * WS_S);
             int gridd = (int)(wantd < (uint64_t)c->sm_count ? wantd : (uint64_t)c->sm_count);
@@ -1241,7 +1240,7 @@ static int launch_fused_t(vs_ctx *c, const SourceDev &src, const FusedConst<K> &
             tail.partials = partials;
             tail.mode = req ? req->mode : 0;
             if (tail.mode >= 1) {
-                VS_TRY(ensure_host_res(c, (size_t)RLEN + HOST_RES_EXTRA));
+                VS_TRY(ensure_host_res(c, result_len(K, 1) + HOST_RES_EXTRA));
                 tail.res_dev = nullptr;                              // results go straight to mapped host memory
                 tail.res_host = c->host_res;
                 tail.n_total = (double)req->n_total;

@@ -584,13 +584,8 @@ int launch_partials_from_values(vs_ctx *c, int k, int l, uint64_t rows, const do
 // ---------------------------------------------------------------------------------------------
 // Finalisation: the estimators of varsens/saltelli.py:577-622 on the sufficient statistics, same
 // operation order (E_2 over n; U and Grams over n-1; mixed normalisation is the reference's).
-// Result buffer: E_2[l] var_y[l] U_j[kl] U_nj[kl] sens[kl] sens_t[kl] sens_2[(kl)^2] sens_2n[(kl)^2]
+// Result buffer: see result_len (vs_internal.cuh).
 // ---------------------------------------------------------------------------------------------
-size_t result_len(int k, int l) {
-    size_t kl = (size_t)k * l;
-    return 2 * (size_t)l + 4 * kl + 2 * kl * kl;
-}
-
 __global__ void __launch_bounds__(256) finalize_kernel(int k, int l, double n, double rows, const double *__restrict__ P, int second_order,
                                                        double *__restrict__ res) {
     finalize_body(k, l, n, rows, P, second_order, res);
@@ -599,7 +594,8 @@ __global__ void __launch_bounds__(256) finalize_kernel(int k, int l, double n, d
 // Partial-sum all-reduce over NVLink peer memory fused with the finalisation (see vs_allreduce_finalize_p2p); the stand-alone
 // form of the exchange the fused kernel runs in its tail (fused_impl.cuh: fused_tail), for partial sums that come from elsewhere
 // (two-phase path, user values).  Single CTA; same low-latency protocol (device.cuh: ll_push / ll_reduce).
-// res[rlen] = 1.0 if a peer did not show up within timeout_ns (the indices are then meaningless), else 0.0.
+// Status slot res[rlen + HOST_RES_STATUS] = 1.0 if a peer did not show up within timeout_ns (the indices are then meaningless),
+// else 0.0.
 __global__ void __launch_bounds__(256) p2p_reduce_finalize_kernel(int k, int l, double n, double rows, int world, int rank,
                                                                   const uint64_t *__restrict__ bufs, unsigned epoch, int plen, int rlen,
                                                                   unsigned long long timeout_ns, const double *__restrict__ mine,
@@ -611,7 +607,7 @@ __global__ void __launch_bounds__(256) p2p_reduce_finalize_kernel(int k, int l, 
     if (!ll_reduce(bufs, world, rank, epoch, plen, reduced, timeout_ns)) timed_out = 1u;
     __syncthreads();
     finalize_body(k, l, n, rows, reduced, second_order, res);
-    if (threadIdx.x == 0) res[rlen] = timed_out ? 1.0 : 0.0;
+    if (threadIdx.x == 0) res[rlen + HOST_RES_STATUS] = timed_out ? 1.0 : 0.0;
 }
 
 int launch_p2p_reduce_finalize(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, int world, int rank, const uint64_t *peer_bufs_dev,

@@ -202,7 +202,6 @@ int launch_eval_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s
 int launch_partials_from_values(vs_ctx *c, int k, int l, uint64_t rows, const double *fvals, const double *shift_dev,
                                 int flags, double *partials);
 int launch_finalize(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, const double *partials, int flags, double *res_dev);
-size_t result_len(int k, int l);
 int launch_p2p_reduce_finalize(vs_ctx *c, int k, int l, uint64_t n, uint64_t rows, int world, int rank, const uint64_t *peer_bufs_dev,
                                const uint64_t *peer_flags_dev, uint32_t epoch, const double *partials, int flags, double *res_dev);
 int launch_gram_scatter(vs_ctx *c, const GramGeom &g, int nblocks, const double *blockpart, double *partials, int plen);
@@ -223,7 +222,16 @@ int launch_fused(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, cons
                  uint64_t i_end, int flags, double *partials, const FusedReq *req, bool *finalized);
 int ensure_host_res(vs_ctx *c, size_t doubles);
 void load_options(Options &o);
-constexpr int HOST_RES_EXTRA = 32;      // doubles after the results: [0] status (0 ok, 1 peer time-out), [1..] tail time stamps (ns)
+
+// Result block, in this order: E_2[l] var_y[l] U_j[kl] U_nj[kl] sens[kl] sens_t[kl] sens_2[(kl)^2] sens_2n[(kl)^2], always
+// sized for the second-order form.  In the ctx's mapped host buffer HOST_RES_EXTRA doubles follow it: the status slot
+// (written by the fused kernel's tail and the stand-alone exchange kernel) and the time stamps of the fused kernel's tail.
+__host__ __device__ constexpr size_t result_len(int k, int l) {
+    return 2 * (size_t)l + 4 * (size_t)k * l + 2 * ((size_t)k * l) * ((size_t)k * l);
+}
+constexpr int HOST_RES_EXTRA = 32;      // doubles after the results
+constexpr int HOST_RES_STATUS = 0;      // offset after the results: 0.0 ok, 1.0 a peer did not publish within the time-out
+constexpr int HOST_RES_STAMPS = 1;      // offset after the results of the 11 tail time stamps (ns, vs_last_tail_ns)
 // microbench.cu
 int launch_fp64_peak(vs_ctx *c, double *tflops);
 
