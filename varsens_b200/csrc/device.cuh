@@ -65,13 +65,14 @@ __device__ __forceinline__ double radical_inverse(const double *__restrict__ T, 
 }
 
 // VS_HALTON_HORNER: x = (x + digit_j) / b from the most significant digit down (one fp64 division per digit).
+// Digits are kept in 32 bits: from dimension 54 on the bases exceed 255 (the 55th prime is 257).
 __device__ __forceinline__ double radical_inverse_horner(uint32_t b, uint64_t magic, uint32_t m) {
     if (b == 2u) return (double)__brev(m) * 2.3283064365386962890625e-10;
-    unsigned char dig[32];
+    uint32_t dig[32];
     int nd = 0;
     while (m != 0u) {
         uint32_t q = (uint32_t)__umul64hi((uint64_t)m, magic);
-        dig[nd++] = (unsigned char)(m - q * b);
+        dig[nd++] = m - q * b;
         m = q;
     }
     double x = 0.0;

@@ -286,6 +286,13 @@ int launch_network_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev
     time_end(c);
     c->launches++;
     VS_CUDA(cudaGetLastError());
+    if (!c->opt.trace.empty()) {                      // VS_TRACE: the form that ran (64 or 32 trajectories per CTA) and its grid
+        if (FILE *fp = fopen(c->opt.trace.c_str(), "a")) {
+            fprintf(fp, "# network_values_kernel nthr=%d gx=%u gy=%u smem=%zu rows=%llu\n", nthr, grid.x, grid.y, smem,
+                    (unsigned long long)rows);
+            fclose(fp);
+        }
+    }
     return VS_OK;
 }
 

@@ -297,6 +297,13 @@ static int launch_eval_t(vs_ctx *c, int k, bool heavy, const SourceDev &src, con
     time_end(c);
     c->launches++;
     VS_CUDA(cudaGetLastError());
+    if (!c->opt.trace.empty()) {                      // VS_TRACE: the form that ran (block size, points per thread, grid)
+        if (FILE *fp = fopen(c->opt.trace.c_str(), "a")) {
+            fprintf(fp, "# eval_values_kernel nthr=%d ppc=%d gx=%u gy=%u smem=%zu rows=%llu\n", nthr, ppc, grid.x, grid.y, smem,
+                    (unsigned long long)rows);
+            fclose(fp);
+        }
+    }
     return VS_OK;
 }
 
