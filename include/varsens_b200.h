@@ -75,11 +75,27 @@ typedef struct vs_scale {
  *                thread, 32 threads at least) is VS_ERR_UNSUPPORTED.  Two-phase route only; VS_FLAG_SEPARABLE is
  *                VS_ERR_UNSUPPORTED.  Frozen arithmetic (bit-identical to the oracle, and to RK4_CHAIN for the chain
  *                written as a network) in varsens_b200/csrc/device.cuh: MassAction.
+ *   MASS_ACTION_ADAPTIVE: the same network integrated by adaptive Dormand-Prince 5(4) with error control, its L observables
+ *                reported at NT output times (l = L*NT outputs per point).  Records, initial amounts and weights exactly as
+ *                MASS_ACTION; only the header differs, and the output times follow the weights:
+ *                  [0] S  [1] R  [2] L  [3] NT  [4] rtol  [5] atol  [6] h0  [7] max_steps
+ *                  R records of 8, S records of 2, L*S weights
+ *                  NT output times  0 < t_1 < t_2 < ... < t_NT   (integration starts at t = 0)
+ *                n_params == 8 + 8R + 2S + L*S + NT; output column m*L + o = observable o at time t_{m+1}.  Limits: those of
+ *                MASS_ACTION, 1 <= NT and L*NT <= 64, times finite and strictly increasing from > 0, rtol finite >= 0, atol
+ *                finite > 0, h0 finite > 0, 1 <= max_steps < 2^31 (an integer); anything else is VS_ERR_ARG.  Each trajectory
+ *                picks its own steps (error of a step against rtol*|X_s| + atol) and lands exactly on every output time.  A
+ *                trajectory that needs more than max_steps attempts, or whose step no longer advances t, is failed: its
+ *                outputs from the time it did not reach on are NaN (an ordinary value, see vs_last_network_stats).  State:
+ *                k + 8S + R doubles per thread, 32 threads at least, else VS_ERR_UNSUPPORTED.  Two-phase route only;
+ *                VS_FLAG_SEPARABLE is VS_ERR_UNSUPPORTED.  Frozen arithmetic in device.cuh: MassActionAdaptive.
  *
- * Every objective has l outputs per point: 1 for the first three, L for MASS_ACTION (vs_objective_outputs).  The entry
+ * Every objective has l outputs per point: 1 for the first three, L for MASS_ACTION, L*NT for MASS_ACTION_ADAPTIVE
+ * (vs_objective_outputs).  The entry
  * points that take an objective write l columns: vs_eval_values rows*(2+2k)*l doubles, vs_fused_partials
  * vs_partials_len(k, l) doubles, vs_run_fused / vs_run_fused_p2p vs_result arrays sized for l. */
-enum vs_objective { VS_OBJ_GFUNCTION = 0, VS_OBJ_ISHIGAMI = 1, VS_OBJ_RK4_CHAIN = 2, VS_OBJ_MASS_ACTION = 3 };
+enum vs_objective { VS_OBJ_GFUNCTION = 0, VS_OBJ_ISHIGAMI = 1, VS_OBJ_RK4_CHAIN = 2, VS_OBJ_MASS_ACTION = 3,
+                   VS_OBJ_MASS_ACTION_ADAPTIVE = 4 };
 
 /* fp64 arithmetic of the Halton radical inverse (the reference delegates it to the third-party ghalton package,
  * varsens/saltelli.py:82-84, whose source is not part of the reference; see DESIGN.md "parity unpinned").  The first three are
@@ -154,8 +170,9 @@ int vs_reference_permutation(uint64_t n, uint32_t seed, uint32_t *perm, uint32_t
  * i.e. exactly the combinations vs_finalize adds up (saltelli.py:612-613, 618-619); vectors from
  * vs_partials_from_values hold the plain entries.  Both kinds add up across shards and ranks. */
 size_t vs_partials_len(int k, int l);
-/* Outputs per point l of a registered objective (1, or L for VS_OBJ_MASS_ACTION) in *l, after the same validation of
- * k, objective and params the evaluating entry points run (VS_ERR_ARG on a malformed description). */
+/* Outputs per point l of a registered objective (1, L for VS_OBJ_MASS_ACTION, L*NT for VS_OBJ_MASS_ACTION_ADAPTIVE) in *l,
+ * after the same validation of k, objective and params the evaluating entry points run (VS_ERR_ARG on a malformed
+ * description). */
 int vs_objective_outputs(int k, int objective, const double *params, int n_params, int *l);
 
 /* ---- generators ---------------------------------------------------------------------------- */
@@ -270,6 +287,13 @@ int vs_last_kernel_ms(vs_ctx *ctx, float *ms);
  * group row + fence + ticket, second-level combine, packing; then that CTA's own prologue, main loop and CTA-level combine}
  * -- 11 doubles. */
 int vs_last_tail_ns(vs_ctx *ctx, int k, double *ns11);
+/* Step counts of the last call on this ctx that evaluated a VS_OBJ_MASS_ACTION_ADAPTIVE network (vs_eval_values,
+ * vs_fused_partials, vs_run_fused, vs_run_fused_p2p), over the trajectories of its base rows [i_begin, i_end) -- not the
+ * extra evaluation of base row 0 for the common shift: stats[0] accepted steps, [1] rejected steps, [2] failed trajectories,
+ * [3] lane work = the sum over warps (32 consecutive rows of one design point) of rows in the warp x the most attempts of
+ * any lane in it.  (accepted + rejected) / lane work is the share of lanes that did useful work.  Synchronises the ctx
+ * stream; VS_ERR_ARG if no adaptive network has been evaluated on this ctx. */
+int vs_last_network_stats(vs_ctx *ctx, uint64_t stats[4]);
 
 #ifdef __cplusplus
 }

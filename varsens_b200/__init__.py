@@ -7,7 +7,7 @@ C ABI in include/varsens_b200.h.  Extras: registered device functors and the ``v
 from .saltelli import Varsens, Sample, Objective
 from .scale import *          # noqa: F401,F403  (the reference star-exports linear/power/percentage/magnitude)
 from . import scale
-from .functors import GFunction, Ishigami, RK4Chain, MassActionNetwork, Param, vectorized
+from .functors import GFunction, Ishigami, RK4Chain, MassActionNetwork, AdaptiveMassActionNetwork, Param, vectorized
 from .sobol import sobol_raw, joe_kuo_direction_numbers, quantlib_direction_numbers, read_sobol_initializers
 from ._cabi import Context, VarsensError
 

@@ -15,7 +15,8 @@ LIB_PATH = os.environ.get("VS_LIB") or os.path.join(_HERE, "libvarsens_b200.so")
 VS_OK = 0
 MEM_HOST, MEM_DEVICE = 0, 1
 SCALE_IDENTITY, SCALE_LINEAR, SCALE_POWER = 0, 1, 2
-OBJ_GFUNCTION, OBJ_ISHIGAMI, OBJ_RK4_CHAIN, OBJ_MASS_ACTION = 0, 1, 2, 3
+OBJ_GFUNCTION, OBJ_ISHIGAMI, OBJ_RK4_CHAIN, OBJ_MASS_ACTION, OBJ_MASS_ACTION_ADAPTIVE = 0, 1, 2, 3, 4
+NETWORK_STATS = ("accepted", "rejected", "failed", "lane_work")      # vs_last_network_stats, in order
 FLAG_SECOND_ORDER, FLAG_SEPARABLE = 1, 2
 
 # every symbol include/varsens_b200.h declares (tests/test_cabi_symbols.py checks the header against this)
@@ -26,7 +27,7 @@ SYMBOLS = (
     "vs_finalize_device", "vs_allreduce_finalize_p2p", "vs_indices_from_values", "vs_fused_partials", "vs_run_fused", "vs_measure_fp64_peak", "vs_last_kernel_ms",
     "vs_ctx_reload_env", "vs_ctx_set_halton_mode", "vs_halton_terms_mode", "vs_run_fused_p2p", "vs_last_tail_ns",
     "vs_halton_arith_check", "vs_reference_permutation", "vs_ctx_set_timing", "vs_sample_flat_shard",
-    "vs_objective_outputs",
+    "vs_objective_outputs", "vs_last_network_stats",
 )
 HALTON_DIVIDE, HALTON_RECIPROCAL, HALTON_RUNNING_RECIPROCAL, HALTON_HORNER = 0, 1, 2, 3
 ERR_TIMEOUT = 6
@@ -110,6 +111,7 @@ def lib():
         L.vs_measure_fp64_peak.argtypes = [vp, P(ctypes.c_double)]
         L.vs_last_kernel_ms.argtypes = [vp, P(ctypes.c_float)]
         L.vs_objective_outputs.argtypes = [i32, i32, vp, i32, P(i32)]
+        L.vs_last_network_stats.argtypes = [vp, vp]
         _lib = L
         return _lib
 
@@ -124,7 +126,7 @@ def check(status):
 def objective_outputs(k, objective, params):
     """Outputs per point l of a registered objective (vs_objective_outputs: host only, validates the parameters).  Every
     objective but a mass-action network has one, known without a call."""
-    if int(objective) != OBJ_MASS_ACTION:
+    if int(objective) not in (OBJ_MASS_ACTION, OBJ_MASS_ACTION_ADAPTIVE):
         return 1
     par = numpy.ascontiguousarray(params, dtype=numpy.float64)
     l = ctypes.c_int()
@@ -303,6 +305,14 @@ class Context(object):
 
     def launch_count(self):
         return int(lib().vs_ctx_launch_count(self._h))
+
+    def network_stats(self):
+        """Step counts of the last call that evaluated an adaptive mass-action network (vs_last_network_stats), over the rows
+        it evaluated: {"accepted", "rejected", "failed" (trajectories), "lane_work"}.  (accepted + rejected) / lane_work is
+        the share of warp lanes that did useful work."""
+        a = numpy.zeros(4, dtype=numpy.uint64)
+        check(lib().vs_last_network_stats(self._h, a.ctypes.data_as(ctypes.c_void_p)))
+        return dict(zip(NETWORK_STATS, (int(v) for v in a)))
 
     def set_timing(self, on=True):
         """Record CUDA events around the main kernel of each call (read them with last_kernel_ms); off by default."""

@@ -116,7 +116,7 @@ int peer_table(vs_ctx *c, int world_size, int rank, const uint64_t *peer_bufs, c
 // Outputs per point of `objective`: 1 for every objective but a mass-action network, whose description is validated here.
 int outputs_of(int k, int objective, const double *params, int n_params, int *l) {
     *l = 1;
-    if (objective != VS_OBJ_MASS_ACTION) return VS_OK;
+    if (objective != VS_OBJ_MASS_ACTION && objective != VS_OBJ_MASS_ACTION_ADAPTIVE) return VS_OK;
     return objective_host(k, objective, params, n_params, nullptr, l);
 }
 
@@ -368,7 +368,7 @@ static int fused_step(vs_ctx *c, int k, uint64_t n, uint64_t discard, const uint
             src0.perm = (const uint32_t *)c->dir_buf.p;
         }
         double *tmp = (double *)c->misc_buf.p + 64;
-        VS_TRY(launch_eval_values(c, k, src0, s, od, 0, 1, tmp));
+        VS_TRY(launch_eval_values(c, k, src0, s, od, 0, 1, tmp, false));   // not part of the shard's step counts
         VS_CUDA(cudaMemcpyAsync(c->misc_buf.p, tmp, l * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
     }
     return launch_partials_from_values(c, k, l, rows, (const double *)c->io_buf.p, (const double *)c->misc_buf.p, flags,
@@ -451,6 +451,15 @@ extern "C" int vs_last_tail_ns(vs_ctx *c, int k, double *ns8) {
     VS_REQUIRE(c && ns8 && c->host_res, VS_ERR_ARG, "no fused step has run on this ctx");
     const double *x = c->host_res + result_len(k, 1) + HOST_RES_STAMPS;    // the fused kernel's tail has one output per point
     for (int i = 0; i < 11; ++i) ns8[i] = x[i];
+    return VS_OK;
+}
+
+extern "C" int vs_last_network_stats(vs_ctx *c, uint64_t stats[4]) {
+    VS_REQUIRE(c && stats, VS_ERR_ARG, "NULL argument");
+    VS_REQUIRE(c->stats_buf.p, VS_ERR_ARG, "no adaptive mass-action network has been evaluated on this ctx");
+    VS_CUDA(cudaSetDevice(c->device));
+    VS_CUDA(cudaMemcpyAsync(stats, c->stats_buf.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+    VS_CUDA(cudaStreamSynchronize(c->stream));
     return VS_OK;
 }
 

@@ -468,6 +468,28 @@ struct RK4ChainDyn {
 // The chain written as a network (X_s <-> X_{s+1}, kf = x[s], kr = x[S+s], X(0) = e_0, observable X_S) therefore yields the
 // same bits as RK4Chain<S> and RK4ChainDyn.
 
+// MassActionAdaptive (VS_OBJ_MASS_ACTION_ADAPTIVE; kernel network_adaptive_kernel in kernels_network.cu).  FROZEN ARITHMETIC,
+// restated bit for bit by the oracle (tests/adaptive_oracle.c).  Only correctly rounded operations (+ - * /, fma, sqrt, fabs,
+// fmax, fmin): CUDA and glibc round pow, exp and log differently, so the step-size controller uses none of them.
+//   right-hand side   MassAction's P, flux_r and d_s above.
+//   tableau           Dormand-Prince 5(4), Hairer-Norsett-Wanner I, Table 5.2: a_ij, and e_j = b_j - bhat_j, each the
+//                     correctly rounded double of its rational (dp5:: in kernels_network.cu).
+//   start             t = 0.0, h = h0, K1 = f(X).  attempts = 0.
+//   attempt           to = the next output time; hs = h, or hs = to - t (clipped) if t + h >= to.  If attempts == max_steps,
+//                     or t + hs == t: the trajectory has failed, outputs of this and every later time are NaN, stop.
+//                     Else attempts += 1 and, for stage i = 2..7: acc = 0.0, acc = fma(a_ij, K_j[s], acc) over the j with
+//                     a_ij != 0, ascending; Y[s] = fma(hs, acc, X[s]); K_i = f(Y).  Y after stage 7 is the 5th-order
+//                     solution, K7 = f(Y) (stored in K2's slot).
+//   error             E_s = hs * (fma chain of e_j K_j[s] from 0.0, j = 1, 3, 4, 5, 6, 7);  sc_s = fma(rtol, fmax(|X_s|, |Y_s|),
+//                     atol);  r = E_s / sc_s;  q = fma(r, r, q) from 0.0 over ascending s;  err = sqrt(q / S).
+//   controller        fac_max = 1.0 on the attempt after a rejection, else 5.0.  fac = fac_max if err == 0; 0.2 if err is
+//                     not finite; else fmin(fac_max, fmax(0.2, 0.9 / sqrt(sqrt(err)))).  (Exponent 1/4 rather than the
+//                     textbook 1/5: two square roots.)
+//   accept iff err <= 1.0:  t = to if clipped, else t + hs;  X = Y;  K1 = K7 (FSAL: each attempt costs 6 right-hand sides,
+//                     the first step 7; a rejected attempt keeps K1).  At a clipped step the L observables at `to` are
+//                     MassAction's: acc = fma(w[o][s], X_s, acc) from 0.0 over the nonzero weights, ascending s.
+//   next step         h = hs * fac (accepted or not).
+
 __host__ __device__ __forceinline__ void tile_coords(int id, int nt, int &tr, int &tc) {
     tr = 0;
     int rowlen = nt;

@@ -331,7 +331,8 @@ int objective_host(int k, int objective, const double *params, int n_params, std
         h.assign(params, params + 2);
         break;
     case VS_OBJ_MASS_ACTION:
-        return network_describe(k, params, n_params, hp, l);
+    case VS_OBJ_MASS_ACTION_ADAPTIVE:
+        return network_describe(k, objective, params, n_params, hp, l);
     default:
         set_error("unknown objective id %d", objective);
         return VS_ERR_ARG;
@@ -442,7 +443,7 @@ extern "C" int vs_ctx_destroy(vs_ctx *c) {
     cudaStreamSynchronize(c->copy_stream);
     if (c->host_res) cudaFreeHost(c->host_res);
     DevBuf *bufs[] = {&c->poll_buf, &c->ticket_buf, &c->peer_buf, &c->pipe_buf, &c->scale_buf, &c->obj_buf, &c->perm_buf, &c->raw_buf, &c->io_buf,
-                      &c->part_buf,  &c->block_buf, &c->res_buf, &c->dir_buf, &c->misc_buf};
+                      &c->part_buf,  &c->block_buf, &c->res_buf, &c->dir_buf, &c->misc_buf, &c->stats_buf};
     for (DevBuf *b : bufs)
         if (b->p) cudaFree(b->p);
     if (c->halton.blob) cudaFree(c->halton.blob);

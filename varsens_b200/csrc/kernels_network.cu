@@ -1,5 +1,6 @@
-// Mass-action reaction networks (VS_OBJ_MASS_ACTION): host validation of the packed description, and the two-phase
-// evaluation kernel that integrates one trajectory per design point.  Frozen arithmetic: device.cuh, MassAction.
+// Mass-action reaction networks (VS_OBJ_MASS_ACTION, VS_OBJ_MASS_ACTION_ADAPTIVE): host validation of the packed description,
+// and the two-phase evaluation kernels that integrate one trajectory per design point, by fixed-step RK4 or by adaptive
+// Dormand-Prince 5(4).  Frozen arithmetic: device.cuh, MassAction and MassActionAdaptive.
 #include "device.cuh"
 
 #include <cmath>
@@ -11,7 +12,7 @@ namespace {
 
 constexpr int NET_MAX_S = 128, NET_MAX_R = 512, NET_MAX_L = 64;
 constexpr int NET_IRREV = -2;       // kr coordinate of an irreversible reaction in the derived table
-constexpr int NET_HDR = 5, NET_REC = 8;
+constexpr int NET_HDR = 5, NET_HDR_ADAPTIVE = 8, NET_REC = 8;
 
 bool int_in(double v, double lo, double hi, int *out) {
     if (!std::isfinite(v) || v != std::floor(v) || v < lo || v > hi) return false;
@@ -27,21 +28,35 @@ bool int_in(double v, double lo, double hi, int *out) {
 //                                                                      irreversible reaction)
 //   ptr  S+1, ent nnz:   species-major stoichiometry, ent = r*8 + (c+2), c in {-2,-1,1,2}, reactions ascending per species
 //   optr L+1, oent 2*nobs: observable-major (species, weight) of the nonzero weights, species ascending
+// An adaptive description (NT > 0) has its NT output times at o_times, after the weights.
 struct NetLayout {
     int S, R, L, nsteps, nnz, nobs;
     double dt;
     int o_init, o_rx, o_ptr, o_ent, o_optr, o_oent;
+    int NT, max_steps, o_times;               // NT = 0: fixed step
+    double rtol, atol, h0;
 };
 
-static NetLayout net_layout(const double *h) {
-    NetLayout n;
+static NetLayout net_layout(const double *h, int objective) {
+    NetLayout n{};
     n.S = (int)h[0];
     n.R = (int)h[1];
     n.L = (int)h[2];
-    n.dt = h[3];
-    n.nsteps = (int)h[4];
-    n.o_init = NET_HDR + NET_REC * n.R;
-    const int np = n.o_init + 2 * n.S + n.L * n.S;
+    int hdr = NET_HDR;
+    if (objective == VS_OBJ_MASS_ACTION_ADAPTIVE) {
+        hdr = NET_HDR_ADAPTIVE;
+        n.NT = (int)h[3];
+        n.rtol = h[4];
+        n.atol = h[5];
+        n.h0 = h[6];
+        n.max_steps = (int)h[7];
+    } else {
+        n.dt = h[3];
+        n.nsteps = (int)h[4];
+    }
+    n.o_init = hdr + NET_REC * n.R;
+    n.o_times = n.o_init + 2 * n.S + n.L * n.S;
+    const int np = n.o_times + n.NT;
     n.nnz = (int)h[np];
     n.nobs = (int)h[np + 1];
     n.o_rx = np + 2;
@@ -52,23 +67,39 @@ static NetLayout net_layout(const double *h) {
     return n;
 }
 
-int network_describe(int k, const double *p, int n_params, std::vector<double> *h, int *l) {
-    VS_REQUIRE(p && n_params >= NET_HDR, VS_ERR_ARG, "mass-action network: %d parameters, the header alone has %d", n_params,
-               NET_HDR);
-    int S = 0, R = 0, L = 0, nsteps = 0, v = 0;
+int network_describe(int k, int objective, const double *p, int n_params, std::vector<double> *h, int *l) {
+    const bool adaptive = objective == VS_OBJ_MASS_ACTION_ADAPTIVE;
+    const int hdr = adaptive ? NET_HDR_ADAPTIVE : NET_HDR;
+    VS_REQUIRE(p && n_params >= hdr, VS_ERR_ARG, "mass-action network: %d parameters, the header alone has %d", n_params, hdr);
+    int S = 0, R = 0, L = 0, nsteps = 0, NT = 0, v = 0;
     VS_REQUIRE(int_in(p[0], 1, NET_MAX_S, &S), VS_ERR_ARG, "mass-action network: S = %g, need an integer in [1,%d]", p[0], NET_MAX_S);
     VS_REQUIRE(int_in(p[1], 1, NET_MAX_R, &R), VS_ERR_ARG, "mass-action network: R = %g, need an integer in [1,%d]", p[1], NET_MAX_R);
     VS_REQUIRE(int_in(p[2], 1, NET_MAX_L, &L), VS_ERR_ARG, "mass-action network: L = %g, need an integer in [1,%d]", p[2], NET_MAX_L);
-    VS_REQUIRE(std::isfinite(p[3]), VS_ERR_ARG, "mass-action network: dt = %g is not finite", p[3]);
-    VS_REQUIRE(int_in(p[4], 0, 2147483647.0, &nsteps), VS_ERR_ARG, "mass-action network: nsteps = %g, need an integer in [0,2^31)",
-               p[4]);
-    const long long want = NET_HDR + (long long)NET_REC * R + 2ll * S + (long long)L * S;
-    VS_REQUIRE(n_params == want, VS_ERR_ARG, "mass-action network with S=%d, R=%d, L=%d needs %lld parameters, got %d", S, R, L,
-               want, n_params);
+    if (adaptive) {
+        VS_REQUIRE(int_in(p[3], 1, NET_MAX_L, &NT) && L * NT <= NET_MAX_L, VS_ERR_ARG,
+                   "adaptive mass-action network: NT = %g output times of L = %d observables, need NT >= 1 and L*NT <= %d", p[3], L,
+                   NET_MAX_L);
+        VS_REQUIRE(std::isfinite(p[4]) && p[4] >= 0.0, VS_ERR_ARG, "adaptive mass-action network: rtol = %g, need finite >= 0", p[4]);
+        VS_REQUIRE(std::isfinite(p[5]) && p[5] > 0.0, VS_ERR_ARG, "adaptive mass-action network: atol = %g, need finite > 0", p[5]);
+        VS_REQUIRE(std::isfinite(p[6]) && p[6] > 0.0, VS_ERR_ARG, "adaptive mass-action network: h0 = %g, need finite > 0", p[6]);
+        VS_REQUIRE(int_in(p[7], 1, 2147483647.0, &v), VS_ERR_ARG,
+                   "adaptive mass-action network: max_steps = %g, need an integer in [1,2^31)", p[7]);
+    } else {
+        VS_REQUIRE(std::isfinite(p[3]), VS_ERR_ARG, "mass-action network: dt = %g is not finite", p[3]);
+        VS_REQUIRE(int_in(p[4], 0, 2147483647.0, &nsteps), VS_ERR_ARG,
+                   "mass-action network: nsteps = %g, need an integer in [0,2^31)", p[4]);
+    }
+    const long long want = hdr + (long long)NET_REC * R + 2ll * S + (long long)L * S + NT;
+    VS_REQUIRE(n_params == want, VS_ERR_ARG, "mass-action network with S=%d, R=%d, L=%d, NT=%d needs %lld parameters, got %d", S, R,
+               L, NT, want, n_params);
+    const double *times = p + want - NT;
+    for (int m = 0; m < NT; ++m)
+        VS_REQUIRE(std::isfinite(times[m]) && times[m] > (m ? times[m - 1] : 0.0), VS_ERR_ARG,
+                   "adaptive mass-action network: output time %d = %g, need finite times with 0 < t_1 < t_2 < ...", m + 1, times[m]);
     std::vector<double> rx((size_t)NET_REC * R);
     std::vector<std::vector<int>> lists(S);
     for (int r = 0; r < R; ++r) {
-        const double *q = p + NET_HDR + (size_t)NET_REC * r;
+        const double *q = p + hdr + (size_t)NET_REC * r;
         int sp[4];
         for (int e = 0; e < 4; ++e)
             VS_REQUIRE(int_in(q[e], -1, S - 1, &sp[e]), VS_ERR_ARG,
@@ -97,12 +128,12 @@ int network_describe(int k, const double *p, int n_params, std::vector<double> *
         }
     }
     for (int s = 0; s < S; ++s) {
-        const double *q = p + NET_HDR + (size_t)NET_REC * R + 2 * (size_t)s;
+        const double *q = p + hdr + (size_t)NET_REC * R + 2 * (size_t)s;
         VS_REQUIRE(int_in(q[0], -1, k - 1, &v), VS_ERR_ARG,
                    "mass-action network: species %d, initial-amount coordinate %g, need -1 or an integer in [0,k=%d)", s, q[0], k);
     }
     if (h) {
-        const double *w = p + NET_HDR + (size_t)NET_REC * R + 2 * (size_t)S;
+        const double *w = p + hdr + (size_t)NET_REC * R + 2 * (size_t)S;
         h->assign(p, p + n_params);
         int nnz = 0, nobs = 0;
         for (int s = 0; s < S; ++s) nnz += (int)lists[s].size();
@@ -124,9 +155,10 @@ int network_describe(int k, const double *p, int n_params, std::vector<double> *
             for (int s = 0; s < S; ++s)
                 if (w[(size_t)o * S + s] != 0.0) { h->push_back(s); h->push_back(w[(size_t)o * S + s]); }
     }
-    *l = L;
+    *l = adaptive ? L * NT : L;
     return VS_OK;
 }
+
 
 // ---------------------------------------------------------------------------------------------------------------------
 // One thread per design point of a base row (the work split of eval_values_kernel's heavy route: grid.y = the 2+2k points).
@@ -142,6 +174,15 @@ struct NetDev {
     NetLayout n;
 };
 
+// The reaction and stoichiometry tables in shared memory (net_load_tables).
+struct NetTables {
+    const double2 *rk;      // R: kf const, kr const
+    const int4 *ri;         // R: a0 a1 b0 b1
+    const int2 *rc;         // R: kf coord, kr coord
+    const int *cptr;        // S+1
+    const int *cent;        // nnz
+};
+
 constexpr int NET_THREADS = 64;
 
 __host__ __device__ static size_t net_table_bytes(const NetLayout &n) {
@@ -149,20 +190,27 @@ __host__ __device__ static size_t net_table_bytes(const NetLayout &n) {
     return (b + 15) / 16 * 16;
 }
 
+// The adaptive kernel adds the output times and the observable lists (times[NT], weights[nobs], optr[L+1], species[nobs]), so
+// that its step loop reads nothing from global memory.
+__host__ __device__ static size_t net_adaptive_table_bytes(const NetLayout &n) {
+    const size_t b = 8 * (size_t)(n.NT + n.nobs) + 4 * (size_t)(n.L + 1 + n.nobs);
+    return net_table_bytes(n) + (b + 15) / 16 * 16;
+}
+
 static size_t net_smem(const NetLayout &n, int k, int nthr) {
+    if (n.NT) return net_adaptive_table_bytes(n) + (size_t)(k + 8 * n.S + n.R) * nthr * sizeof(double);
     return net_table_bytes(n) + (size_t)(k + 3 * n.S + n.R) * nthr * sizeof(double);
 }
 
-__global__ void __launch_bounds__(NET_THREADS) network_values_kernel(int k, SourceDev src, ScaleDev s, NetDev net, uint64_t i_begin,
-                                                                     uint64_t i_end, double *__restrict__ fvals) {
-    extern __shared__ __align__(16) double smem[];
+// Every thread of the CTA copies its share of the tables; the caller synchronises.
+__device__ __forceinline__ NetTables net_load_tables(double *smem, const NetDev &net) {
     const NetLayout &n = net.n;
     const int S = n.S, R = n.R, nthr = blockDim.x, tid = threadIdx.x;
-    double2 *rk = reinterpret_cast<double2 *>(smem);              // R: kf const, kr const
-    int4 *ri = reinterpret_cast<int4 *>(rk + R);                  // R: a0 a1 b0 b1
-    int2 *rc = reinterpret_cast<int2 *>(ri + R);                  // R: kf coord, kr coord
-    int *cptr = reinterpret_cast<int *>(rc + R);                  // S+1
-    int *cent = cptr + S + 1;                                     // nnz
+    double2 *rk = reinterpret_cast<double2 *>(smem);
+    int4 *ri = reinterpret_cast<int4 *>(rk + R);
+    int2 *rc = reinterpret_cast<int2 *>(ri + R);
+    int *cptr = reinterpret_cast<int *>(rc + R);
+    int *cent = cptr + S + 1;
     for (int r = tid; r < R; r += nthr) {
         const double *q = net.tab + n.o_rx + (size_t)NET_REC * r;
         ri[r] = make_int4((int)q[0], (int)q[1], (int)q[2], (int)q[3]);
@@ -171,82 +219,99 @@ __global__ void __launch_bounds__(NET_THREADS) network_values_kernel(int k, Sour
     }
     for (int e = tid; e <= S; e += nthr) cptr[e] = (int)net.tab[n.o_ptr + e];
     for (int e = tid; e < n.nnz; e += nthr) cent[e] = (int)net.tab[n.o_ent + e];
-    __syncthreads();
-    const uint64_t rows = i_end - i_begin;
-    const uint64_t row = (uint64_t)blockIdx.x * nthr + tid;
-    if (row >= rows) return;
-    double *x = smem + net_table_bytes(n) / sizeof(double) + tid;   // x[c * nthr]
-    double *X = x + (size_t)k * nthr, *T = X + (size_t)S * nthr, *A = T + (size_t)S * nthr, *F = A + (size_t)S * nthr;
-    const uint64_t i = i_begin + row, pi = src.perm[i];
-    const int p = blockIdx.y;
+    return NetTables{rk, ri, rc, cptr, cent};
+}
+
+// The scaled coordinates x of design point p (grid.y) of base row i, and the initial state X.
+__device__ __forceinline__ void net_point(int k, const SourceDev &src, const ScaleDev &s, const NetDev &net, uint64_t i, int p,
+                                          double *x, double *X, int nthr) {
+    const uint64_t pi = src.perm[i];
     const int j = p < 2 ? -1 : (p < 2 + k ? p - 2 : p - 2 - k);
     const bool base_a = p == 0 || p >= 2 + k;                     // M_1 and N_nj start from A_i, M_2 and N_j from B_i
     for (int c = 0; c < k; ++c) {
         const bool from_a = (c == j) ? !base_a : base_a;
         x[c * nthr] = from_a ? apply_scale(s, c, source_a(src, k, i, c)) : apply_scale(s, c, source_b(src, k, pi, c));
     }
-    for (int sp = 0; sp < S; ++sp) {
-        const double *q = net.tab + n.o_init + 2 * sp;
+    for (int sp = 0; sp < net.n.S; ++sp) {
+        const double *q = net.tab + net.n.o_init + 2 * sp;
         const int ic = (int)q[0];
         X[sp * nthr] = ic >= 0 ? x[ic * nthr] : q[1];
     }
-    const double dt = n.dt, h2 = __dmul_rn(0.5, dt), h6 = __ddiv_rn(dt, 6.0);
-    // fluxes of state Y into F
-    auto fluxes = [&](const double *Y) {
+}
+
+// fluxes of state Y into F
+__device__ __forceinline__ void net_fluxes(const NetTables &t, int R, int nthr, const double *x, const double *Y, double *F) {
 #pragma unroll 4
-        for (int r = 0; r < R; ++r) {
-            const int4 sp = ri[r];
-            const int2 cc = rc[r];
-            const double2 kc = rk[r];
-            const double kf = cc.x >= 0 ? x[cc.x * nthr] : kc.x;
-            const double pf = sp.x < 0 ? 1.0 : (sp.y < 0 ? Y[sp.x * nthr] : __dmul_rn(Y[sp.x * nthr], Y[sp.y * nthr]));
-            double f;
-            if (cc.y == NET_IRREV) {
-                f = __dmul_rn(kf, pf);
-            } else {
-                const double kr = cc.y >= 0 ? x[cc.y * nthr] : kc.y;
-                const double pr = sp.z < 0 ? 1.0 : (sp.w < 0 ? Y[sp.z * nthr] : __dmul_rn(Y[sp.z * nthr], Y[sp.w * nthr]));
-                f = fma(kf, pf, -__dmul_rn(kr, pr));
-            }
-            F[r * nthr] = f;
+    for (int r = 0; r < R; ++r) {
+        const int4 sp = t.ri[r];
+        const int2 cc = t.rc[r];
+        const double2 kc = t.rk[r];
+        const double kf = cc.x >= 0 ? x[cc.x * nthr] : kc.x;
+        const double pf = sp.x < 0 ? 1.0 : (sp.y < 0 ? Y[sp.x * nthr] : __dmul_rn(Y[sp.x * nthr], Y[sp.y * nthr]));
+        double f;
+        if (cc.y == NET_IRREV) {
+            f = __dmul_rn(kf, pf);
+        } else {
+            const double kr = cc.y >= 0 ? x[cc.y * nthr] : kc.y;
+            const double pr = sp.z < 0 ? 1.0 : (sp.w < 0 ? Y[sp.z * nthr] : __dmul_rn(Y[sp.z * nthr], Y[sp.w * nthr]));
+            f = fma(kf, pf, -__dmul_rn(kr, pr));
         }
-    };
-    // d_s of species sp from the stored fluxes, ascending reaction order
-    auto deriv = [&](int sp) {
-        double d = 0.0;
-        const int e1 = cptr[sp + 1];
-        for (int e = cptr[sp]; e < e1; ++e) {
-            const int code = cent[e];
-            const int c = (code & 7) - 2;
-            const double fl = F[(code >> 3) * nthr];
-            if (c == 1) d = __dadd_rn(d, fl);
-            else if (c == -1) d = __dsub_rn(d, fl);
-            else d = fma((double)c, fl, d);
-        }
-        return d;
-    };
+        F[r * nthr] = f;
+    }
+}
+
+// d_s of species sp from the stored fluxes, ascending reaction order
+__device__ __forceinline__ double net_deriv(const NetTables &t, int nthr, const double *F, int sp) {
+    double d = 0.0;
+    const int e1 = t.cptr[sp + 1];
+    for (int e = t.cptr[sp]; e < e1; ++e) {
+        const int code = t.cent[e];
+        const int c = (code & 7) - 2;
+        const double fl = F[(code >> 3) * nthr];
+        if (c == 1) d = __dadd_rn(d, fl);
+        else if (c == -1) d = __dsub_rn(d, fl);
+        else d = fma((double)c, fl, d);
+    }
+    return d;
+}
+
+__global__ void __launch_bounds__(NET_THREADS) network_values_kernel(int k, SourceDev src, ScaleDev s, NetDev net, uint64_t i_begin,
+                                                                     uint64_t i_end, double *__restrict__ fvals) {
+    extern __shared__ __align__(16) double smem[];
+    const NetLayout &n = net.n;
+    const int S = n.S, R = n.R, nthr = blockDim.x, tid = threadIdx.x;
+    const NetTables tb = net_load_tables(smem, net);
+    __syncthreads();
+    const uint64_t rows = i_end - i_begin;
+    const uint64_t row = (uint64_t)blockIdx.x * nthr + tid;
+    if (row >= rows) return;
+    double *x = smem + net_table_bytes(n) / sizeof(double) + tid;   // x[c * nthr]
+    double *X = x + (size_t)k * nthr, *T = X + (size_t)S * nthr, *A = T + (size_t)S * nthr, *F = A + (size_t)S * nthr;
+    const int p = blockIdx.y;
+    net_point(k, src, s, net, i_begin + row, p, x, X, nthr);
+    const double dt = n.dt, h2 = __dmul_rn(0.5, dt), h6 = __ddiv_rn(dt, 6.0);
     for (int it = 0; it < n.nsteps; ++it) {
-        fluxes(X);                                                // k1
+        net_fluxes(tb, R, nthr, x, X, F);                         // k1
         for (int sp = 0; sp < S; ++sp) {
-            const double d = deriv(sp);
+            const double d = net_deriv(tb, nthr, F, sp);
             A[sp * nthr] = d;
             T[sp * nthr] = fma(h2, d, X[sp * nthr]);
         }
-        fluxes(T);                                                // k2
+        net_fluxes(tb, R, nthr, x, T, F);                         // k2
         for (int sp = 0; sp < S; ++sp) {
-            const double d = deriv(sp);
+            const double d = net_deriv(tb, nthr, F, sp);
             A[sp * nthr] = fma(2.0, d, A[sp * nthr]);
             T[sp * nthr] = fma(h2, d, X[sp * nthr]);
         }
-        fluxes(T);                                                // k3
+        net_fluxes(tb, R, nthr, x, T, F);                         // k3
         for (int sp = 0; sp < S; ++sp) {
-            const double d = deriv(sp);
+            const double d = net_deriv(tb, nthr, F, sp);
             A[sp * nthr] = fma(2.0, d, A[sp * nthr]);
             T[sp * nthr] = fma(dt, d, X[sp * nthr]);
         }
-        fluxes(T);                                                // k4
+        net_fluxes(tb, R, nthr, x, T, F);                         // k4
         for (int sp = 0; sp < S; ++sp) {
-            const double d = deriv(sp);
+            const double d = net_deriv(tb, nthr, F, sp);
             X[sp * nthr] = fma(h6, __dadd_rn(A[sp * nthr], d), X[sp * nthr]);
         }
     }
@@ -263,8 +328,167 @@ __global__ void __launch_bounds__(NET_THREADS) network_values_kernel(int k, Sour
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Adaptive Dormand-Prince 5(4) (VS_OBJ_MASS_ACTION_ADAPTIVE): the work split and tables of network_values_kernel, plus the
+// output times and observable lists in shared memory.  Per-trajectory state, [variable][thread]:
+//   x[k], X[S] the state at t, Y[S] the stage input (Y7 = the 5th-order solution), K[6][S] the stage derivatives K1..K6 (K7 is
+//   written into K2's slot, dead after stage 6; on acceptance the two slots swap roles, so K7 becomes the next K1: FSAL), F[R].
+// Each trajectory picks its own steps; a step that would pass the next output time is clipped to land on it, and the L
+// observables are written there.  Nothing else touches global memory inside the step loop.  Counts (accepted, rejected,
+// failed, lane work) are reduced per warp and added with one atomicAdd each when `stats` is set.
+// ---------------------------------------------------------------------------------------------------------------------
+namespace dp5 {   // Hairer-Norsett-Wanner I, Table 5.2; each coefficient the correctly rounded double of its rational
+constexpr double A21 = 1.0 / 5.0;
+constexpr double A31 = 3.0 / 40.0, A32 = 9.0 / 40.0;
+constexpr double A41 = 44.0 / 45.0, A42 = -56.0 / 15.0, A43 = 32.0 / 9.0;
+constexpr double A51 = 19372.0 / 6561.0, A52 = -25360.0 / 2187.0, A53 = 64448.0 / 6561.0, A54 = -212.0 / 729.0;
+constexpr double A61 = 9017.0 / 3168.0, A62 = -355.0 / 33.0, A63 = 46732.0 / 5247.0, A64 = 49.0 / 176.0, A65 = -5103.0 / 18656.0;
+constexpr double A71 = 35.0 / 384.0, A73 = 500.0 / 1113.0, A74 = 125.0 / 192.0, A75 = -2187.0 / 6784.0, A76 = 11.0 / 84.0;
+// e_j = b_j - bhat_j (b = row 7 of a)
+constexpr double E1 = 71.0 / 57600.0, E3 = -71.0 / 16695.0, E4 = 71.0 / 1920.0, E5 = -17253.0 / 339200.0, E6 = 22.0 / 525.0,
+                 E7 = -1.0 / 40.0;
+}  // namespace dp5
+
+// Y = fma(h, acc, X) with acc = fma(a_j, K_j, acc) from 0.0 over the NJ given stages, ascending
+template <int NJ>
+__device__ __forceinline__ void dp5_stage_input(const double (&a)[NJ], const double *const (&K)[NJ], double h, const double *X,
+                                                double *Y, int S, int nthr) {
+    for (int sp = 0; sp < S; ++sp) {
+        double acc = 0.0;
+#pragma unroll
+        for (int j = 0; j < NJ; ++j) acc = fma(a[j], K[j][sp * nthr], acc);
+        Y[sp * nthr] = fma(h, acc, X[sp * nthr]);
+    }
+}
+
+__device__ __forceinline__ void net_rhs(const NetTables &t, int S, int R, int nthr, const double *x, const double *Y, double *F,
+                                        double *D) {
+    net_fluxes(t, R, nthr, x, Y, F);
+    for (int sp = 0; sp < S; ++sp) D[sp * nthr] = net_deriv(t, nthr, F, sp);
+}
+
+__global__ void __launch_bounds__(NET_THREADS) network_adaptive_kernel(int k, SourceDev src, ScaleDev s, NetDev net, uint64_t i_begin,
+                                                                       uint64_t i_end, double *__restrict__ fvals,
+                                                                       unsigned long long *__restrict__ stats) {
+    extern __shared__ __align__(16) double smem[];
+    const NetLayout &n = net.n;
+    const int S = n.S, R = n.R, L = n.L, NT = n.NT, nthr = blockDim.x, tid = threadIdx.x;
+    const NetTables tb = net_load_tables(smem, net);
+    double *tout = smem + net_table_bytes(n) / sizeof(double);   // NT output times
+    double *ow = tout + NT;                                        // nobs observable weights
+    int *optr = reinterpret_cast<int *>(ow + n.nobs);              // L+1
+    int *osp = optr + L + 1;                                       // nobs species
+    for (int e = tid; e < NT; e += nthr) tout[e] = net.tab[n.o_times + e];
+    for (int e = tid; e <= L; e += nthr) optr[e] = (int)net.tab[n.o_optr + e];
+    for (int e = tid; e < n.nobs; e += nthr) {
+        osp[e] = (int)net.tab[n.o_oent + 2 * e];
+        ow[e] = net.tab[n.o_oent + 2 * e + 1];
+    }
+    __syncthreads();
+    const uint64_t rows = i_end - i_begin;
+    const uint64_t row = (uint64_t)blockIdx.x * nthr + tid;
+    const bool valid = row < rows;                                 // every lane stays for the warp reduction of the counts
+    unsigned attempts = 0, accepted = 0;
+    bool failed = false;
+    if (valid) {
+        double *x = smem + net_adaptive_table_bytes(n) / sizeof(double) + tid;
+        const size_t sl = (size_t)S * nthr;
+        double *X = x + (size_t)k * nthr, *Y = X + sl, *Kb = Y + sl, *F = Kb + 6 * sl;
+        const int p = blockIdx.y;
+        net_point(k, src, s, net, i_begin + row, p, x, X, nthr);
+        double *out = fvals + ((uint64_t)p * rows + row) * (uint64_t)(L * NT);
+        const double rtol = n.rtol, atol = n.atol;
+        const unsigned max_steps = (unsigned)n.max_steps;
+        int k1 = 0;                                                // slot of K1; K2 (and K7) in slot 1 - k1
+        net_rhs(tb, S, R, nthr, x, X, F, Kb);
+        double t = 0.0, h = n.h0;
+        bool after_reject = false;
+        for (int m = 0; m < NT;) {
+            const double to = tout[m];
+            double hs = h;
+            const bool clip = __dadd_rn(t, hs) >= to;
+            if (clip) hs = __dsub_rn(to, t);
+            if (attempts == max_steps || __dadd_rn(t, hs) == t) {   // failed: this and the later output times are NaN
+                for (int e = m * L; e < NT * L; ++e) out[e] = __longlong_as_double(0x7ff8000000000000ll);
+                failed = true;
+                break;
+            }
+            ++attempts;
+            const double *K1 = Kb + k1 * sl;
+            double *K2 = Kb + (1 - k1) * sl, *K3 = Kb + 2 * sl, *K4 = Kb + 3 * sl, *K5 = Kb + 4 * sl, *K6 = Kb + 5 * sl;
+            dp5_stage_input<1>({dp5::A21}, {K1}, hs, X, Y, S, nthr);
+            net_rhs(tb, S, R, nthr, x, Y, F, K2);
+            dp5_stage_input<2>({dp5::A31, dp5::A32}, {K1, K2}, hs, X, Y, S, nthr);
+            net_rhs(tb, S, R, nthr, x, Y, F, K3);
+            dp5_stage_input<3>({dp5::A41, dp5::A42, dp5::A43}, {K1, K2, K3}, hs, X, Y, S, nthr);
+            net_rhs(tb, S, R, nthr, x, Y, F, K4);
+            dp5_stage_input<4>({dp5::A51, dp5::A52, dp5::A53, dp5::A54}, {K1, K2, K3, K4}, hs, X, Y, S, nthr);
+            net_rhs(tb, S, R, nthr, x, Y, F, K5);
+            dp5_stage_input<5>({dp5::A61, dp5::A62, dp5::A63, dp5::A64, dp5::A65}, {K1, K2, K3, K4, K5}, hs, X, Y, S, nthr);
+            net_rhs(tb, S, R, nthr, x, Y, F, K6);
+            dp5_stage_input<5>({dp5::A71, dp5::A73, dp5::A74, dp5::A75, dp5::A76}, {K1, K3, K4, K5, K6}, hs, X, Y, S, nthr);
+            double *K7 = K2;
+            net_rhs(tb, S, R, nthr, x, Y, F, K7);
+            double q = 0.0;
+            for (int sp = 0; sp < S; ++sp) {
+                const int v = sp * nthr;
+                double e = fma(dp5::E1, K1[v], 0.0);
+                e = fma(dp5::E3, K3[v], e);
+                e = fma(dp5::E4, K4[v], e);
+                e = fma(dp5::E5, K5[v], e);
+                e = fma(dp5::E6, K6[v], e);
+                e = fma(dp5::E7, K7[v], e);
+                const double sc = fma(rtol, fmax(fabs(X[v]), fabs(Y[v])), atol);
+                const double r = __ddiv_rn(__dmul_rn(hs, e), sc);
+                q = fma(r, r, q);
+            }
+            const double err = __dsqrt_rn(__ddiv_rn(q, (double)S));
+            const double fac_max = after_reject ? 1.0 : 5.0;
+            const double fac = err == 0.0 ? fac_max
+                               : isfinite(err) ? fmin(fac_max, fmax(0.2, __ddiv_rn(0.9, __dsqrt_rn(__dsqrt_rn(err)))))
+                                               : 0.2;
+            if (err <= 1.0) {
+                ++accepted;
+                t = clip ? to : __dadd_rn(t, hs);
+                double *old = X;
+                X = Y;
+                Y = old;
+                k1 = 1 - k1;
+                after_reject = false;
+                if (clip) {
+                    for (int o = 0; o < L; ++o) {
+                        double acc = 0.0;
+                        for (int e = optr[o]; e < optr[o + 1]; ++e) acc = fma(ow[e], X[osp[e] * nthr], acc);
+                        out[m * L + o] = acc;
+                    }
+                    ++m;
+                }
+            } else {
+                after_reject = true;
+            }
+            h = __dmul_rn(hs, fac);
+        }
+    }
+    if (stats) {
+        unsigned long long a = accepted, r = attempts - accepted, f = failed;
+        for (int o = 16; o; o >>= 1) {
+            a += __shfl_xor_sync(0xffffffffu, a, o);
+            r += __shfl_xor_sync(0xffffffffu, r, o);
+            f += __shfl_xor_sync(0xffffffffu, f, o);
+        }
+        const unsigned most = __reduce_max_sync(0xffffffffu, attempts);
+        const unsigned lanes = __popc(__ballot_sync(0xffffffffu, valid));
+        if ((tid & 31) == 0 && lanes) {
+            atomicAdd(stats + 0, a);
+            atomicAdd(stats + 1, r);
+            atomicAdd(stats + 2, f);
+            atomicAdd(stats + 3, (unsigned long long)lanes * most);
+        }
+    }
+}
+
 int network_check_fit(vs_ctx *c, int k, const ObjectiveDev &o) {
-    const NetLayout n = net_layout(o.host);
+    const NetLayout n = net_layout(o.host, o.id);
     VS_REQUIRE(net_smem(n, k, 32) <= c->smem_optin, VS_ERR_UNSUPPORTED,
                "mass-action network with k=%d, S=%d, R=%d needs %zu bytes of shared memory for 32 trajectories, the device has %zu",
                k, n.S, n.R, net_smem(n, k, 32), c->smem_optin);
@@ -272,24 +496,37 @@ int network_check_fit(vs_ctx *c, int k, const ObjectiveDev &o) {
 }
 
 int launch_network_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, const ObjectiveDev &o, uint64_t i_begin,
-                          uint64_t i_end, double *fvals) {
+                          uint64_t i_end, double *fvals, bool count) {
     VS_TRY(network_check_fit(c, k, o));
     const uint64_t rows = i_end - i_begin;
     if (rows == 0) return VS_OK;
-    NetDev net{o.params, net_layout(o.host)};
+    NetDev net{o.params, net_layout(o.host, o.id)};
+    const bool adaptive = net.n.NT > 0;
+    unsigned long long *stats = nullptr;
+    if (adaptive && count) {                          // vs_last_network_stats: the counts of this call only
+        VS_TRY(ensure(c, c->stats_buf, 4 * sizeof(unsigned long long)));
+        stats = (unsigned long long *)c->stats_buf.p;
+        VS_CUDA(cudaMemsetAsync(stats, 0, 4 * sizeof(unsigned long long), c->stream));
+    }
     const int nthr = net_smem(net.n, k, NET_THREADS) <= c->smem_optin ? NET_THREADS : 32;
     const size_t smem = net_smem(net.n, k, nthr);
-    VS_CUDA(cudaFuncSetAttribute(network_values_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid((unsigned)((rows + nthr - 1) / nthr), (unsigned)(2 + 2 * k));
-    time_begin(c);
-    network_values_kernel<<<grid, nthr, smem, c->stream>>>(k, src, s, net, i_begin, i_end, fvals);
+    if (adaptive) {
+        VS_CUDA(cudaFuncSetAttribute(network_adaptive_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        time_begin(c);
+        network_adaptive_kernel<<<grid, nthr, smem, c->stream>>>(k, src, s, net, i_begin, i_end, fvals, stats);
+    } else {
+        VS_CUDA(cudaFuncSetAttribute(network_values_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        time_begin(c);
+        network_values_kernel<<<grid, nthr, smem, c->stream>>>(k, src, s, net, i_begin, i_end, fvals);
+    }
     time_end(c);
     c->launches++;
     VS_CUDA(cudaGetLastError());
     if (!c->opt.trace.empty()) {                      // VS_TRACE: the form that ran (64 or 32 trajectories per CTA) and its grid
         if (FILE *fp = fopen(c->opt.trace.c_str(), "a")) {
-            fprintf(fp, "# network_values_kernel nthr=%d gx=%u gy=%u smem=%zu rows=%llu\n", nthr, grid.x, grid.y, smem,
-                    (unsigned long long)rows);
+            fprintf(fp, "# %s nthr=%d gx=%u gy=%u smem=%zu rows=%llu\n", adaptive ? "network_adaptive_kernel" : "network_values_kernel",
+                    nthr, grid.x, grid.y, smem, (unsigned long long)rows);
             fclose(fp);
         }
     }

@@ -315,7 +315,7 @@ static int launch_rk4(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s,
 }
 
 int launch_eval_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, const ObjectiveDev &o, uint64_t i_begin,
-                       uint64_t i_end, double *fvals) {
+                       uint64_t i_end, double *fvals, bool count) {
     switch (o.id) {
     case VS_OBJ_GFUNCTION: {
         GFunction f{o.params + k, o.params + 2 * k};
@@ -345,7 +345,8 @@ int launch_eval_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s
         }
     }
     case VS_OBJ_MASS_ACTION:
-        return launch_network_values(c, k, src, s, o, i_begin, i_end, fvals);
+    case VS_OBJ_MASS_ACTION_ADAPTIVE:
+        return launch_network_values(c, k, src, s, o, i_begin, i_end, fvals, count);
     }
     set_error("unknown objective id %d", o.id);
     return VS_ERR_ARG;

@@ -276,8 +276,9 @@ class Objective(object):
     """Objective values fM_1, fM_2 (n,l) and fN_j, fN_nj (k,n,l) (varsens/saltelli.py:252-495).
 
     ``objective_func`` may be
-      * a registered device functor (varsens_b200.GFunction / Ishigami / RK4Chain / MassActionNetwork): evaluated on the
-        GPU; Varsens then uses the fused kernel (or the two-phase path) and these arrays are only built if you read them;
+      * a registered device functor (varsens_b200.GFunction / Ishigami / RK4Chain / MassActionNetwork /
+        AdaptiveMassActionNetwork): evaluated on the GPU; Varsens then uses the fused kernel (or the two-phase path) and
+        these arrays are only built if you read them;
         a functor with l = outputs(k) > 1 outputs gives fM_1 (n, l), fN_j (k, n, l) and flat() (2n(1+k), l);
       * a callable marked with ``varsens_b200.vectorized``: gets CUDA tensors of sample rows;
       * any Python callable of one (k,) row, exactly as in the reference (called 2n(1+k) times).
@@ -362,6 +363,7 @@ class Objective(object):
         s = self.sample
         v = s.ctx.eval_values(self.k, self.n, s._perm_arg(), self._functor.objective_id, self._functor.params(self.k),
                               s.discard, s._scale, s._raw)
+        self._functor.check_run(s.ctx)
         self._vals = numpy.ascontiguousarray(v.reshape(-1, self._functor.outputs(self.k)))
 
     def _host_vals(self):
@@ -478,4 +480,6 @@ class Varsens(object):
 
     def _fused(self, o, k, n, flags):
         s, f = o.sample, o._functor
-        return dist.fused_step(s.ctx, k, n, s._perm_arg(), f.objective_id, f.params(k), s.discard, s._scale, s._raw, flags)
+        res = dist.fused_step(s.ctx, k, n, s._perm_arg(), f.objective_id, f.params(k), s.discard, s._scale, s._raw, flags)
+        f.check_run(s.ctx)
+        return res
