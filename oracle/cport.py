@@ -1,4 +1,5 @@
-"""ctypes front end of oracle/oracle.c (liboracle.so).  TEST INFRASTRUCTURE (oracle/__init__.py)."""
+"""ctypes front end of liboracle.so (oracle/oracle.c; oracle/mass_action.c's entry points are called from
+oracle/mass_action.py).  TEST INFRASTRUCTURE (oracle/__init__.py)."""
 import ctypes
 import os
 import subprocess
@@ -16,8 +17,8 @@ SCALE_IDENTITY, SCALE_LINEAR, SCALE_POWER = 0, 1, 2
 
 def build(force=False):
     so = os.path.join(_HERE, "liboracle.so")
-    src = os.path.join(_HERE, "oracle.c")
-    if force or not os.path.exists(so) or os.path.getmtime(so) < os.path.getmtime(src):
+    newest = max(os.path.getmtime(os.path.join(_HERE, src)) for src in ("oracle.c", "mass_action.c"))
+    if force or not os.path.exists(so) or os.path.getmtime(so) < newest:
         subprocess.check_call(["make", "-s", "-C", _HERE, "liboracle.so"])
     return so
 
@@ -33,6 +34,8 @@ def lib():
         L.orc_sample_flat.argtypes = [i32, u64, u64, vp, vp, i32, vp, vp, u64, u64, vp]
         L.orc_values.argtypes = [i32, u64, u64, vp, vp, i32, vp, vp, i32, vp, u64, u64, vp]
         L.orc_sums.argtypes = [i32, u64, u64, vp, vp, i32, vp, vp, i32, vp, u64, u64, i32, vp, vp]
+        L.ma_values.argtypes = [i32, u64, vp, vp, vp]
+        L.ma_values_adaptive.argtypes = [i32, u64, vp, vp, vp, vp]
         _LIB = L
     return _LIB
 

@@ -1,17 +1,16 @@
 """GPU checks of the adaptive mass-action network objective (VS_OBJ_MASS_ACTION_ADAPTIVE, network_adaptive_kernel): values
-and step counts bit for bit against the oracle's restatement (tests/adaptive_oracle.c) in the 64- and 32-thread forms, past
+and step counts bit for bit against the oracle's restatement (oracle/mass_action.c) in the 64- and 32-thread forms, past
 the first CTA; rejections and failures; indices through the two-phase route; the Python API; the limits.
 
 Every launch checked against its VS_TRACE line has at least 8 CTAs and a ragged last one (n = 8 nthr + 37)."""
 import numpy
 import pytest
 
-import adaptive_oracle as ad
 from conftest import close
 from oracle import exact as oexact, mass_action as ob
 from test_gpu_mass_action import bits_equal, perm_of
 from test_gpu_steady_state import Tracer
-from test_gpu_value_kernels import differ, guarded, launch_line, optin
+from test_gpu_value_kernels import differ, guarded, launch_line, net_smem, net_threads, optin
 from varsens_b200._cabi import OBJ_MASS_ACTION_ADAPTIVE
 
 pytestmark = pytest.mark.gpu
@@ -33,27 +32,9 @@ def ctx(vb):
     return vb.Context.get(0)
 
 
-def ad_smem(par, k, nthr):
-    """Shared memory of network_adaptive_kernel: network_values_kernel's tables (40 bytes a reaction, 4 per species pointer and
-    list entry, rounded up to 16), the output times and observable lists (8 bytes a time and weight, 4 per observable pointer
-    and species, rounded up to 16), then k + 8S + R doubles per trajectory."""
-    S, R, L, NT = (int(v) for v in par[:4])
-    nnz = 0
-    for r in range(R):
-        sp = [int(v) for v in par[8 + 8 * r:8 + 8 * r + 4]]
-        nnz += sum(1 for s in set(sp) if s >= 0 and sp[2:].count(s) != sp[:2].count(s))
-    nobs = int(numpy.count_nonzero(par[8 + 8 * R + 2 * S:8 + 8 * R + 2 * S + L * S]))
-    up = lambda b: -(-b // 16) * 16                                 # noqa: E731
-    return up(40 * R + 4 * (S + 1 + nnz)) + up(8 * (NT + nobs) + 4 * (L + 1 + nobs)) + (k + 8 * S + R) * nthr * 8
-
-
-def threads(par, k):
-    return 64 if ad_smem(par, k, 64) <= optin() else 32
-
-
 def assert_form(lines, par, k, rows, nthr):
     f = launch_line(lines, "network_adaptive_kernel", rows)
-    want = dict(nthr=nthr, gy=2 + 2 * k, smem=ad_smem(par, k, nthr))
+    want = dict(nthr=nthr, gy=2 + 2 * k, smem=net_smem(par, k, nthr, adaptive=True))
     assert {key: f[key] for key in want} == want, (f, want)
 
 
@@ -91,31 +72,31 @@ def test_values_and_counts_equal_the_oracle(ctx, vb, monkeypatch, tmp_path, S, R
     n = 8 * nthr + 37
     p = perm_of(n)
     rtol = 1e-7
-    par = ad.adaptive_of(ob.random_network(5000 + S, S, R, L, k), times_of(NT), rtol=rtol, atol=1e-10)
-    assert threads(par, k) == nthr
+    par = ob.adaptive_of(ob.random_network(5000 + S, S, R, L, k), times_of(NT), rtol=rtol, atol=1e-10)
+    assert net_threads(par, k, adaptive=True) == nthr
     l = L * NT
     for sc, osc in ((None, None), scales(k)[0]):
         kw = {} if sc is None else dict(scale=sc)
         shape = (2 + 2 * k, n, l)
         got, lines = trace(lambda: guarded(ctx, shape, lambda out: ctx.eval_values(k, n, p, MAA, par, discard=3, out=out, **kw)))
         assert_form(lines, par, k, n, nthr)
-        want, st = ad.values_adaptive(k, n, par, discard=3, scale=osc, perm=p)
+        want, st = ob.values_adaptive(k, n, par, discard=3, scale=osc, perm=p)
         assert numpy.isfinite(want).all() and bits_equal(got, want), differ(got, want)
         assert (stats_of(ctx) == st).all(), (stats_of(ctx), st)
         i0, i1 = 37, n - 5
         win, lines = trace(lambda: ctx.eval_values(k, n, p, MAA, par, discard=3, i_begin=i0, i_end=i1, **kw))
         assert_form(lines, par, k, i1 - i0, nthr)
-        want, st = ad.values_adaptive(k, n, par, discard=3, scale=osc, i0=i0, i1=i1, perm=p)
+        want, st = ob.values_adaptive(k, n, par, discard=3, scale=osc, i0=i0, i1=i1, perm=p)
         assert bits_equal(win.reshape(want.shape), want) and bits_equal(win.reshape(want.shape), got[:, i0:i1])
         assert (stats_of(ctx) == st).all(), (stats_of(ctx), st)
     lin, olin = scales(k)[0]
     raw = vb.sobol_raw(k, n)
     got = ctx.eval_values(k, n, p, MAA, par, raw=raw, scale=lin)
-    want, st = ad.values_adaptive(k, n, par, scale=olin, perm=p, raw=raw)
+    want, st = ob.values_adaptive(k, n, par, scale=olin, perm=p, raw=raw)
     assert bits_equal(got.reshape(want.shape), want) and (stats_of(ctx) == st).all()
     pw, opw = scales(k)[1]
     got = ctx.eval_values(k, n, p, MAA, par, scale=pw)
-    want, _ = ad.values_adaptive(k, n, par, scale=opw, perm=p)
+    want, _ = ob.values_adaptive(k, n, par, scale=opw, perm=p)
     numpy.testing.assert_allclose(got.reshape(want.shape), want, rtol=10 * rtol, atol=1e-9)
 
 
@@ -132,17 +113,19 @@ def test_fit_boundary_and_limits_launch_nothing(ctx, vb, monkeypatch, tmp_path):
     full = ob.random_network(4343, S, 512, L, k)
 
     def first(R):
-        fixed = numpy.concatenate([[S, R], full[2:5], full[5:5 + 8 * R], full[5 + 8 * 512:]])
-        return ad.adaptive_of(fixed, [0.5, 1.0], rtol=1e-6, atol=1e-10)
+        net = ob.unpack(full, adaptive=False)
+        net.rec = net.rec[:R]
+        return ob.adaptive_of(ob.pack(net), [0.5, 1.0], rtol=1e-6, atol=1e-10)
     limit = optin()
-    R = max(r for r in range(1, 512) if ad_smem(first(r), k, nthr) <= limit)
-    assert R >= 16 and ad_smem(first(R + 1), k, nthr) > limit and ad_smem(first(R), k, 64) > limit, R
+    R = max(r for r in range(1, 512) if net_smem(first(r), k, nthr, adaptive=True) <= limit)
+    assert R >= 16 and net_smem(first(R + 1), k, nthr, adaptive=True) > limit, R
+    assert net_smem(first(R), k, 64, adaptive=True) > limit, R
     par = first(R)
     lin, olin = scales(k)[0]
     got, lines = trace(lambda: guarded(ctx, (2 + 2 * k, n, L * NT), lambda out: ctx.eval_values(k, n, p, MAA, par, scale=lin,
                                                                                                  out=out)))
     assert_form(lines, par, k, n, nthr)
-    want, st = ad.values_adaptive(k, n, par, scale=olin, perm=p)
+    want, st = ob.values_adaptive(k, n, par, scale=olin, perm=p)
     assert numpy.isfinite(want).all() and bits_equal(got, want), differ(got, want)
     assert (stats_of(ctx) == st).all()
     before = ctx.launch_count()
@@ -152,11 +135,11 @@ def test_fit_boundary_and_limits_launch_nothing(ctx, vb, monkeypatch, tmp_path):
     with pytest.raises(vb.VarsensError) as e:
         ctx.run_fused(k, n, p, MAA, first(R + 1), scale=lin)
     assert e.value.status == ERR_UNSUPPORTED
-    small = ad.adaptive_of(ob.chain_network(2), [1.0])
+    small = ob.adaptive_of(ob.chain_network(2), [1.0])
     with pytest.raises(vb.VarsensError) as e:
         ctx.run_fused(4, 16, perm_of(16), MAA, small, flags=_cabi.FLAG_SECOND_ORDER | _cabi.FLAG_SEPARABLE)
     assert e.value.status == ERR_UNSUPPORTED
-    wide = ad.adaptive_of(ob.random_network(7, 4, 6, 5, 4), times_of(13))
+    wide = ob.adaptive_of(ob.random_network(7, 4, 6, 5, 4), times_of(13))
     with pytest.raises(vb.VarsensError) as e:
         ctx.eval_values(4, 16, perm_of(16), MAA, wide)
     assert e.value.status == ERR_ARG
@@ -171,17 +154,17 @@ def test_rejections_and_failures(ctx, vb):
     lin, olin = scales(k)[0]
     fixed = ob.random_network(606, 8, 12, 2, k)
     times = [0.5, 1.0, 2.0, 4.0]
-    par = ad.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12, h0=2.0)
+    par = ob.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12, h0=2.0)
     got = ctx.eval_values(k, n, p, MAA, par, scale=lin)
-    want, st = ad.values_adaptive(k, n, par, scale=olin, perm=p)
+    want, st = ob.values_adaptive(k, n, par, scale=olin, perm=p)
     assert bits_equal(got, want) and (stats_of(ctx) == st).all()
     assert st[1] >= (2 + 2 * k) * n and st[2] == 0
     util = float(st[0] + st[1]) / float(st[3])
     assert 0.0 < util <= 1.0
     cap = int(0.75 * float(st[0] + st[1]) / ((2 + 2 * k) * n))               # below the mean attempts per trajectory
-    capped = ad.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12, h0=2.0, max_steps=cap)
+    capped = ob.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12, h0=2.0, max_steps=cap)
     got2 = ctx.eval_values(k, n, p, MAA, capped, scale=lin)
-    want2, st2 = ad.values_adaptive(k, n, capped, scale=olin, perm=p)
+    want2, st2 = ob.values_adaptive(k, n, capped, scale=olin, perm=p)
     nan = numpy.isnan(want2)
     assert nan.any() and (~nan).any() and st2[2] > 0
     assert bits_equal(got2, want2) and (stats_of(ctx) == st2).all()
@@ -196,9 +179,9 @@ def test_indices_through_the_two_phase_route(ctx, vb, L, NT):
     k, n = 5, 600
     l = L * NT
     p = perm_of(n)
-    par = ad.adaptive_of(ob.random_network(88 + L, 6, 9, L, k), times_of(NT), rtol=1e-8, atol=1e-12)
+    par = ob.adaptive_of(ob.random_network(88 + L, 6, 9, L, k), times_of(NT), rtol=1e-8, atol=1e-12)
     sc = _cabi.Scale(_cabi.SCALE_LINEAR, numpy.full(k, 0.5), numpy.full(k, 2.0))
-    vals, st = ad.values_adaptive(k, n, par, scale=("linear", 0.5, 2.0), perm=p)
+    vals, st = ob.values_adaptive(k, n, par, scale=("linear", 0.5, 2.0), perm=p)
     ref = oexact.indices(vals.reshape(-1, l), k, n)
     for flags in (0, _cabi.FLAG_SECOND_ORDER):
         res = ctx.run_fused(k, n, p, MAA, par, scale=sc, flags=flags)
@@ -211,7 +194,7 @@ def test_indices_through_the_two_phase_route(ctx, vb, L, NT):
     parts = []
     for a, b in ((0, 97), (97, 350), (350, n)):
         parts.append(ctx.fused_partials(k, n, p, MAA, par, scale=sc, i_begin=a, i_end=b))
-        _, sw = ad.values_adaptive(k, n, par, scale=("linear", 0.5, 2.0), perm=p, i0=a, i1=b)
+        _, sw = ob.values_adaptive(k, n, par, scale=("linear", 0.5, 2.0), perm=p, i0=a, i1=b)
         assert (stats_of(ctx) == sw).all(), (a, b)              # the shard's rows only, not base row 0 of the common shift
     summed = ctx.finalize(k, l, n, parts[0] + parts[1] + parts[2])
     for name in NAMES:
@@ -233,7 +216,7 @@ def test_python_api(ctx, vb):
     scaling = lambda x: vb.linear(x, lo, hi)                                # noqa: E731
     v = vb.Varsens(net, scaling, k, n, verbose=False)
     assert v.E_2.shape == (2 * NT,) and v.sens.shape == (k, 2 * NT) and v.sens_2.shape == (k, 2 * NT, k, 2 * NT)
-    want, _ = ad.values_adaptive(k, n, net.params(k), scale=("linear", lo, hi))
+    want, _ = ob.values_adaptive(k, n, net.params(k), scale=("linear", lo, hi))
     o = v.objective
     assert o.fM_1.shape == (n, 2 * NT) and o.fN_j.shape == (k, n, 2 * NT) and o.flat().shape == (2 * n * (1 + k), 2 * NT)
     assert bits_equal(o.fM_1, want[0]) and bits_equal(o.fN_j, want[2:2 + k])

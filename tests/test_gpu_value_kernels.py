@@ -235,22 +235,17 @@ def test_ishigami_every_form(ctx, monkeypatch, tmp_path, k):
 # ------------------------------------------------------------------------------------------------
 # C. mass-action networks
 # ------------------------------------------------------------------------------------------------
-def net_nnz(par):
-    """Entries of the species-major stoichiometry list: per reaction, the species whose net coefficient is not 0."""
-    R = int(par[1])
-    nnz = 0
-    for r in range(R):
-        sp = [int(v) for v in par[5 + 8 * r:5 + 8 * r + 4]]
-        nnz += sum(1 for s in set(sp) if s >= 0 and sp[2:].count(s) != sp[:2].count(s))
-    return nnz
-
-
-def net_smem(par, k, nthr):
+def net_smem(par, k, nthr, adaptive=False):
     """Shared memory of network_values_kernel: the tables (40 bytes a reaction, 4 per species pointer and list entry, rounded
-    up to 16 bytes), then k + 3S + R doubles per trajectory."""
-    S, R = int(par[0]), int(par[1])
-    table = -(-(40 * R + 4 * (S + 1 + net_nnz(par))) // 16) * 16
-    return table + (k + 3 * S + R) * nthr * 8
+    up to 16 bytes), then k + 3S + R doubles per trajectory.  network_adaptive_kernel: network_values_kernel's tables, the
+    output times and observable lists (8 bytes a time and weight, 4 per observable pointer and species, rounded up to 16),
+    then k + 8S + R doubles per trajectory."""
+    net = ob.unpack(par, adaptive)
+    up = lambda b: -(-b // 16) * 16                                 # noqa: E731
+    table = up(40 * net.R + 4 * (net.S + 1 + net.nnz))
+    if adaptive:
+        return table + up(8 * (net.NT + net.nobs) + 4 * (net.L + 1 + net.nobs)) + (k + 8 * net.S + net.R) * nthr * 8
+    return table + (k + 3 * net.S + net.R) * nthr * 8
 
 
 def optin():
@@ -258,8 +253,8 @@ def optin():
     return torch.cuda.get_device_properties(0).shared_memory_per_block_optin
 
 
-def net_threads(par, k):
-    return 64 if net_smem(par, k, 64) <= optin() else 32
+def net_threads(par, k, adaptive=False):
+    return 64 if net_smem(par, k, 64, adaptive) <= optin() else 32
 
 
 def assert_net_form(lines, par, k, rows, nthr):
@@ -343,9 +338,10 @@ def test_network_windows_and_edges(ctx, vb, monkeypatch, tmp_path, S, R, L, k, n
                                                                   out=out))
         assert bits_equal(dev, win), (lo, hi, differ(dev, win))
     # nsteps = 0: the weighted sums of the initial amounts
-    par0 = par.copy()
-    par0[4] = 0
-    init = par0[5 + 8 * R:5 + 8 * R + 2 * S].reshape(S, 2)
+    net = ob.unpack(par, adaptive=False)
+    net.head["nsteps"] = 0
+    par0 = ob.pack(net)
+    init = net.init
     assert (init[:, 0] >= 0).any() and (init[:, 0] < 0).any()
     got, lines = trace(lambda: ctx.eval_values(k, n, p, MA, par0, discard=3, scale=lin))
     assert_net_form(lines, par0, k, n, nthr)
@@ -353,9 +349,8 @@ def test_network_windows_and_edges(ctx, vb, monkeypatch, tmp_path, S, R, L, k, n
     assert bits_equal(got, want), differ(got, want)
     x = cport.sample_flat(k, n, 3, olin, perm=p)
     X0 = numpy.where(init[:, 0] >= 0, x[:, numpy.maximum(init[:, 0], 0).astype(int)], init[:, 1])
-    w = par0[5 + 8 * R + 2 * S:].reshape(L, S)
-    err = numpy.abs(got.reshape(-1, L) - X0 @ w.T)
-    assert (err <= 4 * S * EPS * (numpy.abs(X0) @ numpy.abs(w).T)).all()
+    err = numpy.abs(got.reshape(-1, L) - X0 @ net.w.T)
+    assert (err <= 4 * S * EPS * (numpy.abs(X0) @ numpy.abs(net.w).T)).all()
     # dt < 0 (short: backwards, second-order reactions blow up in finite time)
     parn = ob.random_network(3000 + S, S, R, L, k, dt=-0.002, nsteps=10)
     got, lines = trace(lambda: ctx.eval_values(k, n, p, MA, parn, scale=lin))
@@ -376,7 +371,9 @@ def test_network_fit_boundary(ctx, vb, monkeypatch, tmp_path):
 
     def first(R):
         """The network of the first R reactions of `full` (same initial amounts and observables)."""
-        return numpy.concatenate([[S, R], full[2:5], full[5:5 + 8 * R], full[5 + 8 * 512:]])
+        net = ob.unpack(full, adaptive=False)
+        net.rec = net.rec[:R]
+        return ob.pack(net)
     limit = optin()
     R = max(r for r in range(1, 512) if net_smem(first(r), k, nthr) <= limit)
     assert R < 511 and net_smem(first(R + 1), k, nthr) > limit and net_smem(first(R), k, 64) > limit, R

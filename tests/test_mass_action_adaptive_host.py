@@ -7,7 +7,6 @@ import math
 import numpy
 import pytest
 
-import adaptive_oracle as ad
 from oracle import mass_action as ob
 
 
@@ -41,7 +40,7 @@ def test_outputs_are_l_times_nt(cabi):
     assert outputs(cabi, 1, ab_network(64, times=(1.0,))) == (0, 64)
     assert outputs(cabi, 1, ab_network(5, times=range(1, 14)))[0] == 1              # 65
     assert outputs(cabi, 1, ab_network(1, times=range(1, 66)))[0] == 1              # 65
-    assert outputs(cabi, 16, ad.adaptive_of(ob.random_network(3, 128, 192, 8, 16), [1.0, 2.0])) == (0, 16)
+    assert outputs(cabi, 16, ob.adaptive_of(ob.random_network(3, 128, 192, 8, 16), [1.0, 2.0])) == (0, 16)
     # the fixed-step objective keeps its own header
     assert outputs(cabi, 1, ob.chain_network(1))[0] == 1
     st = ctypes.c_int()
@@ -121,7 +120,7 @@ def test_adaptive_object_builds_the_documented_layout(cabi):
     d = vb.AdaptiveMassActionNetwork(2, [([0], [1], 1.0)], [1.0, 0.0], [1], times=[4.0])
     assert d.params(1).tolist() == [2, 1, 1, 1, 1e-6, 1e-9, 4e-6, 100000, 0, -1, 1, -1, -1, 1.0, -1, 0.0, -1, 1.0, -1, 0.0,
                                     0.0, 1.0, 4.0]
-    assert numpy.array_equal(d.params(1), ad.adaptive_of(vb.MassActionNetwork(2, [([0], [1], 1.0)], [1.0, 0.0], [1]).params(1),
+    assert numpy.array_equal(d.params(1), ob.adaptive_of(vb.MassActionNetwork(2, [([0], [1], 1.0)], [1.0, 0.0], [1]).params(1),
                                                            [4.0]))
 
 
@@ -159,7 +158,7 @@ TIMES = (0.1, 0.5, 1.0, 2.0, 3.5, 5.0)
 
 
 def test_oracle_decay_matches_closed_form():
-    v, info = ad.points_values([[0.0]], ab_network(2, TIMES))
+    v, info = ob.points_values([[0.0]], ab_network(2, TIMES))
     t = numpy.repeat(TIMES, 2)
     assert numpy.abs(v[0] - (1.0 - numpy.exp(-t))).max() < 1e-7
     assert info[0, 2] == 0 and info[0, 1] >= len(TIMES)
@@ -167,17 +166,16 @@ def test_oracle_decay_matches_closed_form():
 
 def test_oracle_reversible_pair_matches_closed_form():
     kf, kr = 1.0, 0.4
-    v, info = ad.points_values([[0.0]], ab_network(1, TIMES, kr=kr))
+    v, info = ob.points_values([[0.0]], ab_network(1, TIMES, kr=kr))
     exact = kf / (kf + kr) * (1.0 - numpy.exp(-(kf + kr) * numpy.array(TIMES)))
     assert numpy.abs(v[0] - exact).max() < 1e-7 and info[0, 2] == 0
 
 
 def _stiffish(seed, S, R, k):
     """A seeded network with one fast reversible pair X_0 <-> X_1 (rates 300 and 200) added to it."""
-    par = ob.random_network(seed, S, R, 2, k)
-    rec = par[5:5 + 8 * R]
-    fast = [0, -1, 1, -1, -1, 300.0, -1, 200.0]
-    return numpy.concatenate([[S, R + 1, 2, 0.01, 1], rec, fast, par[5 + 8 * R:]])
+    net = ob.unpack(ob.random_network(seed, S, R, 2, k), adaptive=False)
+    net.rec = numpy.vstack([net.rec, [0, -1, 1, -1, -1, 300.0, -1, 200.0]])
+    return ob.pack(net)
 
 
 NETS = [("random", 11, 4, 6, 3), ("random", 12, 9, 14, 5), ("random", 13, 12, 18, 6), ("stiffish", 14, 8, 10, 4)]
@@ -192,10 +190,10 @@ def test_oracle_agrees_with_solve_ivp(kind, seed, S, R, k):
     fixed = ob.random_network(seed, S, R, 2, k) if kind == "random" else _stiffish(seed, S, R, k)
     times = [0.25, 1.0, 2.0]
     pts = _points(k, 3, seed)
-    ref = numpy.array([ad.solve_ivp_values(ad.adaptive_of(fixed, times), x) for x in pts])
+    ref = numpy.array([ob.solve_ivp_values(ob.adaptive_of(fixed, times), x) for x in pts])
     errs = []
     for rtol in (1e-4, 1e-6, 1e-8):
-        v, info = ad.points_values(pts, ad.adaptive_of(fixed, times, rtol=rtol, atol=1e-12))
+        v, info = ob.points_values(pts, ob.adaptive_of(fixed, times, rtol=rtol, atol=1e-12))
         assert (info[:, 2] == 0).all()
         d = numpy.abs(v - ref)
         errs.append(d.max())
@@ -208,10 +206,10 @@ def test_small_max_steps_gives_nan_from_the_failing_time():
     times = (0.5, 1.0, 2.0, 4.0)
     pts = _points(3, 64, 5)
     fixed = ob.random_network(21, 5, 8, 2, 3)
-    full, info = ad.points_values(pts, ad.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12))
+    full, info = ob.points_values(pts, ob.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12))
     assert (info[:, 2] == 0).all()
     cap = int(numpy.median(info[:, 0]))
-    v, capped = ad.points_values(pts, ad.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12, max_steps=cap))
+    v, capped = ob.points_values(pts, ob.adaptive_of(fixed, times, rtol=1e-9, atol=1e-12, max_steps=cap))
     failed = capped[:, 2] == 1
     assert failed.any() and (~failed).any()
     assert (capped[:, 0] <= cap).all() and (capped[failed, 0] == cap).all()
@@ -224,6 +222,6 @@ def test_small_max_steps_gives_nan_from_the_failing_time():
         assert first % 2 == 0 and nan[first:].all() and not nan[:first].any()
         assert (v[p, :first].view(numpy.int64) == full[p, :first].view(numpy.int64)).all()
     k, n = 3, 8
-    vals, stats = ad.values_adaptive(k, n, ad.adaptive_of(fixed, times, max_steps=3), scale=("linear", 0.5, 2.0))
+    vals, stats = ob.values_adaptive(k, n, ob.adaptive_of(fixed, times, max_steps=3), scale=("linear", 0.5, 2.0))
     assert vals.shape == (2 + 2 * k, n, 2 * len(times))
     assert int(stats[2]) == int(numpy.isnan(vals[..., -1]).sum()) == (2 + 2 * k) * n

@@ -99,18 +99,10 @@ out["mid_network"] = {"S": S, "R": R, "L": L, "k": k, "n": n, "steps": steps, "t
                       "varsens_end_to_end_s": min(ts), "sens_shape": list(v.sens.shape)}
 
 # ---- 3. the same network through the @vectorized torch route, reduced n
-par = mid
-rec = par[5:5 + 8 * R].reshape(R, 8)
-init = par[5 + 8 * R:5 + 8 * R + 2 * S].reshape(S, 2)
-W = torch.tensor(par[5 + 8 * R + 2 * S:].reshape(L, S), dtype=torch.float64, device=dev)
-Nmat = torch.zeros((S, R), dtype=torch.float64, device=dev)
-for r, q in enumerate(rec):
-    for s in q[0:2]:
-        if s >= 0:
-            Nmat[int(s), r] -= 1.0
-    for s in q[2:4]:
-        if s >= 0:
-            Nmat[int(s), r] += 1.0
+net = ob.unpack(mid, adaptive=False)
+rec, init = net.rec, net.init
+W = torch.tensor(net.w, dtype=torch.float64, device=dev)
+Nmat = torch.tensor(net.N, dtype=torch.float64, device=dev)
 ix = {name: torch.tensor([int(q[c]) if q[c] >= 0 else S for q in rec], device=dev) for name, c in (("a0", 0), ("a1", 1), ("b0", 2), ("b1", 3))}
 kfc = torch.tensor([int(q[4]) if q[4] >= 0 else k for q in rec], device=dev)
 krc = torch.tensor([int(q[6]) if q[6] >= 0 else k for q in rec], device=dev)

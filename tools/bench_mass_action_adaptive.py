@@ -11,14 +11,11 @@ csrc/kernels_network.cu: network_adaptive_kernel) beside the fixed-step one.  Pr
                 steps): both kernel times and their agreement; and the chain as a fixed-step network (the r03 record).
 Needs a CUDA device (the library has no CPU fallback).  Run:  python tools/bench_mass_action_adaptive.py > adaptive.json"""
 import json, os, subprocess, sys
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy, torch
 import varsens_b200 as vb
 from varsens_b200 import _cabi
 from oracle import mass_action as ob
-import adaptive_oracle as ad
 
 if not torch.cuda.is_available():
     raise SystemExit("bench_mass_action_adaptive: no CUDA device")
@@ -88,25 +85,26 @@ mid = ob.random_network(2024, S, R, L, k, dt=0.01, nsteps=1000)
 p = perm_dev(n)
 scl = _cabi.Scale(_cabi.SCALE_LINEAR, numpy.full(k, 0.5), numpy.full(k, 2.0))
 idx, pts = sampled(k, n, p, scl)
-ref = ad.points_values(pts, ad.adaptive_of(mid, times, rtol=1e-12, atol=1e-15))[0][:, -L:]
+ref = ob.points_values(pts, ob.adaptive_of(mid, times, rtol=1e-12, atol=1e-15))[0][:, -L:]
 out["mid_network"] = {"S": S, "R": R, "L": L, "k": k, "n": n, "times": times, "trajectories": 2 * n * (1 + k),
                       "reference": "oracle restatement at rtol 1e-12, atol 1e-15", "sampled_points": len(idx),
-                      "adaptive": [adaptive_run(k, n, p, scl, ad.adaptive_of(mid, times, rtol=rt, atol=rt * 1e-3), idx, ref, L)
+                      "adaptive": [adaptive_run(k, n, p, scl, ob.adaptive_of(mid, times, rtol=rt, atol=rt * 1e-3), idx, ref, L)
                                    for rt in (1e-6, 1e-9)],
                       "fixed_step": fixed_run(k, n, p, scl, mid, idx, ref)}
 
 # ---- 2. a fast reversible pair the fixed step cannot integrate at dt = 0.01
 k, n, S, R, L = 8, 1 << 12, 8, 12, 2
-base = ob.random_network(7, S, R, L, k, dt=0.01, nsteps=1000)
+net = ob.unpack(ob.random_network(7, S, R, L, k, dt=0.01, nsteps=1000), adaptive=False)
 pair = [0, -1, 1, -1, -1, 1000.0, -1, 800.0]                       # X_0 <-> X_1, kf + kr = 1800: 18 x dt, RK4's bound is 2.8
-fast = numpy.concatenate([[S, R + 1], base[2:5], base[5:5 + 8 * R], pair, base[5 + 8 * R:]])
+net.rec = numpy.vstack([net.rec, pair])
+fast = ob.pack(net)
 p = perm_dev(n)
 scl = _cabi.Scale(_cabi.SCALE_LINEAR, numpy.full(k, 0.5), numpy.full(k, 2.0))
 idx, pts = sampled(k, n, p, scl)
-ref = ad.points_values(pts, ad.adaptive_of(fast, [10.0], rtol=1e-12, atol=1e-15))[0]
+ref = ob.points_values(pts, ob.adaptive_of(fast, [10.0], rtol=1e-12, atol=1e-15))[0]
 out["fast_pair"] = {"S": S, "R": R + 1, "L": L, "k": k, "n": n, "times": [10.0], "pair_rates": [1000.0, 800.0],
                     "reference_max_abs": float(numpy.abs(ref).max()),
-                    "adaptive": adaptive_run(k, n, p, scl, ad.adaptive_of(fast, [10.0], rtol=1e-6, atol=1e-9), idx, ref, L),
+                    "adaptive": adaptive_run(k, n, p, scl, ob.adaptive_of(fast, [10.0], rtol=1e-6, atol=1e-9), idx, ref, L),
                     "fixed_step": fixed_run(k, n, p, scl, fast, idx, ref)}
 
 # ---- 3. the C5 chain as an adaptive network against RK4Chain<10>, and as a fixed-step network
@@ -123,7 +121,7 @@ same = bool(torch.equal(va.view(torch.int64), vn.view(torch.int64)))
 c5 = {"k": k, "n": n, "trajectories": traj, "rk4_chain_kernel_ms": ms_chain, "fixed_network_kernel_ms": ms_fixed,
       "fixed_network_bit_identical_to_chain": same, "adaptive": []}
 for rt in (1e-6, 1e-9):
-    par = ad.adaptive_of(ob.chain_network(10), [10.0], rtol=rt, atol=rt * 1e-3)
+    par = ob.adaptive_of(ob.chain_network(10), [10.0], rtol=rt, atol=rt * 1e-3)
     ms = kernel_ms(lambda: ctx.eval_values(k, n, p, MAA, par, scale=sc, out=vn))
     st = ctx.network_stats()
     c5["adaptive"].append({"rtol": rt, "atol": rt * 1e-3, "kernel_ms": ms, "ratio_over_rk4_chain": ms / ms_chain, "stats": st,

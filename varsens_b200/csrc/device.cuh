@@ -457,7 +457,7 @@ struct RK4ChainDyn {
 };
 
 // MassAction (VS_OBJ_MASS_ACTION, a run-time network; kernel in kernels_network.cu).  FROZEN ARITHMETIC, restated by the
-// oracle (oracle/mass_action.c: f_mass_action) so trajectories are bit-identical given bit-identical rates and initial amounts:
+// oracle (oracle/mass_action.c: ma_rhs, f_mass_action) so trajectories are bit-identical given bit-identical rates and initial amounts:
 //   P      = 1.0 (no species on the side), X[s0] (one), __dmul_rn(X[s0], X[s1]) (two)      Pf over reactants, Pr over products
 //   flux_r = fma(kf, Pf, -__dmul_rn(kr, Pr))   reversible;   __dmul_rn(kf, Pf)   irreversible (reverse term not evaluated)
 //   d_s    = 0.0, then over the reactions with net coefficient c != 0 for s (products - reactants; a catalyst nets to 0),
@@ -469,8 +469,9 @@ struct RK4ChainDyn {
 // same bits as RK4Chain<S> and RK4ChainDyn.
 
 // MassActionAdaptive (VS_OBJ_MASS_ACTION_ADAPTIVE; kernel network_adaptive_kernel in kernels_network.cu).  FROZEN ARITHMETIC,
-// restated bit for bit by the oracle (tests/adaptive_oracle.c).  Only correctly rounded operations (+ - * /, fma, sqrt, fabs,
-// fmax, fmin): CUDA and glibc round pow, exp and log differently, so the step-size controller uses none of them.
+// restated bit for bit by the oracle (oracle/mass_action.c: f_mass_action_adaptive).  Only correctly rounded operations
+// (+ - * /, fma, sqrt, fabs, fmax, fmin): CUDA and glibc round pow, exp and log differently, so the step-size controller uses
+// none of them.
 //   right-hand side   MassAction's P, flux_r and d_s above.
 //   tableau           Dormand-Prince 5(4), Hairer-Norsett-Wanner I, Table 5.2: a_ij, and e_j = b_j - bhat_j, each the
 //                     correctly rounded double of its rational (dp5:: in kernels_network.cu).
