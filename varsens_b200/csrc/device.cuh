@@ -215,9 +215,8 @@ __device__ __forceinline__ void halton_quad_arith(const uint32_t (&ia)[NR], cons
     }
 }
 
-// Shared-memory constants of the run-time-base generators (export mode, product-form evaluation), filled once per CTA.
-constexpr int HL_D0 = 11;      // dimensions >= HL_D0 (bases >= 37): computed terms; below: table rows in shared memory
-constexpr int HL_J = 7;        // digit positions of a 32-bit index in base >= 37 (layout of HaltonDev::arh / arl)
+// Shared-memory constants of the run-time-base generators (export mode, product-form evaluation), filled once per CTA
+// (halton_prefix).  HL_D0, HL_J: vs_internal.cuh.
 struct HaltonShared {
     const uint32_t *base, *off;
     const uint64_t *magic;
@@ -316,12 +315,65 @@ __device__ __forceinline__ void halton_units(int w, const unsigned char *__restr
     }
 }
 
+// The generator prefix of a run-time-base kernel's shared memory:
+//   base[k] off[k] (u32) | magic[k] (u64) | lb[k] wr[k] | dl[k] | arh arl [k][HL_J] | ulist[16][HL_MAXQ] (u8) | table[table_len]
+// halton_prefix_doubles: the doubles before the table (20 k + 64, even: a 16-byte aligned prefix with an even table_len ends
+// 16-byte aligned).
+__host__ __device__ constexpr size_t halton_prefix_doubles(int k) {
+    return (2 * (size_t)k + 1) / 2 + (size_t)k + 2 * (size_t)k + 2 * (size_t)k + 2 * (size_t)k * HL_J + HL_LIST_BYTES / 8;
+}
+struct HaltonPrefix {
+    HaltonShared hs;
+    const unsigned char *ulist;
+    const double *lb, *wr;     // scaling constants (0.0 / 1.0 under identity scaling)
+    double *table;             // the table prefix
+};
+// Carves the prefix out of p and fills it; every thread of the CTA calls it, it ends with __syncthreads.  Unless the points are
+// given (src.raw): base, off, magic and the first table_len doubles of the term table; `computed`: also dl, arh and arl (the
+// multiply-only digit loop and the computed terms); sched_warps > 0: the units of that many warps (halton_schedule).
+__device__ __forceinline__ HaltonPrefix halton_prefix(double *p, int k, const SourceDev &src, const ScaleDev &s, uint32_t table_len,
+                                                      bool computed, int sched_warps) {
+    uint32_t *base = reinterpret_cast<uint32_t *>(p), *off = base + k;
+    uint64_t *magic = reinterpret_cast<uint64_t *>(p + (2 * k + 1) / 2);
+    double *lb = reinterpret_cast<double *>(magic + k), *wr = lb + k;
+    DimLoop *dl = reinterpret_cast<DimLoop *>(wr + k);                 // 16 bytes per dimension
+    double *arh = reinterpret_cast<double *>(dl + k), *arl = arh + (size_t)k * HL_J;
+    unsigned char *ulist = reinterpret_cast<unsigned char *>(arl + (size_t)k * HL_J);
+    double *table = arl + (size_t)k * HL_J + HL_LIST_BYTES / 8;
+    const int tid = threadIdx.x, nthr = blockDim.x;
+    if (!src.raw) {
+        for (int d = tid; d < k; d += nthr) {
+            base[d] = src.h.base[d];
+            off[d] = src.h.off[d];
+            magic[d] = src.h.magic[d];
+            if (computed) dl[d] = dim_loop(src.h.base[d], src.start + 2 * src.n - 1);      // the largest index of the design
+        }
+        if (computed)
+            for (int e = tid; e < k * HL_J; e += nthr) { arh[e] = src.h.arh[e]; arl[e] = src.h.arl[e]; }
+        for (uint32_t e = tid; e < table_len; e += nthr) table[e] = src.h.terms[e];
+    }
+    for (int d = tid; d < k; d += nthr) {
+        lb[d] = s.kind != VS_SCALE_IDENTITY ? s.lb[d] : 0.0;
+        wr[d] = s.kind != VS_SCALE_IDENTITY ? s.wr[d] : 1.0;
+    }
+    __syncthreads();
+    if (sched_warps > 0 && tid == 0) halton_schedule(k, sched_warps, dl, ulist);
+    __syncthreads();
+    return {{base, off, magic, dl, arh, arl, smem_u32(table)}, ulist, lb, wr, table};
+}
+
 // ---------------------------------------------------------------------------------------------
-// scale.py:33 (two roundings: multiply, then add -- never an FMA) and :62.
+// scale.py:33 (two roundings: multiply, then add -- never an FMA) and :62.  The one device statement of both.
 // ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ double scale_value(int kind, double lb, double wr, double p) {
+    if (kind == VS_SCALE_LINEAR) return __dadd_rn(__dmul_rn(p, wr), lb);
+    if (kind == VS_SCALE_POWER) return __dmul_rn(lb, pow(wr, p));
+    return p;
+}
+// s.lb and s.wr are null under identity scaling: read in the branch of their kind only
 __device__ __forceinline__ double apply_scale(const ScaleDev &s, int d, double p) {
-    if (s.kind == VS_SCALE_LINEAR) return __dadd_rn(__dmul_rn(p, s.wr[d]), s.lb[d]);
-    if (s.kind == VS_SCALE_POWER) return __dmul_rn(s.lb[d], pow(s.wr[d], p));
+    if (s.kind == VS_SCALE_LINEAR) return scale_value(VS_SCALE_LINEAR, s.lb[d], s.wr[d], p);
+    if (s.kind == VS_SCALE_POWER) return scale_value(VS_SCALE_POWER, s.lb[d], s.wr[d], p);
     return p;
 }
 

@@ -43,16 +43,12 @@ __host__ __device__ constexpr int gram_tile_for(int M) {
 #define VS_ARITH_D0 11         // prime_at(11) = 37: rows of >= 37 doubles span > 32 banks, random lookups cost 3-5 wavefronts
 #endif
 constexpr int AR_D0 = VS_ARITH_D0;
-constexpr int AR_J = 7;        // digit positions of a 32-bit index in base >= 37
 
 template <int K>
 struct FusedConst {            // kernel parameter -> constant bank; indexed with compile-time subscripts
     static constexpr int AR_N = K > AR_D0 ? K - AR_D0 : 1;
-    double arh[AR_N][AR_J], arl[AR_N][AR_J];   // term of digit at position j of dimension AR_D0 + u = fma(dd, arh, dd * arl), dd = 8 * digit
+    double arh[AR_N][HL_J], arl[AR_N][HL_J];   // term of digit at position j of dimension AR_D0 + u = fma(dd, arh, dd * arl), dd = 8 * digit
     double lb[K], wr[K];
-    uint32_t toff[K];          // offset of dimension d's terms inside the shared copy of the table
-    uint32_t nd[K];            // digits to sum for the largest index of the run
-    uint32_t ndc[K];           // digit rows the cached global table holds per dimension (layout: toff)
     int small_index;           // every Halton index of the run is < 2^29
     int poll_perm;             // see FusedTail::poll_perm
     long long *trace;          // profiling only (VS_TRACE): per-warp clock stamps of CTA 0, else nullptr
@@ -166,9 +162,8 @@ struct IshigamiReg {
 // Returns whether this lane's row exists (the last batch may be ragged).
 template <int K, int SCALE>
 __device__ __forceinline__ double scale_coord(const FusedConst<K> &fc, int d, double p) {
-    if constexpr (SCALE == VS_SCALE_LINEAR) return __dadd_rn(__dmul_rn(p, fc.wr[d]), fc.lb[d]);     // scale.py:33, two roundings
-    else if constexpr (SCALE == VS_SCALE_POWER) return __dmul_rn(fc.lb[d], pow(fc.wr[d], p));       // scale.py:62
-    else return p;
+    if constexpr (SCALE == VS_SCALE_IDENTITY) return p;
+    else return scale_value(SCALE, fc.lb[d], fc.wr[d], p);
 }
 
 // ---- Halton digit sums --------------------------------------------------------------------------------------
@@ -323,7 +318,7 @@ __device__ __forceinline__ void halton_group(const FusedConst<K> &fc, uint64_t b
                     if constexpr (J < nd_ib<IB>(B)) {
                         constexpr uint32_t RO = (uint32_t)(foff(D0 + U) + J * B) * 8u;   // byte offset of the row inside the table
                         constexpr bool AR = (D0 + U) >= AR_D0;               // B-point term computed, not looked up
-                        constexpr int AU = AR ? (D0 + U - AR_D0) : 0, AJ = J < AR_J ? J : AR_J - 1;
+                        constexpr int AU = AR ? (D0 + U - AR_D0) : 0, AJ = J < HL_J ? J : HL_J - 1;
                         constexpr bool F1 = J == 0;
                         if constexpr (J == 0 && !(IB <= 29 && 8ull * B * ((1ull << (IB < 32 ? IB : 31))) <= 0x100000000ull)) {
                             digit_step<B, false, F1, RO>(ma[U], xa[U], basehi);
@@ -984,8 +979,8 @@ fused_wsd_kernel(SourceDev src, FusedConst<K> fc, F f, uint64_t i_begin, uint64_
     if (threadIdx.x < K) {                                // lane = coordinate: the table reads of the K chains overlap
         const int d = threadIdx.x;
         double p = src.raw ? src.raw[d] : halton_coord_fixed<K>(terms, d, (uint32_t)src.start);
-        if (fc.scale_kind == VS_SCALE_LINEAR) p = __dadd_rn(__dmul_rn(p, fc.wr[d]), fc.lb[d]);
-        else if (fc.scale_kind == VS_SCALE_POWER) p = __dmul_rn(fc.lb[d], pow(fc.wr[d], p));
+        if (fc.scale_kind == VS_SCALE_LINEAR) p = scale_value(VS_SCALE_LINEAR, fc.lb[d], fc.wr[d], p);
+        else if (fc.scale_kind == VS_SCALE_POWER) p = scale_value(VS_SCALE_POWER, fc.lb[d], fc.wr[d], p);
         xs_sh[d] = p;
     }
     __syncthreads();
@@ -1167,8 +1162,8 @@ __global__ void shift_kernel(SourceDev src, FusedConst<K> fc, F f, double *out) 
     const int d = threadIdx.x;                     // one thread per coordinate: the table reads of the K chains overlap
     if (d < K) {
         double p = src.raw ? src.raw[d] : halton_coord(src.h, d, (uint32_t)src.start);
-        if (fc.scale_kind == VS_SCALE_LINEAR) p = __dadd_rn(__dmul_rn(p, fc.wr[d]), fc.lb[d]);
-        else if (fc.scale_kind == VS_SCALE_POWER) p = __dmul_rn(fc.lb[d], pow(fc.wr[d], p));
+        if (fc.scale_kind == VS_SCALE_LINEAR) p = scale_value(VS_SCALE_LINEAR, fc.lb[d], fc.wr[d], p);
+        else if (fc.scale_kind == VS_SCALE_POWER) p = scale_value(VS_SCALE_POWER, fc.lb[d], fc.wr[d], p);
         xs[d] = p;
     }
     __syncthreads();
@@ -1335,42 +1330,28 @@ static int fill_const(vs_ctx *c, const SourceDev &src, const ScaleDev &s, FusedC
     for (int d = 0; d < K; ++d) {
         fc.lb[d] = s.kind != VS_SCALE_IDENTITY ? h[d] : 0.0;
         fc.wr[d] = s.kind != VS_SCALE_IDENTITY ? h[K + d] : 1.0;
-        fc.toff[d] = 0;
-        fc.nd[d] = 0;
-        fc.ndc[d] = 0;
     }
     fc.small_index = 0;
     fc.poll_perm = 0;
     fc.trace = nullptr;
     for (int u = 0; u < FusedConst<K>::AR_N; ++u)
-        for (int j = 0; j < AR_J; ++j) { fc.arh[u][j] = 0.0; fc.arl[u][j] = 0.0; }
+        for (int j = 0; j < HL_J; ++j) { fc.arh[u][j] = 0.0; fc.arl[u][j] = 0.0; }
     if (!c->opt.trace.empty()) {
         VS_TRY(ensure(c, c->dir_buf, 16 * 64 * 4 * sizeof(long long)));
         VS_CUDA(cudaMemsetAsync(c->dir_buf.p, 0, 16 * 64 * 4 * sizeof(long long), c->stream));
         fc.trace = (long long *)c->dir_buf.p;
     }
     if (!src.raw) {
-        uint32_t off = 0;
-        for (int d = 0; d < K; ++d) {
-            fc.toff[d] = off;
-            uint32_t need = 0;                                   // digits of this run's largest index
-            for (uint64_t m = src.start + 2 * src.n - 1; m > 0; m /= prime_at(d)) ++need;
-            fc.nd[d] = need;
-            fc.ndc[d] = c->halton.ndigits[d];
-            off += c->halton.ndigits[d] * prime_at(d);         // layout of the (possibly longer) cached table
-        }
-        // the cached table may have more digits than this run needs: its layout is what matters
         fc.small_index = (src.start + 2 * src.n - 1) < (1ull << 29) ? 1 : 0;
         if (K > AR_D0) {
             VS_REQUIRE(c->halton.arith_ok, VS_ERR_UNSUPPORTED, "computed Halton terms do not reproduce the term table in mode %d",
                        c->halton.mode);
             for (int u = 0; u < K - AR_D0; ++u)
-                for (int j = 0; j < AR_J; ++j) {
-                    fc.arh[u][j] = c->halton.arh[(size_t)(AR_D0 + u) * AR_J + j];
-                    fc.arl[u][j] = c->halton.arl[(size_t)(AR_D0 + u) * AR_J + j];
+                for (int j = 0; j < HL_J; ++j) {
+                    fc.arh[u][j] = c->halton.arh[(size_t)(AR_D0 + u) * HL_J + j];
+                    fc.arl[u][j] = c->halton.arl[(size_t)(AR_D0 + u) * HL_J + j];
                 }
         }
-        VS_REQUIRE(off == src.h.total_terms, VS_ERR_ARG, "Halton table layout mismatch (%u vs %u)", off, src.h.total_terms);
         VS_REQUIRE(src.h.fixed && src.h.fixed_len >= foff(K), VS_ERR_ARG, "fixed-layout Halton table missing (%u of %u doubles)",
                    src.h.fixed_len, (uint32_t)foff(K));
     }

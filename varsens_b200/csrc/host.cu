@@ -164,33 +164,32 @@ static void build_terms(const std::vector<uint32_t> &bases, const std::vector<ui
 }
 
 // Constants of the computed-term form (fused_impl.cuh: digit_step_arith) for every (dimension, digit position) a 32-bit
-// index can reach, [k][7]: term(digit) = fma(dd, rh, dd * rl) with dd = 8 * digit.  Returns whether they reproduce the
+// index can reach, [k][HL_J]: term(digit) = fma(dd, rh, dd * rl) with dd = 8 * digit.  Returns whether they reproduce the
 // term-table arithmetic of `mode` bit for bit, for every digit of every position (exhaustive).
 static bool build_arith(const std::vector<uint32_t> &bases, int mode, std::vector<double> &arh, std::vector<double> &arl) {
-    const int AJ = 7;
-    arh.assign(bases.size() * AJ, 0.0);
-    arl.assign(bases.size() * AJ, 0.0);
+    arh.assign(bases.size() * HL_J, 0.0);
+    arl.assign(bases.size() * HL_J, 0.0);
     bool ok = true;
     for (size_t d = 0; d < bases.size(); ++d) {
         volatile double bp = (double)bases[d];
         volatile double ib = 1.0 / (double)bases[d];
         volatile double f = ib;
-        for (int j = 0; j < AJ; ++j) {
+        for (int j = 0; j < HL_J; ++j) {
             if ((double)bp > 4294967296.0 * (double)bases[d]) break;     // position not reachable by a 32-bit index
             double rh, rl;
             if (mode == VS_HALTON_RECIPROCAL) { rh = 1.0 / bp; rl = 0.0; }
             else if (mode == VS_HALTON_RUNNING_RECIPROCAL) { rh = f; rl = 0.0; }
             else { rh = 1.0 / bp; rl = std::fma(-rh, (double)bp, 1.0) / bp; }
-            arh[d * AJ + j] = rh * 0.125;
-            arl[d * AJ + j] = rl * 0.125;
+            arh[d * HL_J + j] = rh * 0.125;
+            arl[d * HL_J + j] = rl * 0.125;
             for (uint32_t digit = 0; digit < bases[d]; ++digit) {
                 volatile double want;
                 if (mode == VS_HALTON_RECIPROCAL) want = (double)digit * (1.0 / bp);
                 else if (mode == VS_HALTON_RUNNING_RECIPROCAL) want = (double)digit * f;
                 else want = (double)digit / bp;
                 const double dd = 8.0 * (double)digit;
-                volatile double t = dd * arl[d * AJ + j];
-                const double got = std::fma(dd, arh[d * AJ + j], (double)t);
+                volatile double t = dd * arl[d * HL_J + j];
+                const double got = std::fma(dd, arh[d * HL_J + j], (double)t);
                 if (got != (double)want) ok = false;
             }
             bp = bp * (double)bases[d];
@@ -268,6 +267,7 @@ int get_halton(vs_ctx *c, int k, uint64_t max_index, HaltonDev *out) {
         hc.k = k;
         hc.mode = mode;
         hc.ndigits = nd;
+        hc.off = off;
         hc.arh = arh_h;
         hc.arl = arl_h;
         hc.arith_ok = arith_ok;

@@ -195,29 +195,14 @@ template <int N> __device__ __forceinline__ void ex_wait_read() { asm volatile("
 __device__ __forceinline__ void ex_fence_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 constexpr int EX_THREADS = 512, EX_STORE_WARPS = 2, EX_GEN = EX_THREADS - 32 * EX_STORE_WARPS;
-constexpr int EX_AR_D0 = HL_D0, EX_AR_J = HL_J;    // dimensions >= EX_AR_D0 (bases >= 37): computed terms, no table rows
-
-// doubles of the fixed part of the shared-memory layout (everything before the term table)
-static size_t ex_fixed_doubles(int k) { return 4 + (2 * (size_t)k + 1) / 2 + 3 * (size_t)k + 2 * (size_t)k + 2 * (size_t)k * EX_AR_J + HL_LIST_BYTES / 8; }
 
 __global__ void __launch_bounds__(EX_THREADS, 1)
 sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restrict__ out) {
     extern __shared__ __align__(16) double smem[];
     const int k = g.k, TI = g.TI, NC = g.copies;
-    // layout: bars[4] | base[k] off[k] (u32) | magic[k] (u64) | lb[k] wr[k] | dl[k] | arh arl [k][7] | ulist[16][32] (u8) | table[table_len] |
-    //         tiles: per buffer pair (2): per copy (NC): A, B (TI*k each)
+    // layout: bars[4] | generator prefix (device.cuh: halton_prefix) | tiles: per buffer pair (2): per copy (NC): A, B (TI*k each)
+    // (the tiles are sources of cp.async.bulk: 16-byte aligned, as k is even and the table length is rounded up to even)
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem);                 // full[2], empty[2]
-    uint32_t *sbase = reinterpret_cast<uint32_t *>(smem + 4);
-    uint32_t *soff = sbase + k;
-    uint64_t *smagic = reinterpret_cast<uint64_t *>(smem + 4 + ((2 * k + 1) / 2));
-    double *slb = reinterpret_cast<double *>(smagic + k);
-    double *swr = slb + k;
-    DimLoop *sdl = reinterpret_cast<DimLoop *>(swr + k);
-    double *sarh = reinterpret_cast<double *>(sdl + k), *sarl = sarh + (size_t)k * EX_AR_J;
-    unsigned char *uwarp = reinterpret_cast<unsigned char *>(sarl + (size_t)k * EX_AR_J);   // [warp][HL_MAXQ]: the units of every generator warp
-    double *table = sarl + (size_t)k * EX_AR_J + HL_LIST_BYTES / 8;
-    double *tiles = table + ((g.table_len + 1) & ~1u);
-    const uint32_t table_saddr = smem_u32(table);
     const size_t tile = (size_t)TI * k;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     if (tid == 0) {
@@ -226,26 +211,10 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
         mbar_init(bars + 2, (uint32_t)NC);                   // every store warp releases the buffer pair
         mbar_init(bars + 3, (uint32_t)NC);
     }
-    if (!src.raw) {
-        for (int d = tid; d < k; d += EX_THREADS) {
-            sbase[d] = src.h.base[d];
-            soff[d] = src.h.off[d];
-            smagic[d] = src.h.magic[d];
-            if (g.fast) sdl[d] = dim_loop(src.h.base[d], src.start + 2 * src.n - 1);      // the largest index of the design
-        }
-        if (g.fast)
-            for (int e = tid; e < k * EX_AR_J; e += EX_THREADS) { sarh[e] = src.h.arh[e]; sarl[e] = src.h.arl[e]; }
-        for (uint32_t e = tid; e < g.table_len; e += EX_THREADS) table[e] = src.h.terms[e];
-    }
-    for (int d = tid; d < k; d += EX_THREADS) {
-        slb[d] = s.kind != VS_SCALE_IDENTITY ? s.lb[d] : 0.0;
-        swr[d] = s.kind != VS_SCALE_IDENTITY ? s.wr[d] : 1.0;
-    }
-    __syncthreads();
-    if (g.fast == 1 && tid == 0) halton_schedule(k, EX_GEN / 32, sdl, uwarp);
-    __syncthreads();
-    const double *T = g.table_len ? table : src.h.terms;
-    const HaltonShared hs{sbase, soff, smagic, sdl, sarh, sarl, table_saddr};
+    const HaltonPrefix gen = halton_prefix(smem + 4, k, src, s, g.table_len, g.fast != 0, g.fast == 1 ? EX_GEN / 32 : 0);
+    const HaltonShared &hs = gen.hs;
+    double *tiles = gen.table + ((g.table_len + 1) & ~1u);
+    const double *T = g.table_len ? gen.table : src.h.terms;
     const uint64_t n = src.n;
     const uint64_t my_tiles = blockIdx.x < g.ntiles ? (g.ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
 
@@ -268,8 +237,13 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
             mbar_wait(bars + 2 + pb, (uint32_t)(((it >> 1) & 1) ^ 1), EX_WAIT_HINT_NS);   // the store warp is done with this buffer pair
             if (gw == 1) ex_stamp(g, it, 2, lane);
             auto emit = [&](int d, double pa, double pbv) {
-                if (s.kind == VS_SCALE_LINEAR) { pa = __dadd_rn(__dmul_rn(pa, swr[d]), slb[d]); pbv = __dadd_rn(__dmul_rn(pbv, swr[d]), slb[d]); }
-                else if (s.kind == VS_SCALE_POWER) { pa = __dmul_rn(slb[d], pow(swr[d], pa)); pbv = __dmul_rn(slb[d], pow(swr[d], pbv)); }
+                if (s.kind == VS_SCALE_LINEAR) {
+                    pa = scale_value(VS_SCALE_LINEAR, gen.lb[d], gen.wr[d], pa);
+                    pbv = scale_value(VS_SCALE_LINEAR, gen.lb[d], gen.wr[d], pbv);
+                } else if (s.kind == VS_SCALE_POWER) {
+                    pa = scale_value(VS_SCALE_POWER, gen.lb[d], gen.wr[d], pa);
+                    pbv = scale_value(VS_SCALE_POWER, gen.lb[d], gen.wr[d], pbv);
+                }
                 if (live) {
                     A[(size_t)lane * k + d] = pa;
                     B[(size_t)lane * k + d] = pbv;
@@ -282,11 +256,11 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
             if (g.fast == 1) {
                 // units of one table dimension or two computed-term dimensions, balanced over the generator warps (halton_schedule)
                 const uint32_t ia[1] = {(uint32_t)(src.start + i)}, ib[1] = {(uint32_t)(src.start + n + pi)};
-                halton_units<1>(gw, uwarp, k, ia, ib, hs, [&](int d, int, double pa, double pbv) { emit(d, pa, pbv); });
+                halton_units<1>(gw, gen.ulist, k, ia, ib, hs, [&](int d, int, double pa, double pbv) { emit(d, pa, pbv); });
             } else if (g.fast == 2) {
                 // comparison form (VS_EXPORT_SLOW_GEN=2): one dimension at a time, round-robin over the generator warps
                 for (int d = gw; d < k; d += EX_GEN / 32) {
-                    const uint32_t b = sbase[d], ma = (uint32_t)(src.start + i), mb = (uint32_t)(src.start + n + pi);
+                    const uint32_t b = hs.base[d], ma = (uint32_t)(src.start + i), mb = (uint32_t)(src.start + n + pi);
                     double pa, pbv;
                     if (b == 2u) {
                         pa = (double)__brev(ma) * 2.3283064365386962890625e-10;
@@ -294,8 +268,8 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
                     } else {
                         const uint32_t ia[1] = {ma}, ib[1] = {mb};
                         double qa[1], qb[1];
-                        if (d < EX_AR_D0) halton_pair<true, 1>(ia, ib, b, smagic[d], sdl[d], table_saddr + 8u * soff[d], nullptr, nullptr, qa, qb);
-                        else halton_pair<false, 1>(ia, ib, b, smagic[d], sdl[d], 0u, sarh + (size_t)d * EX_AR_J, sarl + (size_t)d * EX_AR_J, qa, qb);
+                        if (d < HL_D0) halton_pair<true, 1>(ia, ib, b, hs.magic[d], hs.dl[d], hs.table_saddr + 8u * hs.off[d], nullptr, nullptr, qa, qb);
+                        else halton_pair<false, 1>(ia, ib, b, hs.magic[d], hs.dl[d], 0u, hs.arh + (size_t)d * HL_J, hs.arl + (size_t)d * HL_J, qa, qb);
                         pa = qa[0];
                         pbv = qb[0];
                     }
@@ -308,8 +282,8 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
                         pa = src.raw[i * (uint64_t)k + d];
                         pbv = src.raw[(n + pi) * (uint64_t)k + d];
                     } else {
-                        const uint32_t b = sbase[d];
-                        const uint64_t magic = smagic[d];
+                        const uint32_t b = hs.base[d];
+                        const uint64_t magic = hs.magic[d];
                         uint32_t ma = (uint32_t)(src.start + i), mb = (uint32_t)(src.start + n + pi);
                         if (src.h.mode == VS_HALTON_HORNER) {
                             pa = radical_inverse_horner(b, magic, ma);
@@ -318,7 +292,7 @@ sample_flat_bulk_kernel(ExportGeom g, SourceDev src, ScaleDev s, double *__restr
                             pa = (double)__brev(ma) * 2.3283064365386962890625e-10;
                             pbv = (double)__brev(mb) * 2.3283064365386962890625e-10;
                         } else {
-                            const double *row = T + soff[d];
+                            const double *row = T + hs.off[d];
                             pa = 0.0;
                             pbv = 0.0;
                             while ((ma | mb) != 0u) {                       // an exhausted index keeps adding row[0] == 0.0: exact
@@ -476,15 +450,10 @@ static int launch_sample_flat_bulk(vs_ctx *c, int k, const SourceDev &src, const
         g.re = (row_end - 1) % src.n;
     }
     const size_t avail = c->smem_optin;
-    const size_t fixed = (ex_fixed_doubles(k) + 2) * sizeof(double);
-    // fast generator: table rows only for the small bases (dimensions < EX_AR_D0), computed terms for the rest
+    const size_t fixed = (4 + halton_prefix_doubles(k) + 2) * sizeof(double);      // mbarriers, generator prefix without the table
+    // fast generator: table rows only for the small bases (dimensions < HL_D0), computed terms for the rest
     g.fast = (!src.raw && src.h.mode != VS_HALTON_HORNER && src.h.arith_ok && c->opt.export_slow_gen != 1) ? (c->opt.export_slow_gen == 2 ? 2 : 1) : 0;
-    size_t tab_terms = src.raw ? 0 : src.h.total_terms;
-    if (g.fast && k > EX_AR_D0) {
-        static const uint32_t small_primes[EX_AR_D0] = {2, 3, 5, 7, 11, 13, 17, 19, 23, 29, 31};
-        tab_terms = 0;
-        for (int d = 0; d < EX_AR_D0; ++d) tab_terms += small_primes[d] * c->halton.ndigits[d];   // terms are laid out dimension by dimension
-    }
+    const size_t tab_terms = src.raw ? 0 : g.fast ? halton_table_prefix(c->halton) : src.h.total_terms;
     const size_t tab = ((tab_terms + 1) & ~(size_t)1) * sizeof(double);
     // tile height: 32 rows (one lane per row in the store warp); two copies of every tile if they fit beside the term table
     // store warps / tile copies: one when A and B blocks of the same column alternate (every block wanted), else two (see above)

@@ -100,7 +100,6 @@ __global__ void eval_values_kernel(int k, int pts_per_chunk, SourceDev src, Scal
 // this phase to ~1.5 (tools/bench_configs.py).  The values are the same products associated differently (prefix * term *
 // suffix instead of left to right): <= 2 ulp from F::operator(), far inside the 1e-10 contract on the indices.
 // ---------------------------------------------------------------------------------------------
-constexpr int PF_AR_D0 = HL_D0, PF_AR_J = HL_J;
 
 // NR row groups per lane: a CTA tile has 32 NR rows and 8 NR warps.  NR = 2 (one CTA of 16 warps per SM instead of two of 8)
 // keeps the rows in flight per SM, doubles the independent digit chains per warp and halves the per-dimension prologue per row
@@ -110,39 +109,12 @@ __global__ void __launch_bounds__(256 * NR, NR == 1 ? 2 : 1)
 eval_values_pf_kernel(int k, SourceDev src, ScaleDev s, F f, uint64_t i_begin, uint64_t i_end, uint32_t table_len, double *__restrict__ fvals) {
     constexpr int ROWS = 32 * NR, WARPS = 8 * NR;
     extern __shared__ __align__(16) double smem[];
-    // layout: base[k] off[k] (u32) | magic[k] (u64) | lb wr [k] | arh arl [k][7] | dl[k] | ulist[16][32] (u8) | table[table_len] |
-    //         TA TB [k][ROWS] | PA PB SA SB [k+1][ROWS]
-    uint32_t *sbase = reinterpret_cast<uint32_t *>(smem);
-    uint32_t *soff = sbase + k;
-    uint64_t *smagic = reinterpret_cast<uint64_t *>(smem + ((2 * k + 1) / 2));
-    double *slb = reinterpret_cast<double *>(smagic + k);
-    double *swr = slb + k;
-    double *sarh = swr + k, *sarl = sarh + (size_t)k * PF_AR_J;
-    DimLoop *sdl = reinterpret_cast<DimLoop *>(sarl + (size_t)k * PF_AR_J);       // 16 bytes per dimension
-    unsigned char *ulist = reinterpret_cast<unsigned char *>(sdl + k);            // [warp][HL_MAXQ]: the units of every warp
-    double *table = reinterpret_cast<double *>(sdl + k) + HL_LIST_BYTES / 8;
-    const uint32_t table_saddr = (uint32_t)__cvta_generic_to_shared(table);
-    double *TA = table + table_len, *TB = TA + (size_t)k * ROWS;
+    // layout: generator prefix (device.cuh: halton_prefix) | TA TB [k][ROWS] | PA PB SA SB [k+1][ROWS]
+    const HaltonPrefix gen = halton_prefix(smem, k, src, s, table_len, !src.raw, src.raw ? 0 : WARPS);
+    const HaltonShared &hs = gen.hs;
+    double *TA = gen.table + table_len, *TB = TA + (size_t)k * ROWS;
     double *PA = TB + (size_t)k * ROWS, *PB = PA + (size_t)(k + 1) * ROWS, *SA = PB + (size_t)(k + 1) * ROWS, *SB = SA + (size_t)(k + 1) * ROWS;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (!src.raw) {
-        for (int d = tid; d < k; d += blockDim.x) {
-            sbase[d] = src.h.base[d];
-            soff[d] = src.h.off[d];
-            smagic[d] = src.h.magic[d];
-            sdl[d] = dim_loop(src.h.base[d], src.start + 2 * src.n - 1);          // the largest index of the design
-        }
-        for (int e = tid; e < k * PF_AR_J; e += blockDim.x) { sarh[e] = src.h.arh[e]; sarl[e] = src.h.arl[e]; }
-        for (uint32_t e = tid; e < table_len; e += blockDim.x) table[e] = src.h.terms[e];
-    }
-    for (int d = tid; d < k; d += blockDim.x) {
-        slb[d] = s.kind != VS_SCALE_IDENTITY ? s.lb[d] : 0.0;
-        swr[d] = s.kind != VS_SCALE_IDENTITY ? s.wr[d] : 1.0;
-    }
-    __syncthreads();
-    if (!src.raw && tid == 0) halton_schedule(k, WARPS, sdl, ulist);
-    __syncthreads();
-    const HaltonShared hs{sbase, soff, smagic, sdl, sarh, sarl, table_saddr};
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint64_t rows = i_end - i_begin, n = src.n;
     const uint64_t ntiles = (rows + ROWS - 1) / ROWS;
     // base row of the lane's r-th row of a tile (clamped: the last tile may be ragged) and its permutation entry; the entry of
@@ -175,8 +147,13 @@ eval_values_pf_kernel(int k, SourceDev src, ScaleDev s, F f, uint64_t i_begin, u
         }
         // ---- P1: coordinates and terms
         auto emit = [&](int d, int r, double pa, double pb) {
-            if (s.kind == VS_SCALE_LINEAR) { pa = __dadd_rn(__dmul_rn(pa, swr[d]), slb[d]); pb = __dadd_rn(__dmul_rn(pb, swr[d]), slb[d]); }
-            else if (s.kind == VS_SCALE_POWER) { pa = __dmul_rn(slb[d], pow(swr[d], pa)); pb = __dmul_rn(slb[d], pow(swr[d], pb)); }
+            if (s.kind == VS_SCALE_LINEAR) {
+                pa = scale_value(VS_SCALE_LINEAR, gen.lb[d], gen.wr[d], pa);
+                pb = scale_value(VS_SCALE_LINEAR, gen.lb[d], gen.wr[d], pb);
+            } else if (s.kind == VS_SCALE_POWER) {
+                pa = scale_value(VS_SCALE_POWER, gen.lb[d], gen.wr[d], pa);
+                pb = scale_value(VS_SCALE_POWER, gen.lb[d], gen.wr[d], pb);
+            }
             TA[(size_t)d * ROWS + 32 * r + lane] = f.term(d, pa);
             TB[(size_t)d * ROWS + 32 * r + lane] = f.term(d, pb);
         };
@@ -186,7 +163,7 @@ eval_values_pf_kernel(int k, SourceDev src, ScaleDev s, F f, uint64_t i_begin, u
                 for (int r = 0; r < NR; ++r) emit(d, r, src.raw[ii[r] * (uint64_t)k + d], src.raw[(n + pi[r]) * (uint64_t)k + d]);
         } else {
             // units of one table dimension or two computed-term dimensions, balanced over the warps (device.cuh: halton_schedule)
-            halton_units<NR>(warp, ulist, k, ia, ib, hs, emit);
+            halton_units<NR>(warp, gen.ulist, k, ia, ib, hs, emit);
         }
         __syncthreads();
         // ---- P2: four product chains per row group, lane = row
@@ -255,18 +232,9 @@ static int launch_eval_pf(vs_ctx *c, int k, const SourceDev &src, const ScaleDev
     const uint64_t rows = i_end - i_begin;
     if (rows == 0 || c->opt.no_pf_eval) return VS_OK;
     if (!src.raw && (src.h.mode == VS_HALTON_HORNER || !src.h.arith_ok || halton_unit_count(k) > HL_MAX_UNITS)) return VS_OK;
-    uint32_t table_len = 0;
-    if (!src.raw) {
-        // the table prefix of the dimensions below PF_AR_D0 (terms are laid out dimension by dimension: b_d * ndigits_d each)
-        static const uint32_t small_primes[PF_AR_D0] = {2, 3, 5, 7, 11, 13, 17, 19, 23, 29, 31};
-        table_len = 0;
-        for (int d = 0; d < k && d < PF_AR_D0; ++d) table_len += small_primes[d] * c->halton.ndigits[d];
-        if (k <= PF_AR_D0) table_len = src.h.total_terms;
-    }
+    const uint32_t table_len = src.raw ? 0 : halton_table_prefix(c->halton);
     auto smem_of = [&](int nr) {
-        const size_t doubles = (size_t)(2 * k + 1) / 2 + (size_t)k + 2 * (size_t)k + 2 * (size_t)k * PF_AR_J + 2 * (size_t)k + HL_LIST_BYTES / 8 +
-                               table_len + 2 * (size_t)k * 32 * nr + 4 * (size_t)(k + 1) * 32 * nr + 2;
-        return doubles * sizeof(double);
+        return (halton_prefix_doubles(k) + table_len + 2 * (size_t)k * 32 * nr + 4 * (size_t)(k + 1) * 32 * nr + 2) * sizeof(double);
     };
     // VS_PF_ROWS=64: two row groups per lane (64-row tiles, one CTA of 16 warps per SM).  Measured SLOWER at C4 (3.07 vs 2.76 ms):
     // twice the independent chains per warp do not make up for losing the second CTA whose phases interleave with the first.

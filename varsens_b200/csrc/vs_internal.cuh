@@ -52,9 +52,11 @@ struct HaltonDev {
     int mode;               // enum vs_halton_mode (HORNER: the table is not used)
     const double *fixed;    // the same terms in the fused kernels' fixed layout (all digit positions of a 32-bit index), k <= 32
     uint32_t fixed_len;
-    const double *arh, *arl; // [k][7] double-double reciprocals / 8 of the computed-term form (host.cu: build_arith), device
+    const double *arh, *arl; // [k][HL_J] double-double reciprocals / 8 of the computed-term form (host.cu: build_arith), device
     int arith_ok;           // they reproduce the term table bit for bit
 };
+constexpr int HL_D0 = 11;   // run-time-base generators: dimensions >= HL_D0 (bases >= 37) compute their terms, below: table rows
+constexpr int HL_J = 7;     // digit positions of a 32-bit index in base >= 37 (layout of HaltonDev::arh / arl)
 
 // scale.py:33 / :62 lowered: linear  -> p * w + lb   (w = ub - lb rounded on the host, as numpy does)
 //                            power   -> lb * pow(r, p) (r = ub / lb rounded on the host)
@@ -104,13 +106,16 @@ struct HaltonCache {
     int k = 0;
     int mode = 0;
     std::vector<uint32_t> ndigits;
-    // double-double reciprocals for computed terms (fused_impl.cuh: digit_step_arith), [k][7], and whether they reproduce
+    std::vector<uint32_t> off;      // host copy of HaltonDev::off: dimension after dimension, base * ndigits terms each
+    // double-double reciprocals for computed terms (fused_impl.cuh: digit_step_arith), [k][HL_J], and whether they reproduce
     // every entry of the term table bit for bit (checked when the table is built)
     std::vector<double> arh, arl;
     bool arith_ok = false;
     HaltonDev dev{};
     void *blob = nullptr;
 };
+// Doubles of the term table that hold the dimensions below HL_D0: what the run-time-base generators copy to shared memory.
+inline uint32_t halton_table_prefix(const HaltonCache &hc) { return hc.k > HL_D0 ? hc.off[HL_D0] : hc.dev.total_terms; }
 
 // Switches read from the environment ONCE, at vs_ctx_create (and again on vs_ctx_reload_env) -- never on a launch path.
 struct Options {
