@@ -89,13 +89,21 @@ typedef struct vs_scale {
  *                outputs from the time it did not reach on are NaN (an ordinary value, see vs_last_network_stats).  State:
  *                k + 8S + R doubles per thread, 32 threads at least, else VS_ERR_UNSUPPORTED.  Two-phase route only;
  *                VS_FLAG_SEPARABLE is VS_ERR_UNSUPPORTED.  Frozen arithmetic in device.cuh: MassActionAdaptive.
+ *   MASS_ACTION_STIFF: the same network and exactly the same params as MASS_ACTION_ADAPTIVE (header, records, initial
+ *                amounts, weights, output times, l = L*NT, limits, output times and failure rules), integrated by the
+ *                L-stable adaptive Rosenbrock method Rodas3 for stiff networks (rates many orders of magnitude apart).  One
+ *                sparse Jacobian and LU factorisation per attempted step, in a fill-reducing order derived once per
+ *                network; a zero or non-finite pivot rejects the attempt (step x 0.2) and does not fail the trajectory.
+ *                State: k + 7S + R + nnz(LU) doubles per thread (nnz(LU) = nonzeros of the factor, diagonal included), 32
+ *                threads at least, else VS_ERR_UNSUPPORTED.  Two-phase route only; VS_FLAG_SEPARABLE is
+ *                VS_ERR_UNSUPPORTED.  Frozen arithmetic in device.cuh: MassActionStiff.
  *
- * Every objective has l outputs per point: 1 for the first three, L for MASS_ACTION, L*NT for MASS_ACTION_ADAPTIVE
- * (vs_objective_outputs).  The entry
+ * Every objective has l outputs per point: 1 for the first three, L for MASS_ACTION, L*NT for MASS_ACTION_ADAPTIVE and
+ * MASS_ACTION_STIFF (vs_objective_outputs).  The entry
  * points that take an objective write l columns: vs_eval_values rows*(2+2k)*l doubles, vs_fused_partials
  * vs_partials_len(k, l) doubles, vs_run_fused / vs_run_fused_p2p vs_result arrays sized for l. */
 enum vs_objective { VS_OBJ_GFUNCTION = 0, VS_OBJ_ISHIGAMI = 1, VS_OBJ_RK4_CHAIN = 2, VS_OBJ_MASS_ACTION = 3,
-                   VS_OBJ_MASS_ACTION_ADAPTIVE = 4 };
+                   VS_OBJ_MASS_ACTION_ADAPTIVE = 4, VS_OBJ_MASS_ACTION_STIFF = 5 };
 
 /* fp64 arithmetic of the Halton radical inverse (the reference delegates it to the third-party ghalton package,
  * varsens/saltelli.py:82-84, whose source is not part of the reference; see DESIGN.md "parity unpinned").  The first three are
@@ -170,8 +178,8 @@ int vs_reference_permutation(uint64_t n, uint32_t seed, uint32_t *perm, uint32_t
  * i.e. exactly the combinations vs_finalize adds up (saltelli.py:612-613, 618-619); vectors from
  * vs_partials_from_values hold the plain entries.  Both kinds add up across shards and ranks. */
 size_t vs_partials_len(int k, int l);
-/* Outputs per point l of a registered objective (1, L for VS_OBJ_MASS_ACTION, L*NT for VS_OBJ_MASS_ACTION_ADAPTIVE) in *l,
- * after the same validation of k, objective and params the evaluating entry points run (VS_ERR_ARG on a malformed
+/* Outputs per point l of a registered objective (1, L for VS_OBJ_MASS_ACTION, L*NT for VS_OBJ_MASS_ACTION_ADAPTIVE and
+ * VS_OBJ_MASS_ACTION_STIFF) in *l, after the same validation of k, objective and params the evaluating entry points run (VS_ERR_ARG on a malformed
  * description). */
 int vs_objective_outputs(int k, int objective, const double *params, int n_params, int *l);
 
@@ -287,12 +295,13 @@ int vs_last_kernel_ms(vs_ctx *ctx, float *ms);
  * group row + fence + ticket, second-level combine, packing; then that CTA's own prologue, main loop and CTA-level combine}
  * -- 11 doubles. */
 int vs_last_tail_ns(vs_ctx *ctx, int k, double *ns11);
-/* Step counts of the last call on this ctx that evaluated a VS_OBJ_MASS_ACTION_ADAPTIVE network (vs_eval_values,
+/* Step counts of the last call on this ctx that evaluated a VS_OBJ_MASS_ACTION_ADAPTIVE or VS_OBJ_MASS_ACTION_STIFF network
+ * (vs_eval_values,
  * vs_fused_partials, vs_run_fused, vs_run_fused_p2p), over the trajectories of its base rows [i_begin, i_end) -- not the
  * extra evaluation of base row 0 for the common shift: stats[0] accepted steps, [1] rejected steps, [2] failed trajectories,
  * [3] lane work = the sum over warps (32 consecutive rows of one design point) of rows in the warp x the most attempts of
  * any lane in it.  (accepted + rejected) / lane work is the share of lanes that did useful work.  Synchronises the ctx
- * stream; VS_ERR_ARG if no adaptive network has been evaluated on this ctx. */
+ * stream; VS_ERR_ARG if no adaptive or stiff network has been evaluated on this ctx. */
 int vs_last_network_stats(vs_ctx *ctx, uint64_t stats[4]);
 
 #ifdef __cplusplus

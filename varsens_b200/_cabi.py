@@ -15,7 +15,7 @@ LIB_PATH = os.environ.get("VS_LIB") or os.path.join(_HERE, "libvarsens_b200.so")
 VS_OK = 0
 MEM_HOST, MEM_DEVICE = 0, 1
 SCALE_IDENTITY, SCALE_LINEAR, SCALE_POWER = 0, 1, 2
-OBJ_GFUNCTION, OBJ_ISHIGAMI, OBJ_RK4_CHAIN, OBJ_MASS_ACTION, OBJ_MASS_ACTION_ADAPTIVE = 0, 1, 2, 3, 4
+OBJ_GFUNCTION, OBJ_ISHIGAMI, OBJ_RK4_CHAIN, OBJ_MASS_ACTION, OBJ_MASS_ACTION_ADAPTIVE, OBJ_MASS_ACTION_STIFF = 0, 1, 2, 3, 4, 5
 NETWORK_STATS = ("accepted", "rejected", "failed", "lane_work")      # vs_last_network_stats, in order
 FLAG_SECOND_ORDER, FLAG_SEPARABLE = 1, 2
 
@@ -126,7 +126,7 @@ def check(status):
 def objective_outputs(k, objective, params):
     """Outputs per point l of a registered objective (vs_objective_outputs: host only, validates the parameters).  Every
     objective but a mass-action network has one, known without a call."""
-    if int(objective) not in (OBJ_MASS_ACTION, OBJ_MASS_ACTION_ADAPTIVE):
+    if int(objective) not in (OBJ_MASS_ACTION, OBJ_MASS_ACTION_ADAPTIVE, OBJ_MASS_ACTION_STIFF):
         return 1
     par = numpy.ascontiguousarray(params, dtype=numpy.float64)
     l = ctypes.c_int()

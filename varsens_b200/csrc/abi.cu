@@ -116,7 +116,8 @@ int peer_table(vs_ctx *c, int world_size, int rank, const uint64_t *peer_bufs, c
 // Outputs per point of `objective`: 1 for every objective but a mass-action network, whose description is validated here.
 int outputs_of(int k, int objective, const double *params, int n_params, int *l) {
     *l = 1;
-    if (objective != VS_OBJ_MASS_ACTION && objective != VS_OBJ_MASS_ACTION_ADAPTIVE) return VS_OK;
+    if (objective != VS_OBJ_MASS_ACTION && objective != VS_OBJ_MASS_ACTION_ADAPTIVE && objective != VS_OBJ_MASS_ACTION_STIFF)
+        return VS_OK;
     return objective_host(k, objective, params, n_params, nullptr, l);
 }
 
@@ -456,7 +457,7 @@ extern "C" int vs_last_tail_ns(vs_ctx *c, int k, double *ns8) {
 
 extern "C" int vs_last_network_stats(vs_ctx *c, uint64_t stats[4]) {
     VS_REQUIRE(c && stats, VS_ERR_ARG, "NULL argument");
-    VS_REQUIRE(c->stats_buf.p, VS_ERR_ARG, "no adaptive mass-action network has been evaluated on this ctx");
+    VS_REQUIRE(c->stats_buf.p, VS_ERR_ARG, "no adaptive or stiff mass-action network has been evaluated on this ctx");
     VS_CUDA(cudaSetDevice(c->device));
     VS_CUDA(cudaMemcpyAsync(stats, c->stats_buf.p, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
     VS_CUDA(cudaStreamSynchronize(c->stream));

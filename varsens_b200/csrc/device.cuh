@@ -543,6 +543,35 @@ struct RK4ChainDyn {
 //                     MassAction's: acc = fma(w[o][s], X_s, acc) from 0.0 over the nonzero weights, ascending s.
 //   next step         h = hs * fac (accepted or not).
 
+// MassActionStiff (VS_OBJ_MASS_ACTION_STIFF; kernel network_rosenbrock_kernel in kernels_network.cu).  FROZEN ARITHMETIC,
+// restated bit for bit by the oracle (oracle/mass_action_stiff.c: f_mass_action_stiff), same operation rules as MassActionAdaptive.
+// Rodas3 (Sandu et al. 1997, as tabulated in KPP's Rosenbrock.f90), autonomous form, gamma = 1/2, G = I/(hs gamma) - J(X):
+//   right-hand side   MassAction's.  f(X) is kept across rejected attempts and formed again after each accepted step.
+//   start, attempt    MassActionAdaptive's: t, h = h0, output-time clipping, max_steps, t + hs == t (NaN from there on).
+//   Jacobian, factor  the slots of the factor's pattern (kernels_network.cu: stiff_program) are set to 0.0; then, over the
+//                     reactions ascending, for each of its columns c (reactants, and products if reversible; catalysts
+//                     included): dP = d(side product)/dX_c (0, 1, X_other, or 2 * X_c for a homodimer), d = fma(kf, dPf,
+//                     -(kr * dPr)) if reversible else kf * dPf, and for each species s with net coefficient nu != 0:
+//                     G[s][c] = fma(-nu, d, G[s][c]).  Then G[s][s] += 1 / (0.5 * hs).  Then right-looking LU without
+//                     pivoting in elimination order p = 0 .. S-1: a pivot that is 0 or not finite rejects the attempt with
+//                     h = hs * 0.2 (the trajectory goes on, the next attempt is "after a rejection"); else for each L entry
+//                     (i, p): l = G[i][p] / pivot, G[i][p] = l, and for each U entry (p, j): G[i][j] = fma(-l, G[p][j], G[i][j]).
+//   solve             b = G^{-1} b in place: forward, p ascending, b[i] = fma(-L[i][p], b[p], b[i]) over L entries (i, p);
+//                     back, p descending, acc = b[p], acc = fma(-U[p][j], b[j], acc) over U entries (p, j), j ascending in
+//                     elimination position, b[p] = acc / U[p][p].
+//   stages            c_ij = C_ij / hs (C21 = 4, C31 = 1, C32 = -1, C41 = 1, C42 = -1, C43 = -8/3 correctly rounded).
+//                     K1 = solve(f(X));  K2 = solve(fma(c21, K1, f(X)));  Y = fma(2, K1, X);
+//                     K3 = solve(fma(c32, K2, fma(c31, K1, f(Y))));  Y = Y + K3;
+//                     K4 = solve(fma(c43, K3, fma(c42, K2, fma(c41, K1, f(Y)))));  X_new = Y + K4 (stiffly accurate).
+//   error             sc_s = fma(rtol, fmax(|X_s|, |X_new,s|), atol);  r = K4_s / sc_s;  q = fma(r, r, q) from 0.0 over
+//                     ascending s;  err = sqrt(q / S).
+//   controller        fac_max = 1.0 on the attempt after a rejection, else 6.0.  fac = 0.2 if err is not finite; else
+//                     fmin(fac_max, fmax(0.2, 0.9 / cbrt(fmin(fmax(err, 1e-3), 1e3)))) (the clamp changes no factor: outside
+//                     it the bounds apply), where cbrt(a) = four Newton steps y = fma(2, y, a / (y * y)) / 3 from the bits
+//                     (bits(a) / 3 + 0x2A9F7893782DA1CE) as an unsigned 64-bit integer division.
+//   accept iff err <= 1.0:  t = to if clipped, else t + hs;  X = X_new; observables at a clipped step as MassActionAdaptive.
+//   next step         h = hs * fac (accepted or not).
+
 __host__ __device__ __forceinline__ void tile_coords(int id, int nt, int &tr, int &tc) {
     tr = 0;
     int rowlen = nt;

@@ -332,6 +332,7 @@ int objective_host(int k, int objective, const double *params, int n_params, std
         break;
     case VS_OBJ_MASS_ACTION:
     case VS_OBJ_MASS_ACTION_ADAPTIVE:
+    case VS_OBJ_MASS_ACTION_STIFF:
         return network_describe(k, objective, params, n_params, hp, l);
     default:
         set_error("unknown objective id %d", objective);

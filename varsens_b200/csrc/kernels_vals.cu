@@ -314,6 +314,7 @@ int launch_eval_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s
     }
     case VS_OBJ_MASS_ACTION:
     case VS_OBJ_MASS_ACTION_ADAPTIVE:
+    case VS_OBJ_MASS_ACTION_STIFF:
         return launch_network_values(c, k, src, s, o, i_begin, i_end, fvals, count);
     }
     set_error("unknown objective id %d", o.id);

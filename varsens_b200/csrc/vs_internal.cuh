@@ -174,7 +174,7 @@ struct vs_ctx {
     // scratch
     std::vector<cudaEvent_t> pipe_ev;    // [0]: "compute stream is done with the staging buffer" (ordering of the next H2D copy)
     vs::DevBuf pipe_buf;
-    vs::DevBuf stats_buf;                // 4 x uint64 step counts of the last adaptive-network evaluation (vs_last_network_stats)
+    vs::DevBuf stats_buf;                // 4 x uint64 step counts of the last adaptive or stiff network evaluation (vs_last_network_stats)
     vs::DevBuf scale_buf, obj_buf, perm_buf, raw_buf, io_buf, part_buf, block_buf, res_buf, dir_buf, misc_buf;
 };
 
@@ -203,7 +203,7 @@ int launch_sample_flat(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s
                        uint64_t row_end, double *out);
 int launch_sample_shard(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, uint64_t i_begin, uint64_t i_end, double *out);
 // kernels_vals.cu
-// count = false: an adaptive network's step counts (vs_last_network_stats) are neither reset nor added to
+// count = false: an adaptive or stiff network's step counts (vs_last_network_stats) are neither reset nor added to
 int launch_eval_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, const ObjectiveDev &o,
                        uint64_t i_begin, uint64_t i_end, double *fvals, bool count = true);
 int launch_partials_from_values(vs_ctx *c, int k, int l, uint64_t rows, const double *fvals, const double *shift_dev,
@@ -215,7 +215,7 @@ int launch_gram_scatter(vs_ctx *c, const GramGeom &g, int nblocks, const double 
 // kernels_gram_mma.cu: tensor-path Gram (*handled = false -> caller falls back to gram_kernel)
 int launch_gram_mma(vs_ctx *c, int k, int l, uint64_t rows, const double *fvals, const double *shift_dev, int flags,
                     double *partials, bool *handled);
-// kernels_network.cu: VS_OBJ_MASS_ACTION and VS_OBJ_MASS_ACTION_ADAPTIVE
+// kernels_network.cu: VS_OBJ_MASS_ACTION, VS_OBJ_MASS_ACTION_ADAPTIVE and VS_OBJ_MASS_ACTION_STIFF
 int network_describe(int k, int objective, const double *params, int n_params, std::vector<double> *h, int *l);
 int network_check_fit(vs_ctx *c, int k, const ObjectiveDev &o);       // VS_ERR_UNSUPPORTED if the state does not fit
 int launch_network_values(vs_ctx *c, int k, const SourceDev &src, const ScaleDev &s, const ObjectiveDev &o, uint64_t i_begin,

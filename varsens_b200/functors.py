@@ -207,14 +207,21 @@ class AdaptiveMassActionNetwork(_Network):
     ``species``, ``reactions``, ``initial`` and ``observables`` are those of MassActionNetwork; L * NT <= 64.
     ``rtol`` >= 0, ``atol`` > 0: the error of a step is measured against rtol * |X_s| + atol per species;
     ``h0``           the first step (None: 1e-6 * times[-1]);
-    ``max_steps``    attempted steps per trajectory before it is marked failed.
+    ``max_steps``    attempted steps per trajectory before it is marked failed;
+    ``method``       "dopri5" (explicit, VS_OBJ_MASS_ACTION_ADAPTIVE) or "rodas3": the L-stable Rosenbrock method for stiff
+                     networks, whose rates lie orders of magnitude apart (VS_OBJ_MASS_ACTION_STIFF; same packed parameters).
     A failed trajectory (more than max_steps attempts, or a step too small to advance t) gives NaN from the output time it
     could not reach on; Objective and Varsens then issue a RuntimeWarning with the count.  Packed layout and frozen arithmetic:
-    include/varsens_b200.h (VS_OBJ_MASS_ACTION_ADAPTIVE)."""
-    objective_id = _cabi.OBJ_MASS_ACTION_ADAPTIVE
+    include/varsens_b200.h (VS_OBJ_MASS_ACTION_ADAPTIVE, VS_OBJ_MASS_ACTION_STIFF)."""
+    objective_id = _cabi.OBJ_MASS_ACTION_ADAPTIVE                       # of the default method; each instance sets its own
+    METHODS = {"dopri5": _cabi.OBJ_MASS_ACTION_ADAPTIVE, "rodas3": _cabi.OBJ_MASS_ACTION_STIFF}
 
-    def __init__(self, species, reactions, initial, observables, times, rtol=1e-6, atol=1e-9, h0=None, max_steps=100000):
+    def __init__(self, species, reactions, initial, observables, times, rtol=1e-6, atol=1e-9, h0=None, max_steps=100000,
+                 method="dopri5"):
         err = _cabi.VarsensError
+        if not isinstance(method, str) or method not in self.METHODS:
+            raise err("AdaptiveMassActionNetwork: method = %r, need one of %s" % (method, sorted(self.METHODS)))
+        self.method, self.objective_id = method, self.METHODS[method]
         _Network.__init__(self, species, reactions, initial, observables)
         try:
             t = numpy.asarray(times, dtype=numpy.float64)
